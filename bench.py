@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU arm: the reference path on host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs as .npy
 
 Workload at every N: BASELINE.json configs[1]/[2] — motion-diffusion denoiser TRAINING on synthetic
 AddBiomechanics-shaped windows (F=50 frames, 177 kinematic channels, 30 target channels), bf16 GEMMs,
@@ -197,6 +198,30 @@ def cpu_other_configs() -> dict:
     return out
 
 
+DUMP_SAMPLE = 4 << 20          # parameter / gradient elements kept per array: 2 x 16 MB of fp32, well under 64 MB in all
+
+
+def dump_outputs(out_dir: str, result, arena) -> None:
+    """What the last timed step hands its caller, for comparing two builds output for output:
+    step_result.npy  the fp32[40] the step returns (loss at [0], then its per-channel and report metrics);
+    params.npy       the fp32 parameters the step's optimizer update left in place;
+    grads.npy        the fp32 parameter gradients of that step.
+    Arenas larger than DUMP_SAMPLE elements are written as the same seeded, sorted sample of positions every run.
+    The inputs are seeded, but the bias-gradient and LayerNorm reductions add with float atomics, so two runs differ in the
+    last bits of every gradient and RMSprop compounds that over the steps: compare dumps with a tolerance."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = arena.total
+    idx = None
+    if n > DUMP_SAMPLE:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values.to(arena.device)
+    for name, t in (("step_result", result), ("params", arena.master), ("grads", arena.grad)):
+        if name != "step_result" and idx is not None:
+            t = t[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -209,7 +234,13 @@ def main():
     ap.add_argument("--no-sampling", action="store_true", help="skip the configs[3] reverse-sampling block")
     ap.add_argument("--sampling-steps", type=int, default=1000, help="denoise steps of the sampling block (configs[3]: 1000)")
     ap.add_argument("--sampling-windows", type=int, default=512, help="windows per GPU of the sampling block (configs[3]: 4096 / 8)")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="GPU arm only: after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm only, not to --impl reference")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -270,6 +301,8 @@ def main():
     ms_per_step = elapsed_ms.item() / args.steps
     value = world * B / (ms_per_step * 1e-3)
     final_loss = res[0].item()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, model.arena)
 
     # ------------------------------------------------ e2e: host buffers through the public call ---------------------
     host = trainer.make_host_batch(B, seed=99 + rank)               # pinned CPU tensors (dict of 10 inputs + 4 labels)

@@ -1,6 +1,7 @@
-"""oracle/loss.py and oracle/models.py against the IMPORTED reference, live, on inputs the frozen fixtures never saw
-(build container only: /root/reference or the oracle/_ref snapshot must be importable; skipped elsewhere).  The golden
-files pin a handful of seeded cases; these draw fresh shapes, component selections and constructor arguments every case:
+"""oracle/loss.py and oracle/models.py against the IMPORTED reference, live, on inputs the frozen fixtures never saw.
+The original project's sources must be importable (IBM_REFERENCE_ROOT or the oracle/_ref snapshot); no stored copy of
+these cases' reference outputs exists, so without the sources the module skips.  The golden files pin a handful of
+seeded cases; these draw fresh shapes, component selections and constructor arguments every case:
 
 * RegressionLossEvaluator.__call__ (RegressionLossEvaluator.py:160-263): loss, the four component vectors, the six report
   metrics and autograd gradients — random (B, F), selections with repeats / empty lists, forces placed exactly ON the 10.0
@@ -21,7 +22,7 @@ from oracle import models as om
 from oracle.gen_golden import run_ref_loss, seeded_inputs
 from oracle.refimport import load_reference, reference_available
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="needs the importable reference (build container / oracle/_ref)")
+pytestmark = pytest.mark.skipif(not reference_available(), reason="needs the original project's sources (IBM_REFERENCE_ROOT or oracle/_ref)")
 
 
 def _rand_out_labels(B, F, g, on_threshold=False):

@@ -1,18 +1,19 @@
-"""The window oracle against the reference's own AddBiomechanicsDataset, LIVE: where /root/reference is present (the build
-container; the GPU box has only the frozen tests/golden/windows.npz) the real class runs over freshly drawn synthetic subjects
+"""The window oracle against the reference's own AddBiomechanicsDataset, LIVE: where the original project's sources are
+importable (IBM_REFERENCE_ROOT or the oracle/_ref snapshot; no stored copy of these cases exists, only the frozen
+tests/golden/windows.npz of other cases) the real class runs over freshly drawn synthetic subjects
 through oracle/fake_nimble.py and must agree with oracle/windows.py bit for bit — index (Dataset.py:131-139), every
 __getitem__ dict (Dataset.py:161-285: strided frame gather, label re-order to the dataset's contact-body order, /mass except
 CoP) — on seeds and shapes the frozen fixture never saw, including the degenerate ones: trials shorter than the window,
 trials with every frame missing, a window as long as the trial allows, stride == window size, one subject."""
-import os
 import tempfile
 
 import numpy as np
 import pytest
 
 from oracle import windows as ow
+from oracle.refimport import reference_available
 
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/src/data"), reason="needs the reference tree (build container only)")
+pytestmark = pytest.mark.skipif(not reference_available(), reason="needs the original project's sources (IBM_REFERENCE_ROOT or oracle/_ref)")
 
 CASES = [
     # seed, subjects, T, stride, format, hist_cols, max_len
