@@ -262,8 +262,8 @@ def sampling_leg(dev, world: int, rank: int, pk: dict, model, windows_per_gpu: i
     g = torch.Generator().manual_seed(4242)
     cond_host = torch.randn(world * sb, F, C, generator=g).pin_memory()          # the whole job's windows; a rank reads its shard
     mine = slice(rank * sb, (rank + 1) * sb)
-    ops.pack_inputs([cond_host[mine].reshape(-1, C).to(dev)], sb * F, F, out_bf16=eng.xc(sb, False), frame_stride=eng.ld_in,
-                    win_extra=0, col0=30)
+    buf, fs, we, col0 = eng.input_layout(sb, F, False)
+    ops.pack_inputs([cond_host[mine].reshape(-1, C).to(dev)], sb * F, F, out_bf16=buf, frame_stride=fs, win_extra=we, col0=col0)
     seed = 1
     gd.sample(model, sb, steps=20, seed=seed + rank)                             # captures the 2-step graph, warms the clocks
     e0, e1 = _events()

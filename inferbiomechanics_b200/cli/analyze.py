@@ -102,7 +102,7 @@ class AnalyzeCommand(AbstractCommand):
                         continue
                     if model_type == 'diffusion':
                         # condition = the packed kinematics in the engine's concat buffer; x_T ~ Philox; CUDA-graph replays
-                        store.pack_rows(idx, model.engine().xc(idx.numel(), False), col0=30)
+                        store.pack(idx, model.engine().input_layout(idx.numel(), store.F, False))
                         x0 = diffusion.sample(model, idx.numel(), steps=args.sampling_steps, seed=1234 + rank)
                         if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
                             x0 = x0[:, -1:]

@@ -85,16 +85,12 @@ class WindowStore:
         return [indices[i:i + batch_size] for i in range(0, indices.numel(), batch_size)]    # partial last batch kept
 
     # ---- packing -----------------------------------------------------------------------------------
-    def pack_feedforward(self, idx: torch.Tensor, dst_bf16: torch.Tensor) -> None:
-        """row-per-window [B, ld] bf16, frame-major (FeedForward…py:108 reshape)."""
-        ld = dst_bf16.stride(0)
-        ops.pack_windows(self.frames, self.C, self.win_row0[idx], self.F, self.stride, out_bf16=dst_bf16, frame_stride=self.C,
-                         win_extra=ld - self.F * self.C)
-
-    def pack_rows(self, idx: torch.Tensor, dst_bf16: torch.Tensor, col0: int = 0) -> None:
-        """row-per-frame [B*F, ld] bf16 starting at column col0 (Groundlink / denoiser layouts)."""
-        ops.pack_windows(self.frames, self.C, self.win_row0[idx], self.F, self.stride, out_bf16=dst_bf16,
-                         frame_stride=dst_bf16.stride(0), win_extra=0, col0=col0)
+    def pack(self, idx: torch.Tensor, layout) -> None:
+        """Windows ``idx`` → bf16 rows in an engine's ``input_layout`` ``(buffer, frame_stride, win_extra, col0)``: frame t of
+        window b starts at element (b * F + t) * frame_stride + b * win_extra + col0 of the buffer."""
+        dst_bf16, frame_stride, win_extra, col0 = layout
+        ops.pack_windows(self.frames, self.C, self.win_row0[idx], self.F, self.stride, out_bf16=dst_bf16, frame_stride=frame_stride,
+                         win_extra=win_extra, col0=col0)
 
     def pack_f32(self, idx: torch.Tensor) -> torch.Tensor:
         out = torch.empty(idx.numel(), self.F, self.C, dtype=torch.float32, device=self.device)

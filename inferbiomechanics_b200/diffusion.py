@@ -84,7 +84,7 @@ class GaussianDiffusion:
         t_a.fill_(self.T - 1)
 
         def step(t_in, t_out, z):
-            x0_hat = eng.forward(B, train=False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
+            x0_hat = eng.forward(B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
             ops.posterior_step(x0_hat, 32, x, z, t_in, self.coef_x0, self.coef_xt, self.sigma, M, x_prev=x, xprev_bf16=xc,
                                bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out)
 
@@ -165,7 +165,8 @@ class GaussianDiffusion:
             b = min(a + batch, mine.stop)
             nb = b - a
             main.wait_event(uploaded[i & 1])
-            ops.pack_inputs([stage[i & 1][:nb * F]], nb * F, F, out_bf16=eng.xc(nb, False), frame_stride=eng.ld_in, win_extra=0, col0=30)
+            buf, fs, we, col0 = eng.input_layout(nb, F, False)
+            ops.pack_inputs([stage[i & 1][:nb * F]], nb * F, F, out_bf16=buf, frame_stride=fs, win_extra=we, col0=col0)
             packed[i & 1].record(main)
             if i + 1 < len(starts):
                 upload(i + 1)

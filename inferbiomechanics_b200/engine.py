@@ -6,6 +6,18 @@ only the memory the kernels read and write.
 * ``EncoderLayerPlan``   — /root/reference/src/models/TransformerBaseline.py:8-38 (post-LN layer),
                             shared by the denoiser (d=512) and the TransformerBaseline (d=108 padded)
 * ``DenoiserEngine``     — builder-owned DDPM denoiser (DESIGN.md D-1), forward + backward
+
+The three model engines (and ``GroundlinkEngine``, engine_groundlink.py) share the step interface the Trainer and the
+drop-in modules drive:
+
+* ``input_layout(B, F, train)`` → ``(bf16 buffer, frame_stride, win_extra, col0)``: where the packers write frame t of
+  window b (element ``(b*F + t)*frame_stride + b*win_extra + col0``);
+* ``forward(B, F, train)`` → the fp32 output, ``dout(B, F)`` → the bf16 output-gradient buffer, ``backward(B, F)``;
+* ``quantity_views(x, B, F, Fo)`` → the four (B, Fo, ·) loss-quantity views (cop, force, torque, wrench) of either;
+* ``bucket_boundaries()`` → arena offsets of the gradient groups; backward calls ``bucket_hook(g)`` once group g and all
+  later ones are complete;
+* ``set_rng(seed_mix, rank, step, step_dev)`` seeds the dropout masks; ``refresh_weights()`` re-derives cached weight
+  copies when ``ParamArena.version`` moved.
 """
 from __future__ import annotations
 
@@ -24,6 +36,11 @@ F32 = torch.float32
 
 def _r8(x: int) -> int:
     return ops.round_up(x, 8)
+
+
+def quantity_split(rows: torch.Tensor) -> List[torch.Tensor]:
+    """(…, >=30) rows30 tensor → the four loss quantities (cop, force, torque, wrench) as views."""
+    return [rows[..., 0:6], rows[..., 6:12], rows[..., 12:18], rows[..., 18:30]]
 
 
 class _Buffers:
@@ -56,12 +73,15 @@ class FeedForwardEngine:
 
     Optional per-layer ``[Dropout][BatchNorm1d]`` on the layer INPUT (FeedForward…py:68-72): ``bn`` is a list with one
     entry per Linear (``None`` or ``(weight name, bias name, nn.BatchNorm1d module)`` — the module only holds the
-    running-statistics buffers and eps/momentum), ``dropout_p`` the probability of the Philox inverted dropout."""
+    running-statistics buffers and eps/momentum), ``dropout_p`` the probability of the Philox inverted dropout.
+    ``frame_width``: input columns per frame (a window is one row of F frames)."""
 
     DROPOUT_SEED = 0x66666e6e
 
-    def __init__(self, arena: ParamArena, layers: List[Tuple[str, str, int, int]], activation: str, bn=None, dropout_p: float = 0.0):
+    def __init__(self, arena: ParamArena, layers: List[Tuple[str, str, int, int]], activation: str, frame_width: int, bn=None,
+                 dropout_p: float = 0.0):
         self.arena = arena
+        self.frame_width = frame_width
         self.layers = layers                    # (weight name, bias name, N, K)
         self.act = activation
         self.buf = _Buffers(arena.device)
@@ -71,26 +91,51 @@ class FeedForwardEngine:
         self.in_ld = _r8(self.in_cols)
         self.bn = bn if bn is not None and any(b is not None for b in bn) else None
         self.dropout_p = float(dropout_p)
-        self.step = 0                           # Philox offset base: one fresh mask per (training forward, layer)
-        self.dropout_seed = self.DROPOUT_SEED   # Trainer.seed_rng folds its seed and the data-parallel rank in
-        self.step_dev = None                    # Trainer-owned device step counter: offsets are derived on the device (graph replay)
+        self.set_rng(0, 0, 0, None)
         if self.bn is not None:
             maxc = max(K for (_, _, _, K) in layers)
             self.bn_ws = ops.batchnorm_workspace(maxc, arena.device)
             self.bn_stats = {i: (torch.zeros(K, device=arena.device), torch.ones(K, device=arena.device))
                              for i, (_, _, _, K) in enumerate(layers) if self.bn[i] is not None}
 
+    def set_rng(self, seed_mix: int, rank: int, step: int, step_dev: Optional[torch.Tensor]) -> None:
+        """Dropout masks: Philox keyed by (DROPOUT_SEED ^ seed_mix) + rank, offset by the training-forward count ``step`` —
+        or, when ``step_dev`` (a device-resident step counter) is given, by its value, so that a captured step replays."""
+        self.dropout_seed = (self.DROPOUT_SEED ^ seed_mix) + rank
+        self.step, self.step_dev = step, step_dev
+
+    def refresh_weights(self) -> None:
+        """No derived weight copies beyond the arena's own (the GEMMs read the bf16 shadow)."""
+
+    def bucket_boundaries(self) -> List[int]:
+        """Arena offsets of the gradient groups: group i = Linear layer i (a layer's BatchNorm parameters precede it)."""
+        offs = self.arena.offsets
+        return [offs[self.bn[i][0] if self.bn is not None and self.bn[i] is not None else w][0]
+                for i, (w, _, _, _) in enumerate(self.layers)]
+
     def input_buffer(self, B: int) -> torch.Tensor:
         s = self.buf.get((B,))
         return self.buf.tensor(s, "x0", (B, self.in_ld), BF16, zero=True)
 
-    def dout_buffer(self, B: int) -> torch.Tensor:
+    def input_layout(self, B: int, F: int, train: bool) -> Tuple[torch.Tensor, int, int, int]:
+        """(buffer, frame_stride, win_extra, col0) for the packers: one row per window, frame-major (FeedForward…py:108)."""
+        return self.input_buffer(B), self.frame_width, self.in_ld - self.in_cols, 0
+
+    def dout(self, B: int, F: int) -> torch.Tensor:
         s = self.buf.get((B,))
         return self.buf.tensor(s, "dout", (B, _r8(self.out_cols)), BF16, zero=True)
 
-    def forward(self, B: int, train: bool = False) -> torch.Tensor:
+    def quantity_views(self, x: torch.Tensor, B: int, F: int, Fo: int) -> List[torch.Tensor]:
+        """(B, Fo, ·) views of the four quantities in an output / output-gradient row: quantity-then-frame blocks
+        (FeedForward…py:116-121)."""
+        def blk(a, b, c):
+            return x[:, a * Fo:b * Fo].unflatten(1, (Fo, c))
+        return [blk(0, 6, 6), blk(6, 12, 6), blk(12, 18, 6), blk(18, 30, 12)]
+
+    def forward(self, B: int, F: int, train: bool) -> torch.Tensor:
         """Consumes input_buffer(B); returns fp32 [B, ld>=N_out] (first N_out columns valid).  ``train`` selects batch
-        statistics (and updates the running ones) for BatchNorm and switches dropout on, like nn.Module.training."""
+        statistics (and updates the running ones) for BatchNorm and switches dropout on, like nn.Module.training.
+        ``F`` is implied by the layer widths."""
         s = self.buf.get((B,))
         x = self.input_buffer(B)
         n_layers = len(self.layers)
@@ -130,12 +175,12 @@ class FeedForwardEngine:
             x = y
         return x
 
-    def backward(self, B: int, accumulate_into: Optional[ParamArena] = None) -> None:
-        """Consumes dout_buffer(B) (bf16 d loss/d out); accumulates weight/bias grads into the arena."""
-        arena = accumulate_into or self.arena
+    def backward(self, B: int, F: int) -> None:
+        """Consumes dout(B, F) (bf16 d loss/d out); accumulates weight/bias grads into the arena."""
+        arena = self.arena
         s = self.buf.get((B,))
         train, drop = s.get("mode", (False, False))
-        dy = self.dout_buffer(B)
+        dy = self.dout(B, F)
         n_layers = len(self.layers)
         bias_done = False                       # layer i's bias gradient already produced by BatchNorm i+1's backward
         for i in range(n_layers - 1, -1, -1):
@@ -293,7 +338,19 @@ class DenoiserEngine:
         self.ld_in = _r8(self.k_in)
         self.layers = [EncoderLayerPlan(arena, f"layers.{l}.", d, heads, ff) for l in range(num_layers)]
         self.buf = _Buffers(arena.device)
-        self.bucket_hook = None          # callable(layer_index) fired when a layer's grads are complete
+        self.bucket_hook = None          # callable(group) fired when a group's grads are complete: 0 = stem, l + 1 = layer l, L + 1 = head
+        self._temb_key = None
+
+    def set_rng(self, seed_mix: int, rank: int, step: int, step_dev: Optional[torch.Tensor]) -> None:
+        """No dropout: nothing to seed."""
+
+    def refresh_weights(self) -> None:
+        """The time-MLP table is refreshed by ``temb_table`` itself."""
+
+    def bucket_boundaries(self) -> List[int]:
+        offs = self.arena.offsets
+        first = [offs[f"layers.{l}.multihead_attention.in_proj_weight"][0] for l in range(self.L)]
+        return [0] + first + [offs["out_proj.weight"][0]]
 
     # ---- buffers ----
     def state(self, B: int, train: bool) -> Dict[str, torch.Tensor]:
@@ -302,24 +359,32 @@ class DenoiserEngine:
     def xc(self, B: int, train: bool = True) -> torch.Tensor:
         return self.buf.tensor(self.state(B, train), "xc", (B * self.F, self.ld_in), BF16, zero=True)
 
+    def input_layout(self, B: int, F: int, train: bool) -> Tuple[torch.Tensor, int, int, int]:
+        """(buffer, frame_stride, win_extra, col0) for the packers: the kinematics go to columns 30… of xc."""
+        return self.xc(B, train), self.ld_in, 0, 30
+
     def t_buffer(self, B: int, train: bool = True) -> torch.Tensor:
         return self.buf.tensor(self.state(B, train), "t", (B,), torch.int32, zero=True)
 
-    def dout(self, B: int) -> torch.Tensor:
+    def dout(self, B: int, F: int) -> torch.Tensor:
         return self.buf.tensor(self.state(B, True), "dout", (B * self.F, 32), BF16, zero=True)
 
-    # ---- forward ----
-    def weights_changed(self) -> None:
-        """Called by the native trainer after its fused optimizer (which writes the masters through raw pointers)."""
-        self._w_epoch = getattr(self, "_w_epoch", 0) + 1
+    def quantity_views(self, x: torch.Tensor, B: int, F: int, Fo: int) -> List[torch.Tensor]:
+        """(B, Fo, ·) views of the four quantities of the last Fo frames of an [M, 32] output / output-gradient buffer."""
+        return quantity_split(x.view(B, self.F, 32)[:, self.F - Fo:])
 
+    def _check_frames(self, F: int) -> None:
+        if F != self.F:
+            raise ValueError(f"the denoiser was built for {self.F}-frame windows, got {F}")
+
+    # ---- forward ----
     def temb_table(self, n_timesteps: int) -> torch.Tensor:
         """bf16 [n, d]: the time MLP (Linear·SiLU·Linear of the sinusoidal embedding, DESIGN D-1) of EVERY timestep,
         evaluated once per set of weights.  Reverse sampling runs all windows at the same timestep, so a denoise step
         only adds row t of this table (ibm_add_time_pos with t_row) instead of re-running two GEMMs per step."""
         A, d = self.arena, self.d
-        key = (A._version_sum(), getattr(self, "_w_epoch", 0), n_timesteps)
-        if getattr(self, "_temb_key", None) != key:
+        key = (A.version, n_timesteps)
+        if self._temb_key != key:
             n = n_timesteps
             t = torch.arange(n, dtype=torch.int32, device=A.device)
             emb, pre, act = (torch.empty(n, d, dtype=BF16, device=A.device) for _ in range(3))
@@ -331,10 +396,11 @@ class DenoiserEngine:
             self._temb_table, self._temb_key = table, key
         return self._temb_table
 
-    def forward(self, B: int, train: bool = True, t_scalar: Optional[torch.Tensor] = None, t_count: int = 0) -> torch.Tensor:
+    def forward(self, B: int, F: int, train: bool, t_scalar: Optional[torch.Tensor] = None, t_count: int = 0) -> torch.Tensor:
         """Consumes xc(B) and t_buffer(B) (or a device scalar timestep); returns x0_hat fp32 [M, 32].
         ``t_count`` > 0 with ``t_scalar``: timesteps are < t_count and the time MLP comes from ``temb_table``."""
-        A, d, F = self.arena, self.d, self.F
+        self._check_frames(F)
+        A, d = self.arena, self.d
         M = B * F
         st = self.state(B, train)
         T = self.buf.tensor
@@ -367,14 +433,15 @@ class DenoiserEngine:
         return out
 
     # ---- backward ----
-    def backward(self, B: int) -> None:
-        """Consumes dout(B) (bf16 d loss/d x0_hat rows, cols 30,31 zero); accumulates grads into the arena."""
-        A, d, F, ff = self.arena, self.d, self.F, self.ff
+    def backward(self, B: int, F: int) -> None:
+        """Consumes dout(B, F) (bf16 d loss/d x0_hat rows, cols 30,31 zero); accumulates grads into the arena."""
+        self._check_frames(F)
+        A, d, ff = self.arena, self.d, self.ff
         M = B * F
         st = self.state(B, True)
         T = self.buf.tensor
         g = A.grad_of
-        dout = self.dout(B)
+        dout = self.dout(B, F)
         sc = {"ds": T(st, "ds", (M, d), BF16), "dh": T(st, "dh", (M, ff), BF16), "dx1": T(st, "dx1", (M, d), BF16),
               "do": T(st, "do", (M, d), BF16), "dqkv": T(st, "dqkv", (M, 3 * d), BF16)}
         dxa, dxb = T(st, "dxa", (M, d), BF16), T(st, "dxb", (M, d), BF16)
@@ -383,7 +450,7 @@ class DenoiserEngine:
         ops.colsum(dout, M, 30, g("out_proj.bias"))
         ops.gemm(dout, A.shadow_of("out_proj.weight", (30, d)), dxa, M, d, 30, b_mn=True)
         if self.bucket_hook is not None:
-            self.bucket_hook(self.L)              # head gradients complete
+            self.bucket_hook(self.L + 1)          # head gradients complete
         dx, other = dxa, dxb
         for l in range(self.L - 1, -1, -1):
             layer = self.layers[l]
@@ -393,7 +460,7 @@ class DenoiserEngine:
             layer.backward(x_in, a, dx, sc, M, B, F, other)
             dx, other = other, dx
             if self.bucket_hook is not None:
-                self.bucket_hook(l)
+                self.bucket_hook(l + 1)
         # dx = d loss / d h0
         dtemb, dact, dpre = (T(st, k, (B, d), BF16) for k in ("dtemb", "dact", "dpre"))
         # one pass over dx: time-embedding gradient per window, positional-table gradient, in-projection bias gradient
@@ -406,4 +473,4 @@ class DenoiserEngine:
         ops.colsum(dpre, B, d, g("time_mlp.0.bias"))
         _wgrad(A, "in_proj.weight", d, self.k_in, dx, self.xc(B), M, self.buf, st)
         if self.bucket_hook is not None:
-            self.bucket_hook(-1)
+            self.bucket_hook(0)

@@ -13,20 +13,20 @@ layout that is folded back into the (C_out, C_in, 7) parameter gradient.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Tuple
+from typing import Dict, List, Optional, Tuple
 
 import torch
 
 from . import ops
-from .engine import _Buffers, _r8
+from .engine import _Buffers, _r8, quantity_split
 from .params import ParamArena
 
 BF16, F32 = torch.bfloat16, torch.float32
-FC_DROPOUT_SEED = 0x6c696e6b
 
 
 class GroundlinkEngine:
     CNN_DROPOUT_SEED = 0x636e6e64
+    FC_DROPOUT_SEED = 0x6c696e6b
 
     def __init__(self, arena: ParamArena, c_in: int, features: List[int], fc_dropout: float, cnn_dropout: float = 0.0,
                  cnn_kernel: int = 7, fc_depth: int = 3):
@@ -45,12 +45,22 @@ class GroundlinkEngine:
         self.fc_dropout = fc_dropout
         self.cnn_dropout = float(cnn_dropout)             # nn.Dropout before every Conv1d (Groundlink.py:41, default 0.0)
         self.buf = _Buffers(arena.device)
-        self._wver = None
+        self._w_version = None
         self._w: Dict[str, torch.Tensor] = {}
-        self.step = 0
-        self.cnn_seed, self.fc_seed = self.CNN_DROPOUT_SEED, FC_DROPOUT_SEED     # Trainer.seed_rng folds seed and rank in
-        self.step_dev = None                    # Trainer-owned device step counter: offsets are derived on the device (graph replay)
-        self.bucket_hook = None
+        self.set_rng(0, 0, 0, None)
+        self.bucket_hook = None                 # callable(group) fired when a group's grads are complete: 0-3 = conv layers, 4 = the MLP
+
+    def set_rng(self, seed_mix: int, rank: int, step: int, step_dev: Optional[torch.Tensor]) -> None:
+        """Dropout masks: Philox keyed by (CNN/FC_DROPOUT_SEED ^ seed_mix) + rank, offset by the training-forward count
+        ``step`` — or, when ``step_dev`` (a device-resident step counter) is given, by its value, so that a captured step
+        replays."""
+        self.cnn_seed = (self.CNN_DROPOUT_SEED ^ seed_mix) + rank
+        self.fc_seed = (self.FC_DROPOUT_SEED ^ seed_mix) + rank
+        self.step, self.step_dev = step, step_dev
+
+    def bucket_boundaries(self) -> List[int]:
+        offs = self.arena.offsets
+        return [offs[f"cnn.{p}.weight"][0] for p in self.conv_pos] + [offs[f"fc.{self.fc_pos[0]}.weight"][0]]
 
     def _drop(self, x, y, p, seed, mul, add, step):
         """Philox offset = mul * step + add, the step taken from the device counter when the Trainer owns one."""
@@ -60,9 +70,11 @@ class GroundlinkEngine:
             ops.dropout(x, y, p, seed, mul * step + add)
 
     # ---- weights in GEMM layouts (refreshed when the fp32 masters change) ---------------------------------
-    def _weights(self) -> Dict[str, torch.Tensor]:
-        ver = self.arena._version_sum()
-        if self._wver == ver and self._w:
+    def refresh_weights(self) -> Dict[str, torch.Tensor]:
+        """Re-lays the conv weights out for the GEMMs if the arena's weights version moved.  The copies are updated in place,
+        so a captured step that contains the re-layout keeps reading them."""
+        ver = self.arena.version
+        if self._w_version == ver and self._w:
             return self._w
         dev = self.arena.device
         for i, pos in enumerate(self.conv_pos):
@@ -75,12 +87,8 @@ class GroundlinkEngine:
                 self._w[f"d{i}"] = torch.empty(cin, KT * self.cout_pad[i], dtype=BF16, device=dev)
             ops.conv_weight_to_gemm(w, fw, self.cin_pad[i])
             ops.conv_weight_to_dgrad(w, self._w[f"d{i}"], self.cout_pad[i])
-        self._wver = ver
+        self._w_version = ver
         return self._w
-
-    def weights_changed(self) -> None:
-        """The fused optimizer writes the fp32 masters through raw pointers (no torch version bump): drop the cache."""
-        self._wver = None
 
     # ---- buffers ---------------------------------------------------------------------------------------------
     def _state(self, B: int, T: int):
@@ -105,25 +113,30 @@ class GroundlinkEngine:
             st["slack"] = slack
         return st, Tp, Mp
 
-    def input_rows(self, B: int, T: int) -> Tuple[torch.Tensor, int, int, int]:
+    def input_layout(self, B: int, T: int, train: bool) -> Tuple[torch.Tensor, int, int, int]:
         """(buffer, frame_stride, win_extra, col0) for the packers: frame t of window b → row b*Tp + 3 + t."""
         st, Tp, Mp = self._state(B, T)
         ld = self.ld[0]
         return st["x0"], ld, 2 * self.pad * ld, self.pad * ld
 
-    def out_view(self, B: int, T: int) -> torch.Tensor:
+    def _frames(self, name: str, B: int, T: int) -> torch.Tensor:
         st, Tp, Mp = self._state(B, T)
-        return st["out"].view(B, Tp, 32)[:, self.pad:self.pad + T, :]
+        return st[name].view(B, Tp, 32)[:, self.pad:self.pad + T, :]
 
-    def dout_view(self, B: int, T: int) -> torch.Tensor:
-        st, Tp, Mp = self._state(B, T)
-        return st["dout"].view(B, Tp, 32)[:, self.pad:self.pad + T, :]
+    def dout(self, B: int, T: int) -> torch.Tensor:
+        """(B, T, 32) bf16 view of the output-gradient rows (all other rows stay zero)."""
+        return self._frames("dout", B, T)
+
+    def quantity_views(self, x: torch.Tensor, B: int, T: int, Fo: int) -> List[torch.Tensor]:
+        """(B, Fo, ·) views of the four quantities of a (B, T, 32) output / output-gradient view; Fo = 1 is the last
+        frame, the only output of ``last_frame`` (Groundlink.py:147-148)."""
+        return quantity_split(x[:, T - Fo:])
 
     # ---- forward ---------------------------------------------------------------------------------------------
     def forward(self, B: int, T: int, train: bool) -> torch.Tensor:
-        """Consumes input_rows (frames written at rows b*Tp+3+t); returns the (B, T, 32) fp32 output view."""
+        """Consumes input_layout (frames written at rows b*Tp+3+t); returns the (B, T, 32) fp32 output view."""
         A = self.arena
-        W = self._weights()
+        W = self.refresh_weights()
         st, Tp, Mp = self._state(B, T)
         PAD, KT, depth, C = self.pad, self.kt, self.fc_depth, self.ch[-1]
         self.step += 1
@@ -160,13 +173,13 @@ class GroundlinkEngine:
             else:
                 ops.gemm(a, A.shadow_of(f"fc.{pos}.weight", (30, C)), st["out"], Mp, 30, C)
         st["dropped"] = drop
-        return self.out_view(B, T)
+        return self._frames("out", B, T)
 
     # ---- backward ---------------------------------------------------------------------------------------------
     def backward(self, B: int, T: int) -> None:
-        """Consumes dout (bf16, written through dout_view; all other rows zero); accumulates parameter grads."""
+        """Consumes dout(B, T) (bf16; all other rows zero); accumulates parameter grads."""
         A = self.arena
-        W = self._weights()
+        W = self.refresh_weights()
         g = A.grad_of
         st, Tp, Mp = self._state(B, T)
         drop = st.get("dropped", False)

@@ -17,7 +17,7 @@ import torch.nn as nn
 
 from .. import ops
 from ..engine import DenoiserEngine
-from ..keys import InputDataKeys, MODEL_INPUT_ORDER, OutputDataKeys
+from ..keys import InputDataKeys
 from ._base import EngineModule
 
 
@@ -36,31 +36,22 @@ class _DenoiserFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, B, train, *params):
         eng = model.engine()
-        out = eng.forward(B, train=train)      # train ⇒ keep every layer's activations for backward
+        out = eng.forward(B, eng.F, train)     # train ⇒ keep every layer's activations for backward
         ctx.model, ctx.B = model, B
         return out.clone()
 
     @staticmethod
     def backward(ctx, grad_out):
         model, B = ctx.model, ctx.B
-        eng, arena = model._engine, model._arena
+        eng = model._engine
         M = B * eng.F
-        ops.cast_pad(grad_out.contiguous().view(M, 32), eng.dout(B), M, 30)
-        scratch = arena.scratch_grad()
-        scratch.zero_()
-        arena.grad_target = scratch
-        try:
-            eng.backward(B)
-        finally:
-            arena.grad_target = arena.grad
-        grads = []
-        for i, n in enumerate(arena.names):
-            o, k = arena.offsets[n]
-            grads.append(scratch[o:o + k].view(arena.params[i].shape).clone())
-        return (None, None, None, *grads)
+        ops.cast_pad(grad_out.contiguous().view(M, 32), eng.dout(B, eng.F), M, 30)
+        return (None, None, None, *model._engine_backward(B, eng.F))
 
 
 class DiffusionDenoiser(EngineModule):
+    trains_by_diffusion = True
+
     def __init__(self, num_dofs: int = 23, num_joints: int = 12, root_history_len: int = 10, frames: int = 50,
                  d_model: int = 512, num_heads: int = 8, dim_feedforward: int = 2048, num_layers: int = 8):
         super().__init__()
@@ -90,18 +81,13 @@ class DiffusionDenoiser(EngineModule):
         assert F == self.frames and tuple(input[InputDataKeys.X_T].shape) == (B, F, 30)
         eng = self.engine()
         train = torch.is_grad_enabled()
-        xc = eng.xc(B, train)
-        self._pack_dict(input, xc, F, frame_stride=eng.ld_in, win_extra=0, col0=30)
-        self._pack_dict(input, xc, F, frame_stride=eng.ld_in, win_extra=0, col0=0, keys=(InputDataKeys.X_T,))
+        layout = eng.input_layout(B, F, train)
+        self._pack_dict(input, layout, F)
+        self._pack_dict(input, layout[:3] + (0,), F, keys=(InputDataKeys.X_T,))        # x_t: columns 0..29
         eng.t_buffer(B, train).copy_(input[InputDataKeys.TIMESTEP].to(torch.int32), non_blocking=True)
         return self.forward_packed(B)
 
     def forward_packed(self, B: int) -> Dict[str, torch.Tensor]:
         """Forward from already filled engine buffers xc(B, train), t_buffer(B, train) (window-store fast path)."""
-        x = _DenoiserFunction.apply(self, B, torch.is_grad_enabled(), *self.parameters()).view(B, self.frames, 32)
-        return {
-            OutputDataKeys.GROUND_CONTACT_COPS_IN_ROOT_FRAME: x[:, :, 0:6],
-            OutputDataKeys.GROUND_CONTACT_FORCES_IN_ROOT_FRAME: x[:, :, 6:12],
-            OutputDataKeys.GROUND_CONTACT_TORQUES_IN_ROOT_FRAME: x[:, :, 12:18],
-            OutputDataKeys.GROUND_CONTACT_WRENCHES_IN_ROOT_FRAME: x[:, :, 18:30],
-        }
+        F = self.frames
+        return self._quantities(_DenoiserFunction.apply(self, B, torch.is_grad_enabled(), *self.parameters()), B, F, F)

@@ -16,7 +16,7 @@ import torch.nn as nn
 
 from .. import ops
 from ..engine import FeedForwardEngine
-from ..keys import InputDataKeys, OutputDataKeys
+from ..keys import InputDataKeys
 from ._base import EngineModule
 
 ACTIVATION_FUNCS = {"relu": nn.ReLU(), "tanh": nn.Tanh(), "sigmoid": nn.Sigmoid()}
@@ -27,30 +27,18 @@ class _FeedForwardFunction(torch.autograd.Function):
     only so autograd (and DDP's hooks) see them."""
 
     @staticmethod
-    def forward(ctx, model, B, *params):
+    def forward(ctx, model, B, F, *params):
         eng = model.engine()
-        out = eng.forward(B, train=model.training)
-        ctx.model, ctx.B = model, B
+        out = eng.forward(B, F, model.training)
+        ctx.model, ctx.B, ctx.F = model, B, F
         return out[:, :eng.out_cols].clone()
 
     @staticmethod
     def backward(ctx, grad_out):
-        model, B = ctx.model, ctx.B
-        eng, arena = model._engine, model._arena
-        dout = eng.dout_buffer(B)
-        ops.cast_pad(grad_out.contiguous(), dout, B, eng.out_cols)
-        scratch = arena.scratch_grad()
-        scratch.zero_()
-        arena.grad_target = scratch
-        try:
-            eng.backward(B)
-        finally:
-            arena.grad_target = arena.grad
-        grads = []
-        for n in arena.names:
-            o, k = arena.offsets[n]
-            grads.append(scratch[o:o + k].view(arena.params[len(grads)].shape).clone())
-        return (None, None, *grads)
+        model, B, F = ctx.model, ctx.B, ctx.F
+        eng = model._engine
+        ops.cast_pad(grad_out.contiguous(), eng.dout(B, F), B, eng.out_cols)
+        return (None, None, None, *model._engine_backward(B, F))
 
 
 class FeedForwardBaseline(EngineModule):
@@ -115,7 +103,8 @@ class FeedForwardBaseline(EngineModule):
         # [Dropout][BatchNorm1d] sit on each Linear's input (FeedForward…py:68-72): BatchNorm1d over the packed bf16 rows
         # (ibm_batchnorm_fwd/bwd, batch statistics when self.training), Philox inverted dropout (ibm_dropout_bf16)
         bn = [(f"net.{p}.weight", f"net.{p}.bias", self.net[p]) for p in self._bn_pos] if self.batchnorm else None
-        return FeedForwardEngine(arena, layers, self.activation, bn=bn, dropout_p=self.dropout_prob if self.dropout else 0.0)
+        return FeedForwardEngine(arena, layers, self.activation, self.frame_width, bn=bn,
+                                 dropout_p=self.dropout_prob if self.dropout else 0.0)
 
     def forward(self, input: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
         # 1. same shape assertions as the reference (FeedForward…py:83-94)
@@ -134,25 +123,13 @@ class FeedForwardBaseline(EngineModule):
         assert F * self.frame_width == self.input_size, "window length does not match history_len // stride"
         if self._latency_path(B):
             # batch-of-1 viewers (visualize.py:181, save_prediction_csv.py:103): pack + 3 GEMMs replayed from one CUDA graph
-            def launch(rows):
-                ops.pack_inputs([rows], B * F, F, out_bf16=eng.input_buffer(B), frame_stride=self.frame_width,
-                                win_extra=eng.in_ld - self.input_size, col0=0)
-                return eng.forward(B, train=False)
-            return self._split(self._graphed_inference(input, F, launch)[:, :eng.out_cols], B)
+            return self._quantities(self._graphed_inference(input, F)[:, :eng.out_cols], B, F, self.num_output_frames)
         # 2. concat + flatten + bf16 in one kernel (row-per-window layout, K padded to a multiple of 8)
-        self._pack_dict(input, eng.input_buffer(B), F, frame_stride=self.frame_width, win_extra=eng.in_ld - self.input_size, col0=0)
+        self._pack_dict(input, eng.input_layout(B, F, self.training), F)
         return self.forward_packed(B)
 
     def forward_packed(self, B: int) -> Dict[str, torch.Tensor]:
-        """Forward from an already packed engine.input_buffer(B) (the window-store fast path)."""
-        return self._split(_FeedForwardFunction.apply(self, B, *self.parameters()), B)
-
-    def _split(self, x: torch.Tensor, B: int) -> Dict[str, torch.Tensor]:
-        Fo = self.num_output_frames
-        # 4. quantity-then-frame blocks (FeedForward…py:116-121)
-        return {
-            OutputDataKeys.GROUND_CONTACT_COPS_IN_ROOT_FRAME: x[:, 0 * Fo:6 * Fo].reshape((B, Fo, 6)),
-            OutputDataKeys.GROUND_CONTACT_FORCES_IN_ROOT_FRAME: x[:, 6 * Fo:12 * Fo].reshape((B, Fo, 6)),
-            OutputDataKeys.GROUND_CONTACT_TORQUES_IN_ROOT_FRAME: x[:, 12 * Fo:18 * Fo].reshape((B, Fo, 6)),
-            OutputDataKeys.GROUND_CONTACT_WRENCHES_IN_ROOT_FRAME: x[:, 18 * Fo:30 * Fo].reshape((B, Fo, 12)),
-        }
+        """Forward from an already packed engine.input_buffer(B) (the window-store fast path); quantity-then-frame blocks
+        of the output row (FeedForward…py:116-121)."""
+        F = self.num_frames
+        return self._quantities(_FeedForwardFunction.apply(self, B, F, *self.parameters()), B, F, self.num_output_frames)

@@ -14,9 +14,8 @@ from typing import Dict
 import torch
 import torch.nn as nn
 
-from .. import ops
 from ..engine_groundlink import GroundlinkEngine
-from ..keys import InputDataKeys, OutputDataKeys
+from ..keys import InputDataKeys
 from ._base import EngineModule
 
 
@@ -43,21 +42,9 @@ class _GroundlinkFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out):
         model, B, T = ctx.model, ctx.B, ctx.T
-        eng, arena = model._engine, model._arena
-        dv = eng.dout_view(B, T)
+        dv = model._engine.dout(B, T)
         dv[:, :, :30] = grad_out[:, :, :30].to(torch.bfloat16)          # strided write into the padded-row gradient buffer
-        scratch = arena.scratch_grad()
-        scratch.zero_()
-        arena.grad_target = scratch
-        try:
-            eng.backward(B, T)
-        finally:
-            arena.grad_target = arena.grad
-        grads = []
-        for i, n in enumerate(arena.names):
-            o, k = arena.offsets[n]
-            grads.append(scratch[o:o + k].view(arena.params[i].shape).clone())
-        return (None, None, None, None, *grads)
+        return (None, None, None, None, *model._engine_backward(B, T))
 
 
 class Groundlink(EngineModule):
@@ -128,26 +115,16 @@ class Groundlink(EngineModule):
         assert input[InputDataKeys.ROOT_EULER_HISTORY_IN_ROOT_FRAME].shape[-1] == self.root_history_len * 3
         eng = self.engine()
         B, T = input[InputDataKeys.POS].shape[0], input[InputDataKeys.POS].shape[1]
-        buf, fs, we, col0 = eng.input_rows(B, T)
         if self._latency_path(B):
             # batch-of-1 viewers: packer + 4 implicit-GEMM convolutions + pad refreshes + MLP replayed from one CUDA graph
-            def launch(rows):
-                ops.pack_inputs([rows], B * T, T, out_bf16=buf, frame_stride=fs, win_extra=we, col0=col0)
-                return eng.forward(B, T, False)
-            return self._split(self._graphed_inference(input, T, launch))
+            return self._quantities(self._graphed_inference(input, T), B, T, self._output_frames(T))
         # 2. concat → bf16 rows in the padded-row layout (frame t of window b at row b*(T+6) + 3 + t)
-        self._pack_dict(input, buf, T, frame_stride=fs, win_extra=we, col0=col0)
+        self._pack_dict(input, eng.input_layout(B, T, self.training), T)
         return self.forward_packed(B, T)
 
     def forward_packed(self, B: int, T: int) -> Dict[str, torch.Tensor]:
-        return self._split(_GroundlinkFunction.apply(self, B, T, self.training and torch.is_grad_enabled(), *self.parameters()))
+        out = _GroundlinkFunction.apply(self, B, T, self.training and torch.is_grad_enabled(), *self.parameters())
+        return self._quantities(out, B, T, self._output_frames(T))
 
-    def _split(self, x: torch.Tensor) -> Dict[str, torch.Tensor]:
-        if self.output_data_format != 'all_frames':
-            x = x[:, -1:, :]                       # Groundlink.py:147-148: only the last frame goes through the MLP
-        return {
-            OutputDataKeys.GROUND_CONTACT_COPS_IN_ROOT_FRAME: x[:, :, 0:6],
-            OutputDataKeys.GROUND_CONTACT_FORCES_IN_ROOT_FRAME: x[:, :, 6:12],
-            OutputDataKeys.GROUND_CONTACT_TORQUES_IN_ROOT_FRAME: x[:, :, 12:18],
-            OutputDataKeys.GROUND_CONTACT_WRENCHES_IN_ROOT_FRAME: x[:, :, 18:30],
-        }
+    def _output_frames(self, T: int) -> int:
+        return T if self.output_data_format == 'all_frames' else 1      # Groundlink.py:147-148: last_frame keeps the last one

@@ -7,7 +7,7 @@ import torch
 import torch.nn as nn
 
 from .. import _lib, ops
-from ..keys import MODEL_INPUT_ORDER
+from ..keys import LOSS_QUANTITIES, MODEL_INPUT_ORDER
 from ..params import ParamArena
 
 
@@ -15,6 +15,7 @@ class EngineModule(nn.Module):
     """nn.Module whose parameters are views into a flat HBM arena read by libibm_b200 kernels."""
 
     LATENCY_BATCH = 16      # inference batches up to this size replay a captured CUDA graph (the viewers' batch-of-1 path)
+    trains_by_diffusion = False     # True: the Trainer's step feeds noised labels and timesteps (GaussianDiffusion.q_sample)
 
     def _init_engine_state(self):
         self._arena: Optional[ParamArena] = None
@@ -41,9 +42,7 @@ class EngineModule(nn.Module):
             # module loop (the reference's autograd + DDP idiom): every data-parallel rank draws its own dropout masks, as
             # per-process torch RNGs do; the native Trainer re-seeds with its own seed and step count (Trainer.seed_rng)
             from ..parallel import world
-            for attr in ("dropout_seed", "cnn_seed", "fc_seed"):
-                if hasattr(self._engine, attr):
-                    setattr(self._engine, attr, getattr(self._engine, attr) + world()[0])
+            self._engine.set_rng(0, world()[0], 0, None)
         else:
             self._arena.sync_shadow()
         return self._engine
@@ -53,12 +52,34 @@ class EngineModule(nn.Module):
         self.engine()
         return self._arena
 
+    # ---- engine backward for the autograd bridges ------------------------------------------------------
+    def _engine_backward(self, B: int, F: int) -> tuple:
+        """Runs the engine backward (its dout already written) into the scratch gradient arena, leaving the ``.grad`` arena
+        alone, and returns one gradient per parameter for autograd."""
+        arena = self._arena
+        scratch = arena.scratch_grad()
+        scratch.zero_()
+        arena.grad_target = scratch
+        try:
+            self._engine.backward(B, F)
+        finally:
+            arena.grad_target = arena.grad
+        grads = []
+        for n, p in zip(arena.names, arena.params):
+            o, k = arena.offsets[n]
+            grads.append(scratch[o:o + k].view(p.shape).clone())
+        return tuple(grads)
+
+    def _quantities(self, x: torch.Tensor, B: int, F: int, Fo: int) -> Dict[str, torch.Tensor]:
+        """The output dict of an engine output (or a clone of one): the four quantities of the last Fo frames."""
+        return dict(zip(LOSS_QUANTITIES, self._engine.quantity_views(x, B, F, Fo)))
+
     # ---- dict → packed bf16 rows ---------------------------------------------------------------
-    def _pack_dict(self, input: Dict[str, torch.Tensor], dst_bf16: torch.Tensor, F: int, frame_stride: int, win_extra: int,
-                   col0: int, keys: Sequence[str] = MODEL_INPUT_ORDER) -> None:
+    def _pack_dict(self, input: Dict[str, torch.Tensor], layout, F: int, keys: Sequence[str] = MODEL_INPUT_ORDER) -> None:
         """torch.concat([...10 keys...], -1) of the reference (FeedForward…py:97-108), as one kernel
-        writing bf16 rows.  CPU tensors are concatenated into one pinned staging buffer and moved with a
-        single H2D copy (the reference issues one copy per forward too, after its concat)."""
+        writing bf16 rows into ``layout`` (an engine's ``input_layout``).  CPU tensors are concatenated into one pinned
+        staging buffer and moved with a single H2D copy (the reference issues one copy per forward too, after its concat)."""
+        dst_bf16, frame_stride, win_extra, col0 = layout
         dev = dst_bf16.device
         ts = [input[k] for k in keys]
         B = ts[0].shape[0]
@@ -86,17 +107,23 @@ class EngineModule(nn.Module):
         return (not torch.is_grad_enabled() and not self.training and B <= self.LATENCY_BATCH
                 and os.environ.get("IBM_INFER_GRAPHS", "1") != "0")
 
-    def _graphed_inference(self, input: Dict[str, torch.Tensor], F: int, launch, keys: Sequence[str] = MODEL_INPUT_ORDER) -> torch.Tensor:
-        """``launch(rows)``: packs ``rows`` (device fp32 [B*F, C], the concat of the input keys) and runs the engine forward,
-        returning the engine's output buffer.  The first two calls per (batch, frames) run eagerly (every lazily created buffer
-        exists afterwards), the third captures, later ones copy the inputs into the static staging rows and replay.  Weights are
-        read through the arena's stable pointers; ``engine()`` has already refreshed the bf16 shadow if a parameter changed."""
+    def _graphed_inference(self, input: Dict[str, torch.Tensor], F: int, keys: Sequence[str] = MODEL_INPUT_ORDER) -> torch.Tensor:
+        """Packs the inputs into the engine's input layout and runs the inference forward, returning a clone of the engine's
+        output.  The first two calls per (batch, frames) run eagerly (every lazily created buffer exists afterwards), the
+        third captures, later ones copy the inputs into the static staging rows and replay.  Weights are read through the
+        arena's stable pointers; ``engine()`` has already refreshed the bf16 shadow if a parameter changed."""
         eng = self._engine
         dev = self._arena.device
         ts = [input[k] for k in keys]
         B = ts[0].shape[0]
         n_rows = B * F
         C = sum(t.shape[-1] for t in ts)
+
+        def launch(rows):
+            buf, fs, we, col0 = eng.input_layout(B, F, False)
+            ops.pack_inputs([rows], n_rows, F, out_bf16=buf, frame_stride=fs, win_extra=we, col0=col0)
+            return eng.forward(B, F, False)
+
         key = (B, F, C, id(eng))
         st = self._lat.get(key)
         if st is None:
@@ -119,7 +146,6 @@ class EngineModule(nn.Module):
             with torch.cuda.graph(g):
                 st["out"] = launch(st["rows"])
             st["graph"] = g
-        if hasattr(eng, "_weights"):
-            eng._weights()                  # engines with re-laid-out weight copies refresh them outside the graph (version check)
+        eng.refresh_weights()               # re-laid-out weight copies are refreshed outside the graph
         st["graph"].replay()
         return st["out"].clone()

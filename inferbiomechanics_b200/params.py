@@ -47,6 +47,7 @@ class ParamArena:
                 p.grad = self.grad[o:o + k].view(p.shape)
         self._ptrs = [p.data_ptr() for p in self.params]
         self._versions: Optional[int] = None
+        self._device_writes = 0
         self.padded: Dict[str, torch.Tensor] = {}      # bf16 copies with ld rounded up to 8 for odd-K weights
         self.sync_shadow(force=True)
 
@@ -57,6 +58,17 @@ class ParamArena:
 
     def _version_sum(self) -> int:
         return sum(p._version for p in self.params)
+
+    @property
+    def version(self) -> int:
+        """Changes whenever the fp32 masters may have changed: torch's in-place writes (each parameter's ``_version``) plus
+        device-side writes (``bump_version``).  Caches of weights derived from the masters key on it."""
+        return self._version_sum() + self._device_writes
+
+    def bump_version(self) -> None:
+        """Records a write of the masters that torch does not see: the fused optimizer writes them through raw pointers,
+        eagerly or from a replayed CUDA graph."""
+        self._device_writes += 1
 
     # -- views ----------------------------------------------------------------------------------
     def shadow_of(self, name: str, shape=None) -> torch.Tensor:
@@ -108,9 +120,10 @@ class ParamArena:
             ops.cast_pad(self.master[o:o + k].view(rows, k // rows), buf, rows, k // rows)
 
     def mark_shadow_fresh(self) -> None:
-        """Called after the fused optimizer kernel (which writes the shadow itself)."""
+        """Called after the fused optimizer kernel (which writes the masters and the shadow itself)."""
         self.refresh_padded()
         self._versions = self._version_sum()
+        self.bump_version()
 
     def zero_grad(self) -> None:
         self.grad.zero_()

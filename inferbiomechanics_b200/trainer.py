@@ -10,8 +10,9 @@
     backward engine → flat fp32 grad arena       (bucketed NCCL allreduce fired layer by layer)
     fused optimizer → params + state + bf16 shadow (1 kernel, 1/W folded in)
 
-Works for ``FeedForwardBaseline``, ``Groundlink`` and ``DiffusionDenoiser``.  The drop-in classes remain usable with
-the reference's own autograd loop; this is the path bench.py times.
+Works for ``FeedForwardBaseline``, ``Groundlink`` and ``DiffusionDenoiser`` through their engines' common step interface
+(``input_layout``, ``forward``, ``dout``, ``quantity_views``, ``backward``, ``bucket_boundaries``, ``set_rng``).  The
+drop-in classes remain usable with the reference's own autograd loop; this is the path bench.py times.
 """
 from __future__ import annotations
 
@@ -25,26 +26,33 @@ import torch
 from . import ops, parallel
 from .data.window_store import WindowStore
 from .diffusion import GaussianDiffusion
-from .keys import LOSS_QUANTITIES
+from .engine import quantity_split
+from .keys import LOSS_QUANTITIES, MODEL_INPUT_ORDER
 from .loss.RegressionLossEvaluator import COP_FORCE_THRESHOLD, component_weights
-from .models.DiffusionDenoiser import DiffusionDenoiser
-from .models.FeedForwardRegressionBaseline import FeedForwardBaseline
-from .models.Groundlink import Groundlink
 
 ALL_COMPONENTS = argparse.Namespace(predict_grf_components=list(range(6)), predict_cop_components=list(range(6)),
                                     predict_moment_components=list(range(6)), predict_wrench_components=list(range(12)))
 
 
-def _views30(rows: torch.Tensor):
-    """(B,F,>=30) rows30 tensor → the four quantity views (cop, force, torque, wrench)."""
-    return [rows[:, :, 0:6], rows[:, :, 6:12], rows[:, :, 12:18], rows[:, :, 18:30]]
-
-
-def _views_ff(x: torch.Tensor, B: int, Fo: int):
-    """FeedForward output/grad layout (FeedForward…py:116-121): quantity-then-frame blocks of a [B, >=30*Fo] row."""
-    def blk(a, b, c):
-        return x[:, a * Fo:b * Fo].unflatten(1, (Fo, c))
-    return [blk(0, 6, 6), blk(6, 12, 6), blk(12, 18, 6), blk(18, 30, 12)]
+def _time_kernel(fn, iters: int = 20) -> float:
+    """Average GPU time of one launch: `iters` launches are captured in a CUDA graph and the replay is timed with
+    events, so host-side launch overhead (ctypes marshalling is ~50-100 us per call, longer than these kernels)
+    is not part of the number."""
+    for _ in range(3):
+        fn()
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        for _ in range(iters):
+            fn()
+    g.replay()                                   # warm replay
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.synchronize()
+    e0.record()
+    g.replay()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / iters
 
 
 class Trainer:
@@ -58,32 +66,24 @@ class Trainer:
         self.rank, self.world = parallel.world()
         self.step_count = 0
         self.seed = seed
-        self.is_denoiser = isinstance(model, DiffusionDenoiser)
-        self.is_groundlink = isinstance(model, Groundlink)
-        if self.is_denoiser:
-            self.diffusion = diffusion or GaussianDiffusion(device=self.arena.device)
+        # diffusion training (the denoiser): noised labels as input, no graph capture, overlapped allreduce buckets
+        self.diffusion = (diffusion or GaussianDiffusion(device=self.arena.device)) if model.trains_by_diffusion else None
         n = self.arena.total
         dev = self.arena.device
         self.state0 = torch.zeros(n, device=dev) if opt_type != "sgd" else None
         self.state1 = torch.zeros(n, device=dev) if opt_type in ("adam", "adadelta", "adamax") else None
         self.results: List[torch.Tensor] = []              # fp32[40] per step, device-resident
         self._result_ring = [torch.zeros(40, device=dev) for _ in range(8)]
-        # layer groups for the bucketed allreduce
-        bounds = self._group_boundaries()
         bucket_mb = float(os.environ.get("IBM_BUCKET_MB", bucket_mb))      # experiments: bucket size of the gradient allreduce
         # FeedForward / Groundlink gradients are a few MB: one allreduce of the whole arena after backward ("tail") costs less
         # than a bucket per layer group (0.46 vs 0.51 ms per B = 32 step on 2 GPUs) and leaves one point in the step where a
         # captured step is cut in two (see _train_step_graphed).  The denoiser keeps the overlapped buckets unless IBM_ALLREDUCE says otherwise.
         self.use_graphs = os.environ.get("IBM_TRAIN_GRAPHS", "1") != "0"
-        self.dp_graphs = self.use_graphs and not self.is_denoiser and os.environ.get("IBM_TRAIN_GRAPHS_DP", "1") != "0"
-        self.bucketer = parallel.GradBucketer(self.arena.grad, parallel.make_buckets(bounds, n, int(bucket_mb * (1 << 20) / 4)),
-                                              mode=None if self.is_denoiser else os.environ.get("IBM_ALLREDUCE", "tail"))
-        if self.is_denoiser:
-            self.eng.bucket_hook = lambda l: self.bucketer.group_done(l + 1)      # group 0 = stem, l+1 = layer l, L+1 = head
-        elif self.is_groundlink:
-            self.eng.bucket_hook = lambda i: self.bucketer.group_done(i)          # groups 0-3 = conv layers, 4 = the per-frame MLP
-        else:
-            self.eng.bucket_hook = lambda i: self.bucketer.group_done(i)          # group i = Linear layer i
+        self.dp_graphs = self.use_graphs and self.diffusion is None and os.environ.get("IBM_TRAIN_GRAPHS_DP", "1") != "0"
+        buckets = parallel.make_buckets(self.eng.bucket_boundaries(), n, int(bucket_mb * (1 << 20) / 4))
+        self.bucketer = parallel.GradBucketer(self.arena.grad, buckets,
+                                              mode=None if self.diffusion is not None else os.environ.get("IBM_ALLREDUCE", "tail"))
+        self.eng.bucket_hook = self.bucketer.group_done
         # DDP constructor semantics: everyone starts from rank 0's parameters (train.py:175)
         self.bucketer.broadcast_(self.arena.master)
         self.arena.sync_shadow(force=True)
@@ -91,10 +91,10 @@ class Trainer:
         # dropout kernels (Philox offset) and the optimizer kernel (Adam / Adamax bias correction), so that a captured step
         # can be replayed although those values change from step to step
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=dev)
-        if hasattr(self.eng, "step_dev"):
-            self.eng.step_dev = self.step_dev
         self.seed_rng()
-        self._lab: Dict[int, torch.Tensor] = {}
+        self._store_labels: Dict[int, torch.Tensor] = {}       # batch size -> (B, Fo, 30) labels packed from a window store
+        self._host_stage: Dict[tuple, tuple] = {}              # (batch size, slot) -> (device staging tensors, ready, consumed)
+        self._host_labels: Dict[int, torch.Tensor] = {}        # batch size -> (B, Fo, 30) labels packed from host batches
         self._gen = torch.Generator(device=dev).manual_seed(seed + 7919 * self.rank)
         # CUDA-graph replay of the (launch-bound) FeedForward step: key -> [eager steps seen, graph, static idx, static result]
         self._graphs: Dict[tuple, list] = {}
@@ -103,25 +103,8 @@ class Trainer:
         """Dropout masks: Philox keyed by (engine constant ^ trainer seed) + rank, offset by the GLOBAL step count — every
         data-parallel rank draws its own mask (the reference's per-process torch RNG does), and a resumed run continues the
         sequence instead of replaying the masks of step 1."""
-        eng, mix = self.eng, (self.seed * 0x9E3779B1) & 0x7FFFFFFF
-        for attr in ("dropout_seed", "cnn_seed", "fc_seed"):
-            if hasattr(eng, attr):
-                base = {"dropout_seed": getattr(eng, "DROPOUT_SEED", 0), "cnn_seed": getattr(eng, "CNN_DROPOUT_SEED", 0),
-                        "fc_seed": 0x6c696e6b}[attr]
-                setattr(eng, attr, (base ^ mix) + self.rank)
-        if hasattr(eng, "step"):
-            eng.step = self.step_count
+        self.eng.set_rng((self.seed * 0x9E3779B1) & 0x7FFFFFFF, self.rank, self.step_count, self.step_dev)
         self.step_dev.fill_(self.step_count)
-
-    def _group_boundaries(self) -> List[int]:
-        offs = self.arena.offsets
-        if self.is_denoiser:
-            first = [offs[f"layers.{l}.multihead_attention.in_proj_weight"][0] for l in range(self.model.num_layers)]
-            return [0] + first + [offs["out_proj.weight"][0]]
-        if self.is_groundlink:
-            return [offs[f"cnn.{p}.weight"][0] for p in self.eng.conv_pos] + [offs[f"fc.{self.eng.fc_pos[0]}.weight"][0]]
-        bn = getattr(self.eng, "bn", None)        # a layer's BatchNorm parameters precede its Linear in the arena
-        return [offs[bn[i][0] if bn is not None and bn[i] is not None else w][0] for i, (w, _, _, _) in enumerate(self.eng.layers)]
 
     # ---- one optimisation step on windows idx of a store -------------------------------------------
     def _graphable(self) -> bool:
@@ -133,7 +116,7 @@ class Trainer:
         collective on the capture stream — so NCCL is kept out of the graphs).  Not captured: the denoiser (its step is
         GPU-bound and draws timesteps with a torch generator).  IBM_TRAIN_GRAPHS=0 switches replay off altogether,
         IBM_TRAIN_GRAPHS_DP=0 for data-parallel runs only."""
-        if not self.use_graphs or self.is_denoiser:
+        if not self.use_graphs or self.diffusion is not None:
             return False
         return self.world == 1 or (self.dp_graphs and self.bucketer.mode == "tail")
 
@@ -165,6 +148,9 @@ class Trainer:
             graphs.append(nxt)
 
         self.bucketer.finish_hook = cut if self.world > 1 else None
+        # the replays must re-derive cached weight layouts (Groundlink's conv GEMM layouts) from the masters the previous
+        # step wrote: a stale weights version makes the captured forward record that refresh
+        self.arena.bump_version()
         try:
             with torch.cuda.stream(side):
                 graphs[0].capture_begin(capture_error_mode=mode)
@@ -200,8 +186,7 @@ class Trainer:
             finally:
                 self._result_ring = ring
             self.step_count = count              # capture does not execute: the replay below is this step
-            if hasattr(self.eng, "step"):
-                self.eng.step = count
+            self.seed_rng()
             g[1] = graphs
         g[2].copy_(idx, non_blocking=True)
         g[1][0].replay()
@@ -209,44 +194,55 @@ class Trainer:
             self.bucketer.allreduce_all()
             graph.replay()
         self.step_count += 1
-        self.arena._versions = self.arena._version_sum()
+        self.arena.bump_version()                # the replayed optimizer wrote the masters
         result = self._result_ring[self.step_count % len(self._result_ring)]
         result.copy_(g[3], non_blocking=True)
         return result
 
     def _train_step_eager(self, store: WindowStore, idx: torch.Tensor) -> torch.Tensor:
-        B = idx.numel()
+        B, F = idx.numel(), store.F
         lab = self._labels(store, idx)
         self._begin_step()
-        if self.is_denoiser:
-            store.pack_rows(idx, self.eng.xc(B, True), col0=30)
-            return self._finish_denoiser_step(B, lab)
-        if self.is_groundlink:
-            buf, fs, we, col0 = self.eng.input_rows(B, store.F)         # padded-row layout: frame t of window b at row b*(T+6)+3+t
-            ops.pack_windows(store.frames, store.C, store.win_row0[idx], store.F, store.stride, out_bf16=buf, frame_stride=fs,
-                             win_extra=we, col0=col0)
-            return self._finish_groundlink_step(B, store.F, lab)
-        store.pack_feedforward(idx, self.eng.input_buffer(B))
-        return self._finish_ff_step(B, lab)
+        store.pack(idx, self.eng.input_layout(B, F, True))
+        return self._step(B, F, lab)
 
     def _labels(self, store: WindowStore, idx: torch.Tensor) -> torch.Tensor:
         B = idx.numel()
-        if B not in self._lab:
-            self._lab[B] = torch.empty(B, store.Fo, 30, dtype=torch.float32, device=self.arena.device)
-        return store.labels(idx, self._lab[B])
+        if B not in self._store_labels:
+            self._store_labels[B] = torch.empty(B, store.Fo, 30, dtype=torch.float32, device=self.arena.device)
+        return store.labels(idx, self._store_labels[B])
 
     def _begin_step(self) -> None:
         self.arena.zero_grad()
         self.bucketer.begin_step()
         ops.counter_add(self.step_dev, 1)        # the step that starts now: value step_count + 1 on the device
 
+    def _step(self, B: int, F: int, lab: torch.Tensor) -> torch.Tensor:
+        """The step after packing: forward, fused loss forward / backward on the (B, Fo, ·) quantity views of the output and
+        of its gradient, backward into the flat gradient arena, allreduce, fused optimizer."""
+        eng = self.eng
+        if self.diffusion is not None:
+            # x_t = q_sample(labels, t) into columns 0..29 of the input rows, t drawn per window
+            t = eng.t_buffer(B, True)
+            t.copy_(torch.randint(0, self.diffusion.T, (B,), device=t.device, generator=self._gen, dtype=torch.int32))
+            xc, ld, _, _ = eng.input_layout(B, F, True)
+            self.diffusion.q_sample(lab.view(B, -1), t, None, xt_bf16=xc, bf16_ld=ld, seed=self.seed + self.rank, offset=self.step_count)
+        Fo = lab.shape[1]
+        outs = eng.quantity_views(eng.forward(B, F, True), B, F, Fo)
+        labs, gviews = quantity_split(lab), eng.quantity_views(eng.dout(B, F), B, F, Fo)
+        result = self._result_ring[self.step_count % len(self._result_ring)]
+        ops.regression_loss_fwd(outs, labs, self.weights, COP_FORCE_THRESHOLD, result=result)
+        ops.regression_loss_bwd(outs, labs, self.weights, gviews, threshold=COP_FORCE_THRESHOLD)
+        eng.backward(B, F)
+        self.bucketer.finish()
+        self.optimizer_step()
+        return result
+
     def optimizer_step(self) -> None:
         self.step_count += 1
         ops.optimizer_step(self.opt_type, self.arena.master, self.arena.grad, self.state0, self.state1, self.arena.shadow,
                            self.lr, 1.0 / self.world, self.step_count, step_dev=self.step_dev)
         self.arena.mark_shadow_fresh()
-        if hasattr(self.eng, "weights_changed"):
-            self.eng.weights_changed()           # engines that cache re-laid-out weights (Groundlink's conv GEMM layouts)
 
     # ---- optimizer state in torch.optim's own state_dict layout (checkpoints, train.py:270-278) -----------------------
     _OPT_CLASS = {"adagrad": "Adagrad", "adam": "Adam", "sgd": "SGD", "rmsprop": "RMSprop", "adadelta": "Adadelta", "adamax": "Adamax"}
@@ -320,364 +316,228 @@ class Trainer:
     # ---- evaluation (no_grad forward + loss), used by analyze / dev-eval ------------------------------
     @torch.no_grad()
     def eval_step(self, store: WindowStore, idx: torch.Tensor) -> torch.Tensor:
-        B = idx.numel()
-        lab = self._labels(store, idx)
-        if self.is_denoiser:
+        if self.diffusion is not None:
             raise NotImplementedError("denoiser evaluation = reverse sampling; use GaussianDiffusion.sample")
-        if self.is_groundlink:
-            T = store.F
-            buf, fs, we, col0 = self.eng.input_rows(B, T)
-            ops.pack_windows(store.frames, store.C, store.win_row0[idx], store.F, store.stride, out_bf16=buf, frame_stride=fs,
-                             win_extra=we, col0=col0)
-            out = self.eng.forward(B, T, False)
-            if store.Fo == 1:
-                out = out[:, -1:, :]
-            return ops.regression_loss_fwd(_views30(out), _views30(lab), self.weights)
-        store.pack_feedforward(idx, self.eng.input_buffer(B))
-        out = self.eng.forward(B)
-        return ops.regression_loss_fwd(_views_ff(out, B, self.model.num_output_frames), _views30(lab), self.weights)
+        B, F = idx.numel(), store.F
+        lab = self._labels(store, idx)
+        store.pack(idx, self.eng.input_layout(B, F, False))
+        out = self.eng.forward(B, F, False)
+        return ops.regression_loss_fwd(self.eng.quantity_views(out, B, F, store.Fo), quantity_split(lab), self.weights)
 
+    # ---- host-fed step (the e2e path) ----------------------------------------------------------------------------
+    def make_host_batch(self, B: int, seed: int = 0, frames: Optional[int] = None):
+        """Synthetic pinned host tensors shaped like a reference DataLoader batch (SURVEY §8d)."""
+        m = self.model
+        g = torch.Generator().manual_seed(seed)
+        # window length, root-history columns and output frames of the model family: FeedForward has num_frames and a
+        # stride-long history, the denoiser a fixed frame count, Groundlink windows of any length (frames=T)
+        F = frames if frames is not None else getattr(m, "num_frames", getattr(m, "frames", None))
+        if F is None:
+            raise ValueError("Groundlink windows have no fixed length: pass frames=T")
+        hist = 3 * getattr(m, "stride", m.root_history_len)
+        Fo = F if getattr(m, "output_data_format", "all_frames") == "all_frames" else 1
+        widths = {"pos": 23, "vel": 23, "acc": 23, "rootLinearVelInRootFrame": 3, "rootAngularVelInRootFrame": 3,
+                  "rootLinearAccInRootFrame": 3, "rootAngularAccInRootFrame": 3, "jointCentersInRootFrame": 36,
+                  "rootPosHistoryInRootFrame": hist, "rootEulerHistoryInRootFrame": hist}
+        inputs = {k: torch.randn(B, F, widths[k], generator=g).pin_memory() for k in MODEL_INPUT_ORDER}
+        scale = {LOSS_QUANTITIES[0]: 1.0, LOSS_QUANTITIES[1]: 10.0, LOSS_QUANTITIES[2]: 1.0, LOSS_QUANTITIES[3]: 1.0}
+        labels = {k: (torch.randn(B, Fo, 12 if i == 3 else 6, generator=g) * scale[k]).pin_memory() for i, k in enumerate(LOSS_QUANTITIES)}
+        return {"inputs": inputs, "labels": labels}
 
-# =====================================================================================================
-# Host-fed step (the e2e path), profiling helpers used by bench.py
-# =====================================================================================================
-def _make_host_batch(self, B: int, seed: int = 0, frames: Optional[int] = None):
-    """Synthetic pinned host tensors shaped like a reference DataLoader batch (SURVEY §8d)."""
-    from .keys import MODEL_INPUT_ORDER
-    g = torch.Generator().manual_seed(seed)
-    if self.is_groundlink and frames is None:
-        raise ValueError("Groundlink windows have no fixed length: pass frames=T")
-    F = frames if frames is not None else (self.eng.F if self.is_denoiser else self.model.num_frames)
-    hist = self.model.root_history_len * 3 if (self.is_denoiser or self.is_groundlink) else self.model.stride * 3
-    widths = {"pos": 23, "vel": 23, "acc": 23, "rootLinearVelInRootFrame": 3, "rootAngularVelInRootFrame": 3,
-              "rootLinearAccInRootFrame": 3, "rootAngularAccInRootFrame": 3, "jointCentersInRootFrame": 36,
-              "rootPosHistoryInRootFrame": hist, "rootEulerHistoryInRootFrame": hist}
-    inputs = {k: torch.randn(B, F, widths[k], generator=g).pin_memory() for k in MODEL_INPUT_ORDER}
-    Fo = F if self.is_denoiser else (1 if self.is_groundlink and self.model.output_data_format != "all_frames" else
-                                     F if self.is_groundlink else self.model.num_output_frames)
-    scale = {LOSS_QUANTITIES[0]: 1.0, LOSS_QUANTITIES[1]: 10.0, LOSS_QUANTITIES[2]: 1.0, LOSS_QUANTITIES[3]: 1.0}
-    labels = {k: (torch.randn(B, Fo, 12 if i == 3 else 6, generator=g) * scale[k]).pin_memory() for i, k in enumerate(LOSS_QUANTITIES)}
-    return {"inputs": inputs, "labels": labels}
+    def train_step_host(self, inputs, labels) -> float:
+        """One optimisation step fed from (pinned) host tensors: async H2D copies of the 14 tensors, one packing kernel for
+        the ten inputs and one for the four label tensors, the native step, then a D2H read of the loss."""
+        for loss in self.train_steps_host([(inputs, labels)]):
+            return loss
 
+    def train_steps_host(self, batches):
+        """Generator over host batches ``(inputs, labels)`` (dicts of pinned CPU tensors, as a DataLoader with
+        ``pin_memory=True`` yields them): one optimisation step per batch, yielding that step's loss as a python float.
 
-def _train_step_host(self, inputs, labels) -> float:
-    """One optimisation step fed from (pinned) host tensors: per-key async H2D copies, one packing kernel for the
-    ten inputs and one for the four label tensors, the native step, then a D2H read of the loss."""
-    from .keys import MODEL_INPUT_ORDER
-    dev = self.arena.device
-    B = inputs[MODEL_INPUT_ORDER[0]].shape[0]
-    key = ("host", B)
-    if key not in self._lab:
-        self._lab[key] = {k: torch.empty(v.shape, dtype=torch.float32, device=dev) for k, v in {**inputs, **labels}.items()}
-    stage = self._lab[key]
-    for k, v in {**inputs, **labels}.items():
-        stage[k].copy_(v, non_blocking=True)
-    F = stage[MODEL_INPUT_ORDER[0]].shape[1]
-    Fo = stage[LOSS_QUANTITIES[0]].shape[1]
-    if ("lab", B) not in self._lab:
-        self._lab[("lab", B)] = torch.empty(B, Fo, 30, dtype=torch.float32, device=dev)
-    lab = self._lab[("lab", B)]
-    ops.pack_inputs([stage[k].view(B * Fo, -1) for k in LOSS_QUANTITIES], B * Fo, Fo, out_f32=lab.view(B * Fo, 30))
-    srcs = [stage[k].view(B * F, -1) for k in MODEL_INPUT_ORDER]
-    self._begin_step()
-    self._pack_host_inputs(srcs, B, F)
-    result = self._finish_step(B, F, lab)
-    return float(result[0].item())
+        Every step: H2D copy of the step's 14 tensors, packing kernels, the native step, a D2H read of the loss — pipelined
+        the way a prefetching loader feeds a training loop: the copies of batch i+1 run on a copy stream into the other half
+        of a double-buffered staging area while step i computes, and the loss of step i is read back only after step i+1 has
+        been enqueued, so the GPU never waits for Python to launch the next step."""
+        dev = self.arena.device
+        copy_stream = getattr(self, "_copy_stream", None)
+        if copy_stream is None:
+            copy_stream = self._copy_stream = torch.cuda.Stream(device=dev)
+        main = torch.cuda.current_stream(dev)
+        it = iter(batches)
 
+        def upload(batch, slot):
+            inputs, labels = batch
+            B = inputs[MODEL_INPUT_ORDER[0]].shape[0]
+            key = (B, slot)
+            if key not in self._host_stage:
+                self._host_stage[key] = ({k: torch.empty(v.shape, dtype=torch.float32, device=dev) for k, v in {**inputs, **labels}.items()},
+                                         torch.cuda.Event(), torch.cuda.Event())
+            stage, ready, consumed = self._host_stage[key]
+            copy_stream.wait_event(consumed)                  # the step that last read this slot has packed it
+            with torch.cuda.stream(copy_stream):
+                for k, v in {**inputs, **labels}.items():
+                    stage[k].copy_(v, non_blocking=True)
+                ready.record(copy_stream)
+            return B, stage, ready, consumed
 
-def _train_steps_host(self, batches):
-    """Generator over host batches ``(inputs, labels)`` (dicts of pinned CPU tensors, as a DataLoader with
-    ``pin_memory=True`` yields them): one optimisation step per batch, yielding that step's loss as a python float.
+        def launch(up):
+            B, stage, ready, consumed = up
+            main.wait_event(ready)
+            F = stage[MODEL_INPUT_ORDER[0]].shape[1]
+            Fo = stage[LOSS_QUANTITIES[0]].shape[1]
+            if B not in self._host_labels:
+                self._host_labels[B] = torch.empty(B, Fo, 30, dtype=torch.float32, device=dev)
+            lab = self._host_labels[B]
+            ops.pack_inputs([stage[k].view(B * Fo, -1) for k in LOSS_QUANTITIES], B * Fo, Fo, out_f32=lab.view(B * Fo, 30))
+            self._begin_step()
+            # the ten per-key input tensors (FeedForward…py:97-108 concat order) -> the engine's packed bf16 layout, one kernel
+            buf, fs, we, col0 = self.eng.input_layout(B, F, True)
+            ops.pack_inputs([stage[k].view(B * F, -1) for k in MODEL_INPUT_ORDER], B * F, F, out_bf16=buf, frame_stride=fs,
+                            win_extra=we, col0=col0)
+            consumed.record(main)                             # staging slot is free once both packers have run
+            return self._step(B, F, lab)
 
-    Same work per step as ``train_step_host`` — H2D copy of the step's 14 tensors, packing kernels, the native step, a D2H
-    read of the loss — but pipelined the way a prefetching loader feeds a training loop: the copies of batch i+1 run on a
-    copy stream into the other half of a double-buffered staging area while step i computes, and the loss of step i is
-    read back only after step i+1 has been enqueued, so the GPU never waits for Python to launch the next step."""
-    from .keys import MODEL_INPUT_ORDER
-    dev = self.arena.device
-    copy_stream = getattr(self, "_copy_stream", None)
-    if copy_stream is None:
-        copy_stream = self._copy_stream = torch.cuda.Stream(device=dev)
-    main = torch.cuda.current_stream(dev)
-    it = iter(batches)
-
-    def upload(batch, slot):
-        inputs, labels = batch
-        B = inputs[MODEL_INPUT_ORDER[0]].shape[0]
-        key = ("hostpipe", B, slot)
-        if key not in self._lab:
-            self._lab[key] = ({k: torch.empty(v.shape, dtype=torch.float32, device=dev) for k, v in {**inputs, **labels}.items()},
-                              torch.cuda.Event(), torch.cuda.Event())
-        stage, ready, consumed = self._lab[key]
-        copy_stream.wait_event(consumed)                  # the step that last read this slot has packed it
-        with torch.cuda.stream(copy_stream):
-            for k, v in {**inputs, **labels}.items():
-                stage[k].copy_(v, non_blocking=True)
-            ready.record(copy_stream)
-        return B, stage, ready, consumed
-
-    def launch(up):
-        B, stage, ready, consumed = up
-        main.wait_event(ready)
-        F = stage[MODEL_INPUT_ORDER[0]].shape[1]
-        Fo = stage[LOSS_QUANTITIES[0]].shape[1]
-        if ("lab", B) not in self._lab:
-            self._lab[("lab", B)] = torch.empty(B, Fo, 30, dtype=torch.float32, device=dev)
-        lab = self._lab[("lab", B)]
-        ops.pack_inputs([stage[k].view(B * Fo, -1) for k in LOSS_QUANTITIES], B * Fo, Fo, out_f32=lab.view(B * Fo, 30))
-        srcs = [stage[k].view(B * F, -1) for k in MODEL_INPUT_ORDER]
-        self._begin_step()
-        self._pack_host_inputs(srcs, B, F)
-        consumed.record(main)                             # staging slot is free once both packers have run
-        return self._finish_step(B, F, lab)
-
-    try:
-        nxt = upload(next(it), 0)
-    except StopIteration:
-        return
-    slot, pending = 0, None                               # pending: (result tensor, event) of the step enqueued last
-    while nxt is not None:
-        cur = nxt
-        result = launch(cur)
-        done = torch.cuda.Event()
-        done.record(main)
-        slot ^= 1
         try:
-            nxt = upload(next(it), slot)                  # copies of the next batch overlap this step's kernels
+            nxt = upload(next(it), 0)
         except StopIteration:
-            nxt = None
-        if pending is not None:
-            pending[1].synchronize()
-            yield float(pending[0][0].item())
-        # the result ring holds 8 steps: cloning is not needed for a one-step delay
-        pending = (result, done)
-    pending[1].synchronize()
-    yield float(pending[0][0].item())
+            return
+        slot, pending = 0, None                               # pending: (result tensor, event) of the step enqueued last
+        while nxt is not None:
+            cur = nxt
+            result = launch(cur)
+            done = torch.cuda.Event()
+            done.record(main)
+            slot ^= 1
+            try:
+                nxt = upload(next(it), slot)                  # copies of the next batch overlap this step's kernels
+            except StopIteration:
+                nxt = None
+            if pending is not None:
+                pending[1].synchronize()
+                yield float(pending[0][0].item())
+            # the result ring holds 8 steps: cloning is not needed for a one-step delay
+            pending = (result, done)
+        pending[1].synchronize()
+        yield float(pending[0][0].item())
 
+    # ---- profiling helpers used by bench.py ------------------------------------------------------------------------
+    def profile_gemms(self, store, idx):
+        """One extra training step with CUDA events around every tcgen05 GEMM launch (on the launching stream):
+        returns (total GEMM ms, total algorithmic FLOPs = 2*M*N*K per launch, number of launches)."""
+        real = ops.gemm
+        recs = []
 
-def _pack_host_inputs(self, srcs, B: int, F: int) -> None:
-    """The ten per-key input tensors (FeedForward…py:97-108 concat order) -> the model's packed bf16 layout, one kernel."""
-    eng = self.eng
-    if self.is_denoiser:
-        ops.pack_inputs(srcs, B * F, F, out_bf16=eng.xc(B, True), frame_stride=eng.ld_in, win_extra=0, col0=30)
-    elif self.is_groundlink:
-        buf, fs, we, col0 = eng.input_rows(B, F)
-        ops.pack_inputs(srcs, B * F, F, out_bf16=buf, frame_stride=fs, win_extra=we, col0=col0)
-    else:
-        ops.pack_inputs(srcs, B * F, F, out_bf16=eng.input_buffer(B), frame_stride=self.model.frame_width,
-                        win_extra=eng.in_ld - self.model.input_size, col0=0)
+        def timed(A, Bm, out, M, N, K, **kw):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            r = real(A, Bm, out, M, N, K, **kw)
+            e1.record()
+            recs.append((e0, e1, 2.0 * M * N * K, (M, N, K)))
+            return r
 
+        # every other C-ABI entry point is timed the same way (per-kernel ms of one step, live, no profiler)
+        real_call = ops.call
+        krecs = []
 
-def _finish_step(self, B: int, F: int, lab: torch.Tensor) -> torch.Tensor:
-    if self.is_denoiser:
-        return self._finish_denoiser_step(B, lab)
-    if self.is_groundlink:
-        return self._finish_groundlink_step(B, F, lab)
-    return self._finish_ff_step(B, lab)
+        def timed_call(name, *a):
+            if name == "ibm_gemm_bf16":
+                return real_call(name, *a)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            real_call(name, *a)
+            e1.record()
+            krecs.append((name, e0, e1))
 
+        ops.gemm = timed
+        ops.call = timed_call
+        try:
+            self.train_step(store, idx)
+            torch.cuda.synchronize()
+        finally:
+            ops.gemm = real
+            ops.call = real_call
+        self.last_gemm_records = [(e0.elapsed_time(e1), fl, shp) for e0, e1, fl, shp in recs]
+        per = {}
+        for name, e0, e1 in krecs:
+            p = per.setdefault(name, [0, 0.0])
+            p[0] += 1
+            p[1] += e0.elapsed_time(e1)
+        self.last_kernel_ms = {k: {"launches": v[0], "ms": round(v[1], 4)} for k, v in sorted(per.items(), key=lambda kv: -kv[1][1])}
+        return sum(r[0] for r in self.last_gemm_records), sum(r[1] for r in self.last_gemm_records), len(recs)
 
-def _finish_groundlink_step(self, B: int, T: int, lab: torch.Tensor) -> torch.Tensor:
-    """Groundlink (Groundlink.py:135-156): implicit-GEMM CNN + per-frame MLP forward, fused loss on the strided
-    (B, T, 32) output view, backward into the flat gradient arena, fused optimizer."""
-    eng = self.eng
-    out = eng.forward(B, T, True)
-    gout = eng.dout_view(B, T)
-    if lab.shape[1] == 1:                               # last_frame: only the final frame is an output (Groundlink.py:147-148)
-        out, gout = out[:, -1:, :], gout[:, -1:, :]
-    outs, labs, gviews = _views30(out), _views30(lab), _views30(gout)
-    result = self._result_ring[self.step_count % len(self._result_ring)]
-    ops.regression_loss_fwd(outs, labs, self.weights, COP_FORCE_THRESHOLD, result=result)
-    ops.regression_loss_bwd(outs, labs, self.weights, gviews, threshold=COP_FORCE_THRESHOLD)
-    eng.backward(B, T)
-    self.bucketer.finish()
-    self.optimizer_step()
-    return result
+    def aux_measurements(self, store, idx, pk, world):
+        """HBM-bound kernels against the measured copy bandwidth (inputs >= 300 MB exceed L2), the per-shape GEMM table and the
+        per-kernel times of one training step.  Reverse sampling (BASELINE configs[3]) is bench_legs.sampling_leg."""
+        B = idx.numel()
+        dev = self.arena.device
+        hbm = pk["hbm_gbs"]
+        out = {}
+        if self.diffusion is not None:
+            eng, F = self.eng, self.eng.F
+            # stream of 16384 windows (819 200 rows): every operand set is > 200 MB, i.e. larger than the 126 MB L2,
+            # so consecutive timed launches cannot re-use each other's lines
+            Bb = 16384
+            M = Bb * F
+            rows = torch.randn(M, 32, device=dev)
+            lab = torch.randn(Bb, F, 30, device=dev) * 5
+            outs, labs = quantity_split(rows.view(Bb, F, 32)), quantity_split(lab)
+            res = torch.zeros(40, device=dev)
+            g16buf = torch.zeros(M, 32, dtype=torch.bfloat16, device=dev)
+            g16 = quantity_split(g16buf.view(Bb, F, 32))
 
+            def entry(ms, by):
+                return {"bound": "hbm", "ms": ms, "achieved": by / ms / 1e6, "peak": hbm, "unit": "GB/s", "frac": by / ms / 1e6 / hbm,
+                        "algorithmic_bytes": by, "rows": M}
 
-def _finish_denoiser_step(self, B: int, lab: torch.Tensor) -> torch.Tensor:
-    eng = self.eng
-    xc = eng.xc(B, True)
-    t = eng.t_buffer(B, True)
-    t.copy_(torch.randint(0, self.diffusion.T, (B,), device=t.device, generator=self._gen, dtype=torch.int32))
-    self.diffusion.q_sample(lab.view(B, -1), t, None, xt_bf16=xc, bf16_ld=eng.ld_in, seed=self.seed + self.rank, offset=self.step_count)
-    out = eng.forward(B, train=True)
-    outs, labs = _views30(out.view(B, eng.F, 32)), _views30(lab)
-    gviews = _views30(eng.dout(B).view(B, eng.F, 32))
-    result = self._result_ring[self.step_count % len(self._result_ring)]
-    ops.regression_loss_fwd(outs, labs, self.weights, COP_FORCE_THRESHOLD, result=result)
-    ops.regression_loss_bwd(outs, labs, self.weights, gviews, threshold=COP_FORCE_THRESHOLD)
-    eng.backward(B)
-    self.bucketer.finish()
-    self.optimizer_step()
-    return result
-
-
-def _finish_ff_step(self, B: int, lab: torch.Tensor) -> torch.Tensor:
-    eng = self.eng
-    out = eng.forward(B, train=True)
-    Fo = self.model.num_output_frames
-    outs, labs = _views_ff(out, B, Fo), _views30(lab)
-    gviews = _views_ff(eng.dout_buffer(B), B, Fo)
-    result = self._result_ring[self.step_count % len(self._result_ring)]
-    ops.regression_loss_fwd(outs, labs, self.weights, COP_FORCE_THRESHOLD, result=result)
-    ops.regression_loss_bwd(outs, labs, self.weights, gviews, threshold=COP_FORCE_THRESHOLD)
-    eng.backward(B)
-    self.bucketer.finish()
-    self.optimizer_step()
-    return result
-
-
-def _profile_gemms(self, store, idx):
-    """One extra training step with CUDA events around every tcgen05 GEMM launch (on the launching stream):
-    returns (total GEMM ms, total algorithmic FLOPs = 2*M*N*K per launch, number of launches)."""
-    real = ops.gemm
-    recs = []
-
-    def timed(A, Bm, out, M, N, K, **kw):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        r = real(A, Bm, out, M, N, K, **kw)
-        e1.record()
-        recs.append((e0, e1, 2.0 * M * N * K, (M, N, K)))
-        return r
-
-    # every other C-ABI entry point is timed the same way (per-kernel ms of one step, live, no profiler)
-    real_call = ops.call
-    krecs = []
-
-    def timed_call(name, *a):
-        if name == "ibm_gemm_bf16":
-            return real_call(name, *a)
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        real_call(name, *a)
-        e1.record()
-        krecs.append((name, e0, e1))
-
-    ops.gemm = timed
-    ops.call = timed_call
-    try:
-        self.train_step(store, idx)
-        torch.cuda.synchronize()
-    finally:
-        ops.gemm = real
-        ops.call = real_call
-    self.last_gemm_records = [(e0.elapsed_time(e1), fl, shp) for e0, e1, fl, shp in recs]
-    per = {}
-    for name, e0, e1 in krecs:
-        p = per.setdefault(name, [0, 0.0])
-        p[0] += 1
-        p[1] += e0.elapsed_time(e1)
-    self.last_kernel_ms = {k: {"launches": v[0], "ms": round(v[1], 4)} for k, v in sorted(per.items(), key=lambda kv: -kv[1][1])}
-    return sum(r[0] for r in self.last_gemm_records), sum(r[1] for r in self.last_gemm_records), len(recs)
-
-
-def _time_kernel(fn, iters: int = 20) -> float:
-    """Average GPU time of one launch: `iters` launches are captured in a CUDA graph and the replay is timed with
-    events, so host-side launch overhead (ctypes marshalling is ~50-100 us per call, longer than these kernels)
-    is not part of the number."""
-    for _ in range(3):
-        fn()
-    torch.cuda.synchronize()
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        for _ in range(iters):
-            fn()
-    g.replay()                                   # warm replay
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    e0.record()
-    g.replay()
-    e1.record()
-    torch.cuda.synchronize()
-    return e0.elapsed_time(e1) / iters
-
-
-def _aux_measurements(self, store, idx, pk, world):
-    """HBM-bound kernels against the measured copy bandwidth (inputs >= 300 MB exceed L2), the per-shape GEMM table and the
-    per-kernel times of one training step.  Reverse sampling (BASELINE configs[3]) is bench_legs.sampling_leg."""
-    B = idx.numel()
-    dev = self.arena.device
-    hbm = pk["hbm_gbs"]
-    out = {}
-    if self.is_denoiser:
-        eng, F = self.eng, self.eng.F
-        # stream of 16384 windows (819 200 rows): every operand set is > 200 MB, i.e. larger than the 126 MB L2,
-        # so consecutive timed launches cannot re-use each other's lines
-        Bb = 16384
-        M = Bb * F
-        rows = torch.randn(M, 32, device=dev)
-        lab = torch.randn(Bb, F, 30, device=dev) * 5
-        outs, labs = _views30(rows.view(Bb, F, 32)), _views30(lab)
-        res = torch.zeros(40, device=dev)
-        g16buf = torch.zeros(M, 32, dtype=torch.bfloat16, device=dev)
-        g16 = _views30(g16buf.view(Bb, F, 32))
-
-        def entry(ms, by):
-            return {"bound": "hbm", "ms": ms, "achieved": by / ms / 1e6, "peak": hbm, "unit": "GB/s", "frac": by / ms / 1e6 / hbm,
-                    "algorithmic_bytes": by, "rows": M}
-
-        out["loss_fwd"] = entry(_time_kernel(lambda: ops.regression_loss_fwd(outs, labs, self.weights, result=res)), M * 240.0)
-        out["loss_bwd_bf16"] = entry(_time_kernel(lambda: ops.regression_loss_bwd(outs, labs, self.weights, g16)), M * 300.0)
-        x0 = lab.view(Bb, -1)
-        eps = torch.randn_like(x0)
-        xt = torch.empty_like(x0)
-        t = torch.randint(0, 1000, (Bb,), device=dev, dtype=torch.int32)
-        d = self.diffusion
-        out["q_sample"] = entry(_time_kernel(lambda: ops.q_sample(x0, eps, t, d.sqrt_abar, d.sqrt_one_minus_abar, xt_f32=xt)), M * 360.0)
-        tdev = torch.full((1,), 500, dtype=torch.int32, device=dev)
-        xp = torch.empty(M, 30, device=dev)
-        out["posterior_step"] = entry(_time_kernel(lambda: ops.posterior_step(rows, 32, x0.view(M, 30), eps.view(M, 30), tdev, d.coef_x0,
-                                                                              d.coef_xt, d.sigma, M, x_prev=xp)), M * 480.0)
-        del rows, lab, g16buf, eps, xt, xp
-        # the same two kernels over an analysis-sized stream (65 536 windows = 3.3 M rows, 786 MB forward): the fixed costs of
-        # a 40 us launch (ramp-up, last-block fp64 reduction) are amortised, which is the regime of the analyze pass
-        Bs = 65536
-        Ms = Bs * F
-        rows = torch.randn(Ms, 32, device=dev)
-        lab = torch.randn(Bs, F, 30, device=dev) * 5
-        outs, labs = _views30(rows.view(Bs, F, 32)), _views30(lab)
-        g16buf = torch.zeros(Ms, 32, dtype=torch.bfloat16, device=dev)
-        g16 = _views30(g16buf.view(Bs, F, 32))
-        e = entry(_time_kernel(lambda: ops.regression_loss_fwd(outs, labs, self.weights, result=res), iters=10), Ms * 240.0)
-        e["rows"] = Ms
-        out["loss_fwd_stream"] = e
-        e = entry(_time_kernel(lambda: ops.regression_loss_bwd(outs, labs, self.weights, g16), iters=10), Ms * 300.0)
-        e["rows"] = Ms
-        out["loss_bwd_bf16_stream"] = e
-        del rows, lab, g16buf, outs, labs, g16
-        # per-shape table of the GEMM launches of one training step (from profile_gemms)
-        shapes = {}
-        for ms, fl, shp in getattr(self, "last_gemm_records", []):
-            e = shapes.setdefault("x".join(str(v) for v in shp), [0, 0.0, 0.0])
-            e[0] += 1; e[1] += ms; e[2] += fl
-        out["other_kernels_ms_per_step"] = getattr(self, "last_kernel_ms", {})
-        # the HBM-bound layer kernels as they run INSIDE the training step (power-capped clocks, cold L2, neighbours' tails):
-        # algorithmic bytes per launch / in-step CUDA-event time per launch, against the measured copy bandwidth
-        Mrows, d_ = B * F, eng.d
-        per_launch = {"ibm_attention_fwd": 8.0 * d_ * Mrows, "ibm_attention_bwd": 14.0 * d_ * Mrows,
-                      "ibm_layernorm_fwd": (4.0 * d_ + 8.0) * Mrows, "ibm_layernorm_bwd": (6.0 * d_ + 8.0) * Mrows,
-                      "ibm_regression_loss_fwd": 240.0 * Mrows, "ibm_regression_loss_bwd": 300.0 * Mrows}
-        tab = {}
-        for name, by in per_launch.items():
-            rec = out["other_kernels_ms_per_step"].get(name)
-            if rec and rec["ms"] > 0:
-                us = rec["ms"] * 1e3 / rec["launches"]
-                tab[name] = {"launches": rec["launches"], "us_per_launch": round(us, 1), "algorithmic_bytes": by,
-                             "achieved": by / us / 1e3, "peak": hbm, "unit": "GB/s", "frac": by / us / 1e3 / hbm}
-        out["hbm_kernels_in_step"] = tab
-        out["gemm_shapes_MxNxK"] = {k: {"launches": v[0], "ms": round(v[1], 4), "tflops": round(v[2] / (v[1] * 1e-3) / 1e12, 1)}
-                                    for k, v in shapes.items()}
-    return out
-
-
-Trainer.make_host_batch = _make_host_batch
-Trainer.train_step_host = _train_step_host
-Trainer.train_steps_host = _train_steps_host
-Trainer._finish_denoiser_step = _finish_denoiser_step
-Trainer._finish_ff_step = _finish_ff_step
-Trainer._finish_groundlink_step = _finish_groundlink_step
-Trainer._finish_step = _finish_step
-Trainer._pack_host_inputs = _pack_host_inputs
-Trainer.profile_gemms = _profile_gemms
-Trainer.aux_measurements = _aux_measurements
+            out["loss_fwd"] = entry(_time_kernel(lambda: ops.regression_loss_fwd(outs, labs, self.weights, result=res)), M * 240.0)
+            out["loss_bwd_bf16"] = entry(_time_kernel(lambda: ops.regression_loss_bwd(outs, labs, self.weights, g16)), M * 300.0)
+            x0 = lab.view(Bb, -1)
+            eps = torch.randn_like(x0)
+            xt = torch.empty_like(x0)
+            t = torch.randint(0, 1000, (Bb,), device=dev, dtype=torch.int32)
+            d = self.diffusion
+            out["q_sample"] = entry(_time_kernel(lambda: ops.q_sample(x0, eps, t, d.sqrt_abar, d.sqrt_one_minus_abar, xt_f32=xt)), M * 360.0)
+            tdev = torch.full((1,), 500, dtype=torch.int32, device=dev)
+            xp = torch.empty(M, 30, device=dev)
+            out["posterior_step"] = entry(_time_kernel(lambda: ops.posterior_step(rows, 32, x0.view(M, 30), eps.view(M, 30), tdev, d.coef_x0,
+                                                                                  d.coef_xt, d.sigma, M, x_prev=xp)), M * 480.0)
+            del rows, lab, g16buf, eps, xt, xp
+            # the same two kernels over an analysis-sized stream (65 536 windows = 3.3 M rows, 786 MB forward): the fixed costs of
+            # a 40 us launch (ramp-up, last-block fp64 reduction) are amortised, which is the regime of the analyze pass
+            Bs = 65536
+            Ms = Bs * F
+            rows = torch.randn(Ms, 32, device=dev)
+            lab = torch.randn(Bs, F, 30, device=dev) * 5
+            outs, labs = quantity_split(rows.view(Bs, F, 32)), quantity_split(lab)
+            g16buf = torch.zeros(Ms, 32, dtype=torch.bfloat16, device=dev)
+            g16 = quantity_split(g16buf.view(Bs, F, 32))
+            e = entry(_time_kernel(lambda: ops.regression_loss_fwd(outs, labs, self.weights, result=res), iters=10), Ms * 240.0)
+            e["rows"] = Ms
+            out["loss_fwd_stream"] = e
+            e = entry(_time_kernel(lambda: ops.regression_loss_bwd(outs, labs, self.weights, g16), iters=10), Ms * 300.0)
+            e["rows"] = Ms
+            out["loss_bwd_bf16_stream"] = e
+            del rows, lab, g16buf, outs, labs, g16
+            # per-shape table of the GEMM launches of one training step (from profile_gemms)
+            shapes = {}
+            for ms, fl, shp in getattr(self, "last_gemm_records", []):
+                e = shapes.setdefault("x".join(str(v) for v in shp), [0, 0.0, 0.0])
+                e[0] += 1; e[1] += ms; e[2] += fl
+            out["other_kernels_ms_per_step"] = getattr(self, "last_kernel_ms", {})
+            # the HBM-bound layer kernels as they run INSIDE the training step (power-capped clocks, cold L2, neighbours' tails):
+            # algorithmic bytes per launch / in-step CUDA-event time per launch, against the measured copy bandwidth
+            Mrows, d_ = B * F, eng.d
+            per_launch = {"ibm_attention_fwd": 8.0 * d_ * Mrows, "ibm_attention_bwd": 14.0 * d_ * Mrows,
+                          "ibm_layernorm_fwd": (4.0 * d_ + 8.0) * Mrows, "ibm_layernorm_bwd": (6.0 * d_ + 8.0) * Mrows,
+                          "ibm_regression_loss_fwd": 240.0 * Mrows, "ibm_regression_loss_bwd": 300.0 * Mrows}
+            tab = {}
+            for name, by in per_launch.items():
+                rec = out["other_kernels_ms_per_step"].get(name)
+                if rec and rec["ms"] > 0:
+                    us = rec["ms"] * 1e3 / rec["launches"]
+                    tab[name] = {"launches": rec["launches"], "us_per_launch": round(us, 1), "algorithmic_bytes": by,
+                                 "achieved": by / us / 1e3, "peak": hbm, "unit": "GB/s", "frac": by / us / 1e3 / hbm}
+            out["hbm_kernels_in_step"] = tab
+            out["gemm_shapes_MxNxK"] = {k: {"launches": v[0], "ms": round(v[1], 4), "tflops": round(v[2] / (v[1] * 1e-3) / 1e12, 1)}
+                                        for k, v in shapes.items()}
+        return out

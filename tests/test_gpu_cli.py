@@ -135,11 +135,14 @@ def test_trainer_resume_continues_the_uninterrupted_run(tmp_path, opt):
         Trainer(fresh(), opt_type="adagrad", lr=1e-3).load_optimizer_state_dict(ck["optimizer_state_dict"])
 
 
-@pytest.mark.parametrize("kind,opt", [("feedforward_dropout_bn", "adam"), ("feedforward", "adamax"), ("groundlink", "rmsprop")])
+@pytest.mark.parametrize("kind,opt", [("feedforward_dropout_bn", "adam"), ("feedforward", "adamax"), ("groundlink", "rmsprop"),
+                                      ("groundlink_eval", "rmsprop")])
 def test_graph_replayed_steps_equal_eager_steps(monkeypatch, kind, opt):
     """Small-batch steps are captured once and replayed (Trainer._graphable): with dropout, BatchNorm, Adam/Adamax and for
     Groundlink too — the Philox offsets and the bias-correction step come from a device-resident counter.  Same seeds =>
-    same masks => the replayed run equals the eager run (2e-5 absolute: fp32 reduce-add order of split-K weight gradients)."""
+    same masks => the replayed run equals the eager run (2e-5 absolute: fp32 reduce-add order of split-K weight gradients).
+    ``groundlink_eval`` evaluates right before the capture and between replays: both the captured steps and the evaluations
+    must read the conv weights the optimizer last wrote, not a cached GEMM layout of older ones."""
     from inferbiomechanics_b200.data.window_store import WindowStore
     from inferbiomechanics_b200.models.FeedForwardRegressionBaseline import FeedForwardBaseline
     from inferbiomechanics_b200.models.Groundlink import Groundlink
@@ -148,7 +151,7 @@ def test_graph_replayed_steps_equal_eager_steps(monkeypatch, kind, opt):
     def run(graphs: bool):
         monkeypatch.setenv("IBM_TRAIN_GRAPHS", "1" if graphs else "0")
         torch.manual_seed(0)
-        if kind == "groundlink":
+        if kind.startswith("groundlink"):
             m = Groundlink(23, 12, 10, "all_frames").cuda().train()
             store = WindowStore.synthetic(512, 20, 1, 177, "all_frames", seed=3, device="cuda")
             B = 16
@@ -160,14 +163,19 @@ def test_graph_replayed_steps_equal_eager_steps(monkeypatch, kind, opt):
             B = 32
         tr = Trainer(m, opt_type=opt, lr=1e-3, seed=9)
         idx = store.shard(0, 1)
-        losses = [tr.train_step(store, idx[(i % 4) * B:(i % 4 + 1) * B])[0].item() for i in range(7)]
+        losses, evals = [], []
+        for i in range(7):
+            losses.append(tr.train_step(store, idx[(i % 4) * B:(i % 4 + 1) * B])[0].item())
+            if kind == "groundlink_eval" and i in (1, 4):     # after the last eager step before the capture, and between replays
+                evals.append(tr.eval_step(store, idx[:B])[0].item())
         replayed = any(g[1] is not None for g in tr._graphs.values())
-        return {n: p.detach().clone() for n, p in m.named_parameters()}, losses, replayed, tr
+        return {n: p.detach().clone() for n, p in m.named_parameters()}, losses + evals, replayed, tr
 
     pe, le, re_, _ = run(False)
     pg, lg, rg, tr = run(True)
     assert rg and not re_                                   # steps 3.. of the second run were graph replays
     assert int(tr.step_dev.item()) == tr.step_count == 7
+    assert len(le) == len(lg) == (9 if kind == "groundlink_eval" else 7)
     for a, b in zip(le, lg):
         assert abs(a - b) <= 1e-4 * abs(a), (le, lg)
     for n in pe:

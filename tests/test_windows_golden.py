@@ -72,7 +72,7 @@ def test_oracle_sampler_and_loader_match_torch(name):
 # ------------------------------------------------ CUDA path ---------------------------------------------------
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", CASES)
-def test_window_store_matches_reference_class(name):
+def test_window_store_and_pack_match_reference_class(name):
     from inferbiomechanics_b200.data.window_store import WindowStore
     subjects, T, s, fmt, _ = _case(name)
     nb = int(GOLD[f"{name}/meta"][7])
@@ -88,7 +88,7 @@ def test_window_store_matches_reference_class(name):
     F, C = store.F, store.C
     ld = (F * C + 7) // 8 * 8
     ff16 = torch.zeros(len(pick), ld, dtype=torch.bfloat16, device="cuda")
-    store.pack_feedforward(idx, ff16)
+    store.pack(idx, (ff16, C, ld - F * C, 0))                      # FeedForward layout: one row per window
     for bi, i in enumerate(pick):
         g_in = np.concatenate([GOLD[f"{name}/w{int(i)}/in/{k}"] for k in ow.INPUT_ORDER], axis=-1)
         assert np.array_equal(x[bi], g_in)
