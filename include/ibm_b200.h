@@ -187,6 +187,16 @@ int ibm_ddpm_posterior_step(const float* x0_hat, int64_t x0_ld, const float* x_t
                             int64_t bf16_ld, uint64_t seed, uint64_t offset, int32_t* t_next_dev,
                             void* stream);
 
+/* One step of a respaced sampler (DDIM, DESIGN.md D-1) with the arguments and semantics of
+ * ibm_ddpm_posterior_step: x_p = coef_x0[t] x0_hat + coef_xt[t] x_t + [t>0] sigma[t] z, Philox counter
+ * offset + t.  The tables hold the coefficients of the step from t to its successor p, and
+ * t_succ (device int32 [T]) names p: t_next_dev, if not NULL, receives t_succ[t] instead of t-1. */
+int ibm_ddpm_respaced_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const float* z,
+                           const int32_t* t_dev, const float* coef_x0, const float* coef_xt,
+                           const float* sigma, int64_t M, float* x_prev, void* xprev_bf16,
+                           int64_t bf16_ld, uint64_t seed, uint64_t offset, int32_t* t_next_dev,
+                           const int32_t* t_succ, void* stream);
+
 /* sinusoidal timestep embedding, bf16 [B, dim] (ld = dim): [sin(t w_k) | cos(t w_k)],
  * w_k = 10000^(-k/(dim/2)).  t: int32[B], or if t_is_scalar a single device int32 broadcast. */
 int ibm_timestep_embed(const int32_t* t, int32_t t_is_scalar, int64_t B, int32_t dim, void* out_bf16,

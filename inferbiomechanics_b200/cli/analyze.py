@@ -6,7 +6,8 @@ independent, so here each rank takes a CONTIGUOUS range of windows in large equa
 collective during the pass), keeps the per-batch fp32[40] results on the device and merges them once at the end —
 equal batch sizes keep the reference's mean-of-batch-means aggregate (RegressionLossEvaluator.py:383-387) exact.
 Per-window plots (matplotlib) and the names CSV are outside the hot path.  ``--model-type diffusion`` runs the
-1000-step reverse sampler per batch and scores the sampled trajectories with the same evaluator.
+reverse sampler per batch (``--sampler ddpm``: the 1000-step chain; ``ddim``: ``--sampling-steps`` respaced steps) and
+scores the sampled trajectories with the same evaluator.
 """
 from __future__ import annotations
 
@@ -19,12 +20,11 @@ import torch.distributed as dist
 
 from .. import parallel
 from ..diffusion import GaussianDiffusion
-from ..keys import LOSS_QUANTITIES
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
 from ..trainer import Trainer
 from . import _data
 from .abstract_command import AbstractCommand
-from .train import _ResultLog, input_dict, label_dict
+from .train import _ResultLog, input_dict, label_dict, sample_and_score
 
 
 class AnalyzeCommand(AbstractCommand):
@@ -58,11 +58,20 @@ class AnalyzeCommand(AbstractCommand):
         # additions of the B200 path
         sp.add_argument('--synthetic-windows', type=int, default=0, help='Analyze synthetic windows instead of *.ibmstore files.')
         sp.add_argument('--batch-size', type=int, default=4096, help='Windows per launch (the reference analyses one at a time).')
-        sp.add_argument('--sampling-steps', type=int, default=1000, help='Reverse-diffusion steps for --model-type diffusion.')
+        sp.add_argument('--sampling-steps', type=int, default=1000,
+                        help='Reverse-diffusion steps for --model-type diffusion.  --sampler ddpm: the first N steps of the '
+                             '1000-step chain (N < 1000 truncates it and scores a partially denoised sample); --sampler ddim: '
+                             'the number S of respaced steps (1..1000).')
+        sp.add_argument('--sampler', type=str, default='ddpm', choices=['ddpm', 'ddim'],
+                        help='Reverse sampler for --model-type diffusion: the ancestral DDPM chain or few-step DDIM.')
+        sp.add_argument('--eta', type=float, default=0.0,
+                        help='DDIM noise scale in [0, 1] (0: deterministic given x_T; 1: respaced ancestral sampling).')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'analyze':
             return False
+        if args.sampler == 'ddpm' and args.eta != 0.0:
+            raise ValueError("--eta applies to --sampler ddim only")
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
         root_history_len = 10
@@ -101,18 +110,14 @@ class AnalyzeCommand(AbstractCommand):
                         log.add(trainer.eval_step(store, idx))
                         continue
                     if model_type == 'diffusion':
-                        # condition = the packed kinematics in the engine's concat buffer; x_T ~ Philox; CUDA-graph replays
-                        store.pack(idx, model.engine().input_layout(idx.numel(), store.F, False))
-                        x0 = diffusion.sample(model, idx.numel(), steps=args.sampling_steps, seed=1234 + rank)
-                        if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
-                            x0 = x0[:, -1:]
-                        cuts = [(0, 6), (6, 12), (12, 18), (18, 30)]
-                        inputs = {}
-                        outputs = {k: x0[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, cuts)}
-                    else:
-                        inputs = input_dict(store, idx, model_type, args.stride, root_history_len)
-                        outputs = model(inputs)
-                    ev(inputs, outputs, label_dict(store, idx), [], [], args)
+                        if args.sampler == 'ddim':
+                            sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, ddim_steps=args.sampling_steps,
+                                             eta=args.eta)
+                        else:
+                            sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, steps=args.sampling_steps)
+                        continue
+                    inputs = input_dict(store, idx, model_type, args.stride, root_history_len)
+                    ev(inputs, model(inputs), label_dict(store, idx), [], [], args)
             src = log.ev if native else ev
             # one merge of the per-rank batch results at the very end (≈ 40 floats per batch); no collective before
             if world > 1:

@@ -21,6 +21,7 @@ import torch.distributed as dist
 
 from .. import parallel
 from ..data.window_store import WindowStore
+from ..diffusion import GaussianDiffusion
 from ..keys import LOSS_QUANTITIES, MODEL_INPUT_ORDER
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
 from ..trainer import Trainer
@@ -42,10 +43,25 @@ def input_dict(store: WindowStore, idx: torch.Tensor, model_type: str, stride: i
     return out
 
 
+QUANTITY_CUTS = [(0, 6), (6, 12), (12, 18), (18, 30)]       # column ranges of the four loss quantities in a 30-wide row
+
+
 def label_dict(store: WindowStore, idx: torch.Tensor):
     lab = store.labels(idx)
-    cuts = [(0, 6), (6, 12), (12, 18), (18, 30)]
-    return {k: lab[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, cuts)}
+    return {k: lab[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, QUANTITY_CUTS)}
+
+
+def sample_and_score(diffusion, model, store: WindowStore, idx: torch.Tensor, ev: RegressionLossEvaluator, args, seed: int,
+                     *, steps=None, ddim_steps=None, eta: float = 0.0) -> None:
+    """Reverse-sample the denoiser's trajectories for windows ``idx`` of ``store`` and score them with ``ev`` against the
+    store's labels: the condition is the packed kinematics in the engine's concat buffer, x_T ~ Philox(``seed``), and
+    ``steps`` / ``ddim_steps`` / ``eta`` select the sampler as in ``GaussianDiffusion.sample``."""
+    store.pack(idx, model.engine().input_layout(idx.numel(), store.F, False))
+    x0 = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta)
+    if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
+        x0 = x0[:, -1:]
+    outputs = {k: x0[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, QUANTITY_CUTS)}
+    ev({}, outputs, label_dict(store, idx), [], [], args)
 
 
 class _ResultLog:
@@ -137,12 +153,17 @@ class TrainCommand(AbstractCommand):
         sp.add_argument('--synthetic-windows', type=int, default=0,
                         help='Train on this many synthetic AddBiomechanics-shaped windows instead of <dataset-home>/*.ibmstore.')
         sp.add_argument('--max-batches', type=int, default=0, help='Stop every epoch after this many batches (0 = all).')
+        sp.add_argument('--dev-sampling-steps', type=int, default=0,
+                        help='--model-type diffusion: score the dev set before each epoch on samples of this many DDIM steps '
+                             '(eta = 0); 0 skips the dev pass of the denoiser.')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'train':
             return False
         if args.compute_report:
             raise NotImplementedError("--compute-report needs nimblephysics inverse dynamics (RegressionLossEvaluator.py:265-286)")
+        if args.dev_sampling_steps < 0:
+            raise ValueError(f"--dev-sampling-steps must be >= 0, got {args.dev_sampling_steps}")
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
         root_history_len = 10
@@ -194,14 +215,19 @@ class TrainCommand(AbstractCommand):
             train_batches, dev_batches = train_batches[:args.max_batches], dev_batches[:args.max_batches]
         train_log, dev_log = _ResultLog('train'), _ResultLog(DEV)
         train_ev, dev_ev = RegressionLossEvaluator(None, 'train', device=device), RegressionLossEvaluator(None, DEV, device=device)
+        # the denoiser is evaluated by reverse sampling, as in analyze: a few DDIM steps per dev batch, or no dev pass
+        dev_diffusion = GaussianDiffusion(device=device) if model_type == 'diffusion' and args.dev_sampling_steps else None
 
         for epoch in range(epoch_checkpoint + 1, args.epochs):
             print(f'[{rank=}] Evaluating Dev Set Before Epoch {epoch}')
             with torch.no_grad():
                 model.eval()
-                if model_type != 'diffusion':                 # denoiser evaluation = reverse sampling (analyze)
+                if model_type != 'diffusion' or dev_diffusion is not None:
                     for i, idx in enumerate(dev_batches):
-                        if native:
+                        if dev_diffusion is not None:
+                            sample_and_score(dev_diffusion, model, dev_store, idx, dev_log.ev, args, 1234 + rank,
+                                             ddim_steps=args.dev_sampling_steps)
+                        elif native:
                             dev_log.add(trainer.eval_step(dev_store, idx))
                         else:
                             inputs = input_dict(dev_store, idx, model_type, args.stride, root_history_len)

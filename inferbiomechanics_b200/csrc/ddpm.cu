@@ -63,13 +63,16 @@ q_sample_kernel(const float* __restrict__ x0, const float* __restrict__ eps, con
 
 // ---- posterior step --------------------------------------------------------------------------
 // One float2 per thread-iteration: 30 is even so a pair never straddles a row; x0_hat has its own
-// leading dimension (the head GEMM writes 32-float rows).
+// leading dimension (the head GEMM writes 32-float rows).  kSucc: the next timestep is t_succ[t]
+// (a respaced DDIM sequence) instead of t-1; the instantiation without it is the DDPM chain.
+template <bool kSucc>
 __global__ void __launch_bounds__(kThreads)
 posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __restrict__ xt,
                  const float* __restrict__ z, const int32_t* __restrict__ t_dev, const float* __restrict__ c1t,
                  const float* __restrict__ c2t, const float* __restrict__ sig, long long M,
                  float* __restrict__ xprev, __nv_bfloat16* __restrict__ xp_bf16, long long bf16_ld,
-                 uint64_t seed, uint64_t offset, int32_t* __restrict__ t_next) {
+                 uint64_t seed, uint64_t offset, int32_t* __restrict__ t_next,
+                 const int32_t* __restrict__ t_succ) {
   const int tt = __ldg(t_dev);
   const float c1 = __ldg(c1t + tt), c2 = __ldg(c2t + tt);
   const float s = tt > 0 ? __ldg(sig + tt) : 0.f;
@@ -94,7 +97,7 @@ posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __
     if (xprev) *reinterpret_cast<float2*>(xprev + 2 * p) = r;
     if (xp_bf16) *reinterpret_cast<uint32_t*>(xp_bf16 + m * bf16_ld + c) = pack_bf16x2(r.x, r.y);
   }
-  if (t_next && blockIdx.x == 0 && threadIdx.x == 0) *t_next = tt - 1;
+  if (t_next && blockIdx.x == 0 && threadIdx.x == 0) *t_next = kSucc ? __ldg(t_succ + tt) : tt - 1;
 }
 
 // ---- sinusoidal timestep embedding -----------------------------------------------------------
@@ -305,9 +308,27 @@ extern "C" int ibm_ddpm_posterior_step(const float* x0_hat, int64_t x0_ld, const
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "posterior_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "posterior_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "posterior_step: bf16 ld must be even");
-  posterior_kernel<<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev);
+      seed, offset, t_next_dev, nullptr);
+  IBM_LAUNCH_CHECK();
+  return IBM_OK;
+}
+
+extern "C" int ibm_ddpm_respaced_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const float* z,
+                                      const int32_t* t_dev, const float* coef_x0, const float* coef_xt,
+                                      const float* sigma, int64_t M, float* x_prev, void* xprev_bf16, int64_t bf16_ld,
+                                      uint64_t seed, uint64_t offset, int32_t* t_next_dev, const int32_t* t_succ,
+                                      void* stream) {
+  using namespace ibm;
+  IBM_CHECK_ARCH();
+  IBM_CHECK_ARG(x0_hat && x_t && t_dev && coef_x0 && coef_xt && sigma && t_succ, "respaced_step: null argument");
+  IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "respaced_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
+  IBM_CHECK_ARG(x_prev || xprev_bf16, "respaced_step: no output requested");
+  IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "respaced_step: bf16 ld must be even");
+  posterior_kernel<true><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
+      seed, offset, t_next_dev, t_succ);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }

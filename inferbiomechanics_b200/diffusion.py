@@ -5,6 +5,10 @@ the reference has no diffusion code).
   x_t   = sqrt(abar_t) x0 + sqrt(1-abar_t) eps                      on-device Philox noise
   x_{t-1} = c1_t x0_hat + c2_t x_t + [t>0] sigma_t z                posterior step: fused kernel
 
+Few-step sampling (DDIM, Song et al. 2021) walks a respaced sequence ts = round(linspace(T-1, 0, S)) with the
+same kernel: each step from t to its successor p = succ[t] is linear in (x0_hat, x_t, z) with per-timestep tables
+(``ddim_schedule``); eta = 1 over all T steps is the DDPM chain above, bit for bit.
+
 The reverse loop runs the denoiser forward + one fused posterior kernel per step; the timestep lives
 in device memory so two consecutive steps are captured once in a CUDA graph and replayed (sampling at
 512 windows/GPU is launch-bound otherwise).  Windows are independent: multi-GPU sampling shards them
@@ -20,9 +24,53 @@ import torch
 from . import ops
 
 
+def ddim_schedule(ddim_steps: int, eta: float = 0.0, num_timesteps: int = 1000, beta_start: float = 1e-4,
+                  beta_end: float = 2e-2) -> dict:
+    """Host tables (numpy, no GPU) of S = ``ddim_steps``-step DDIM sampling over the trained schedule (DESIGN.md D-1).
+
+    ``ts`` (int64 [S]) = round(linspace(T-1, 0, S)): the timesteps walked, strictly decreasing from T-1.  The step from
+    t = ts[i] to p = ts[i+1] (p = -1 after the last, abar[-1] := 1) is, with a = abar in fp64,
+      sigma = eta sqrt((1-a_p)/(1-a_t)) sqrt(1 - a_t/a_p),   c = sqrt(max(1 - a_p - sigma^2, 0))
+      x_p   = coef_x0[t] x0_hat + coef_xt[t] x_t + [t>0] sigma[t] z
+      coef_x0 = sqrt(a_p) - c sqrt(a_t)/sqrt(1-a_t),   coef_xt = c/sqrt(1-a_t)
+    which is sqrt(a_p) x0_hat + c eps_hat + sigma z for eps_hat = (x_t - sqrt(a_t) x0_hat)/sqrt(1-a_t).  ``coef_x0``,
+    ``coef_xt``, ``sigma`` (fp32 [T]) and ``succ`` (int32 [T], = p) are indexed by timestep, 0 off the sequence.  The
+    expressions are evaluated in exactly this order: at S = T and eta = 1 the fp32 tables then equal the DDPM
+    posterior tables bit for bit (sigma at t >= 1; the step at t = 0 draws no noise in either)."""
+    T = num_timesteps
+    _check_schedule(T, None, ddim_steps, eta)
+    abar = np.cumprod(1.0 - np.linspace(beta_start, beta_end, T, dtype=np.float64))
+    ts = np.round(np.linspace(T - 1, 0, ddim_steps)).astype(np.int64)
+    succ = np.append(ts[1:], -1)
+    a_t = abar[ts]
+    a_p = np.where(succ >= 0, abar[np.maximum(succ, 0)], 1.0)
+    sigma = eta * np.sqrt((1.0 - a_p) / (1.0 - a_t)) * np.sqrt(1.0 - a_t / a_p)
+    c = np.sqrt(np.maximum(1.0 - a_p - sigma * sigma, 0.0))
+    tab = dict(coef_x0=np.sqrt(a_p) - c * np.sqrt(a_t) / np.sqrt(1.0 - a_t), coef_xt=c / np.sqrt(1.0 - a_t), sigma=sigma)
+    out = {k: np.zeros(T, dtype=np.float32) for k in tab}
+    for k, v in tab.items():
+        out[k][ts] = v.astype(np.float32)
+    out["succ"] = np.zeros(T, dtype=np.int32)
+    out["succ"][ts] = succ
+    out["ts"] = ts
+    return out
+
+
+def _check_schedule(T: int, steps: Optional[int], ddim_steps: Optional[int], eta: float) -> None:
+    if steps is not None and ddim_steps is not None:
+        raise ValueError("give either steps (a truncated DDPM chain) or ddim_steps (a respaced DDIM sequence), not both")
+    if ddim_steps is not None and not 1 <= ddim_steps <= T:
+        raise ValueError(f"ddim_steps must lie in [1, {T}], got {ddim_steps}")
+    if not 0.0 <= eta <= 1.0:
+        raise ValueError(f"eta must lie in [0, 1], got {eta}")
+    if eta != 0.0 and ddim_steps is None:
+        raise ValueError("eta applies to DDIM sampling only: give ddim_steps")
+
+
 class GaussianDiffusion:
     def __init__(self, num_timesteps: int = 1000, beta_start: float = 1e-4, beta_end: float = 2e-2, device="cuda"):
         self.T = num_timesteps
+        self.beta_start, self.beta_end = beta_start, beta_end
         betas = np.linspace(beta_start, beta_end, num_timesteps, dtype=np.float64)
         alphas = 1.0 - betas
         abar = np.cumprod(alphas)
@@ -37,6 +85,7 @@ class GaussianDiffusion:
         self.sigma = f(np.exp(0.5 * post_logvar))
         self.device = torch.device(device)
         self._graphs = {}
+        self._ddim = {}                 # (S, eta) -> device tables of ddim_schedule
         # reverse sampling: take the time MLP from the engine's per-timestep table (DenoiserEngine.temb_table) instead of
         # evaluating it every step; False re-runs it per step (parity check, tests/test_gpu_models.py)
         self.use_temb_table = True
@@ -51,24 +100,51 @@ class GaussianDiffusion:
                      seed=seed, offset=offset, eps_out=eps_out)
         return xt_f32
 
+    def ddim_tables(self, ddim_steps: int, eta: float = 0.0) -> dict:
+        """``ddim_schedule`` of this schedule on the device (cached per (S, eta)): coef_x0 / coef_xt / sigma fp32 [T],
+        succ int32 [T], ts (host numpy)."""
+        key = (ddim_steps, float(eta))
+        tab = self._ddim.get(key)
+        if tab is None:
+            h = ddim_schedule(ddim_steps, eta, self.T, self.beta_start, self.beta_end)
+            tab = {k: v if k == "ts" else torch.from_numpy(v).to(self.device) for k, v in h.items()}
+            self._ddim[key] = tab
+        return tab
+
     # ---- reverse process -----------------------------------------------------------------------
     @torch.no_grad()
     def sample(self, model, B: int, *, x_T: Optional[torch.Tensor] = None, noise: Optional[Callable[[int], torch.Tensor]] = None,
-               steps: Optional[int] = None, seed: int = 0, use_graph: bool = True) -> torch.Tensor:
+               steps: Optional[int] = None, seed: int = 0, use_graph: bool = True, ddim_steps: Optional[int] = None,
+               eta: float = 0.0) -> torch.Tensor:
         """Reverse-sample x_0 (B,F,30) for the kinematics already packed in model.engine().xc(B, False)
-        (columns 30…).  ``noise(t)`` supplies z per step for parity tests; None ⇒ on-device Philox."""
+        (columns 30…).  ``noise(t)`` supplies z per step for parity tests; None ⇒ on-device Philox.
+
+        ``ddim_steps=None``: the DDPM chain; ``steps`` < T runs only its first ``steps`` steps and returns x at timestep
+        T - steps (a truncated chain, not a sample).  ``ddim_steps=S``: S-step DDIM with noise scale ``eta`` in [0, 1]
+        (``ddim_schedule``); eta = 0 draws no noise after x_T.  ``noise(t)`` is called with each timestep walked."""
+        _check_schedule(self.T, steps, ddim_steps, eta)
         eng = model.engine()
         F, M = eng.F, B * eng.F
         xc = eng.xc(B, False)
-        key = (id(model), B)
+        if ddim_steps is None:
+            sched = None
+            ts = range(self.T - 1, self.T - 1 - (self.T if steps is None else steps), -1)
+            coef_x0, coef_xt, sigma, succ = self.coef_x0, self.coef_xt, self.sigma, None
+        else:
+            sched = (ddim_steps, float(eta))
+            tab = self.ddim_tables(ddim_steps, eta)
+            ts = tab["ts"].tolist()
+            coef_x0, coef_xt, sigma, succ = tab["coef_x0"], tab["coef_xt"], tab["sigma"], tab["succ"]
+        # the captured launches read the schedule's tables through baked-in pointers, so each schedule has its own graph
+        key = (id(model), B, sched)
         st = self._graphs.get(key)
         if st is None or st["model"] is not model:
-            # the entry holds the model (its id() cannot be recycled while cached) and, below, the time-MLP table the
-            # captured launches read
+            # the entry holds the model (its id() cannot be recycled while cached), the schedule's tables and, below, the
+            # time-MLP table the captured launches read
             st = dict(x=torch.empty(M, 30, dtype=torch.float32, device=self.device),
                       t_a=torch.zeros(1, dtype=torch.int32, device=self.device),
                       t_b=torch.zeros(1, dtype=torch.int32, device=self.device), graph=None, seed=None, model=model, table=None,
-                      table_key=None)
+                      table_key=None, sched_tables=(coef_x0, coef_xt, sigma, succ))
             self._graphs[key] = st
         x, t_a, t_b = st["x"], st["t_a"], st["t_b"]
         if x_T is None:
@@ -80,18 +156,19 @@ class GaussianDiffusion:
         else:
             x.copy_(x_T.reshape(M, 30))
             ops.pack_inputs([x], M, F, out_bf16=xc, frame_stride=eng.ld_in, win_extra=0, col0=0)
-        n_steps = self.T if steps is None else steps
+        n_steps = len(ts)
         t_a.fill_(self.T - 1)
 
         def step(t_in, t_out, z):
             x0_hat = eng.forward(B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
-            ops.posterior_step(x0_hat, 32, x, z, t_in, self.coef_x0, self.coef_xt, self.sigma, M, x_prev=x, xprev_bf16=xc,
-                               bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out)
+            ops.posterior_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, x_prev=x, xprev_bf16=xc,
+                               bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ)
 
-        if noise is not None or not use_graph or n_steps % 2:
+        # DDPM runs an odd step count eagerly, as it always has; DDIM replays the graph for the even part of any S >= 2
+        if noise is not None or not use_graph or (n_steps % 2 if sched is None else n_steps < 2):
             cur, nxt = t_a, t_b
-            for i in range(n_steps):
-                step(cur, nxt, noise(self.T - 1 - i) if noise is not None else None)
+            for t in ts:
+                step(cur, nxt, noise(t) if noise is not None else None)
                 cur, nxt = nxt, cur
             return x.view(B, F, 30).clone()
 
@@ -117,12 +194,15 @@ class GaussianDiffusion:
             done -= 2
         for _ in range((n_steps - done) // 2):
             st["graph"].replay()
+        if n_steps % 2:
+            step(t_a, t_b, None)                  # the last step of an odd S: the ping-pong left its timestep in t_a
         return x.view(B, F, 30).clone()
 
     # ---- BASELINE configs[3]: a set of windows sharded over the ranks, no collective ------------------------------
     @torch.no_grad()
     def sample_windows(self, model, cond: torch.Tensor, *, batch: int = 512, steps: Optional[int] = None, seed: int = 0,
-                       rank: Optional[int] = None, world: Optional[int] = None):
+                       rank: Optional[int] = None, world: Optional[int] = None, ddim_steps: Optional[int] = None,
+                       eta: float = 0.0):
         """Reverse-sample GRF / CoP / torque / wrench trajectories for ``cond``: (N, F, C_in) fp32 packed kinematics of N
         windows (model concat order, FeedForward...py:97-108) in HOST memory (pinned for asynchronous copies).
 
@@ -130,8 +210,10 @@ class GaussianDiffusion:
         batches of ``batch`` windows — H2D copy of the batch's conditions, one packing kernel into the denoiser's concat buffer,
         ``steps`` (default: the full schedule) CUDA-graph-replayed denoise steps, D2H copy of the trajectories — and returns
         ``(range, x0)`` with x0 a pinned host tensor (len(range), F, 30).  No collective; per-rank noise stream = seed + rank.
-        The copies of batch i+1 / i-1 overlap the sampling of batch i (separate streams)."""
+        The copies of batch i+1 / i-1 overlap the sampling of batch i (separate streams).  ``ddim_steps`` / ``eta`` select
+        DDIM sampling as in ``sample``."""
         from . import parallel
+        _check_schedule(self.T, steps, ddim_steps, eta)
         r, w = parallel.world()
         rank = r if rank is None else rank
         world = w if world is None else world
@@ -170,7 +252,7 @@ class GaussianDiffusion:
             packed[i & 1].record(main)
             if i + 1 < len(starts):
                 upload(i + 1)
-            x0 = self.sample(model, nb, steps=steps, seed=seed + rank + 7919 * i)
+            x0 = self.sample(model, nb, steps=steps, seed=seed + rank + 7919 * i, ddim_steps=ddim_steps, eta=eta)
             ready = torch.cuda.Event()
             ready.record(main)
             with torch.cuda.stream(down):

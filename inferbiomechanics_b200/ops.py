@@ -282,9 +282,15 @@ def q_sample(x0, eps, t, sqrt_abar, sqrt_1m_abar, xt_f32=None, xt_bf16=None, bf1
 
 
 def posterior_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev=None, xprev_bf16=None, bf16_ld=0,
-                   seed=0, offset=0, t_next=None):
-    call("ibm_ddpm_posterior_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
-         _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), stream_ptr())
+                   seed=0, offset=0, t_next=None, t_succ=None):
+    """t_succ (device int32 [T]): the step of a respaced (DDIM) sequence, t_next receives t_succ[t]; None ⇒ the DDPM
+    posterior step, t_next receives t-1."""
+    if t_succ is None:
+        call("ibm_ddpm_posterior_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
+             _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), stream_ptr())
+    else:
+        call("ibm_ddpm_respaced_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
+             _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), stream_ptr())
 
 
 def timestep_embed(t, out_bf16, dim, scalar=False):
