@@ -266,7 +266,8 @@ int ibm_conv_wgrad_from_gemm(const float* g, int32_t cout, int32_t cin, int32_t 
 
 /* Temporal replicate padding for the implicit-GEMM convolution (Groundlink.py:41, padding_mode="replicate").
  * Padded row layout: window b owns rows [b*Tp, (b+1)*Tp), Tp = T + 2*pad, frame t at row b*Tp + pad + t.
- * replicate: pad rows <- first / last frame row.  fold (its adjoint): edge frame rows += pad rows, pad rows <- 0. */
+ * replicate: pad rows <- first / last frame row.  fold (its adjoint): edge frame rows += pad rows, pad rows <- 0
+ * (T == 1: the one frame row gains both sides' pad rows).  T > 0, pad >= 0; pad == 0 (kernel size 1) is a no-op. */
 int ibm_replicate_pad_rows(void* X_bf16, int64_t ld, int64_t n_win, int32_t T, int32_t pad, int32_t cols, void* stream);
 int ibm_fold_pad_rows(void* G_bf16, int64_t ld, int64_t n_win, int32_t T, int32_t pad, int32_t cols, void* stream);
 /* Inverted dropout (nn.Dropout, Groundlink.py:53,59): y = x * keep/(1-p), keep from Philox4x32-10(seed, offset);

@@ -207,7 +207,8 @@ extern "C" int ibm_conv_wgrad_from_gemm(const float* g, int32_t cout, int32_t ci
 // Activations live in a padded row layout: window b owns rows [b*Tp, (b+1)*Tp), Tp = T + 2*pad, frame t at row
 // b*Tp + pad + t.  replicate_pad copies the first/last frame rows into the pad rows; fold_pad is its adjoint
 // (pad-row gradients are added into the edge frames, then the pad rows are zeroed so they cannot leak into the
-// shifted dgrad/wgrad GEMMs).
+// shifted dgrad/wgrad GEMMs).  With T == 1 both edges are the same row, so the side-0 thread folds both sides' pad
+// rows into it and the side-1 thread does nothing (two threads storing one row would drop one side's sum).
 namespace ibm {
 __global__ void __launch_bounds__(kThreads)
 replicate_pad_kernel(__nv_bfloat16* __restrict__ X, long long ld, long long n_win, int T, int pad, int cols8) {
@@ -231,8 +232,10 @@ fold_pad_kernel(__nv_bfloat16* __restrict__ G, long long ld, long long n_win, in
     const int c = (int)(i % cols8) * 8;
     const long long r = i / cols8;
     const int side = (int)(r & 1);
+    if (side && T == 1) continue;
     const long long b = r >> 1;
     const int edge = side ? T + pad - 1 : pad;
+    const int last_side = T == 1 ? 1 : side;
     float acc[8];
     {
       uint4 u = *reinterpret_cast<const uint4*>(G + (b * Tp + edge) * ld + c);
@@ -242,16 +245,18 @@ fold_pad_kernel(__nv_bfloat16* __restrict__ G, long long ld, long long n_win, in
       t = unpack_bf16x2(u.z); acc[4] = t.x; acc[5] = t.y;
       t = unpack_bf16x2(u.w); acc[6] = t.x; acc[7] = t.y;
     }
-    for (int k = 0; k < pad; ++k) {
-      const int prow = side ? T + pad + k : k;
-      __nv_bfloat16* pp = G + (b * Tp + prow) * ld + c;
-      uint4 u = *reinterpret_cast<const uint4*>(pp);
-      float2 t;
-      t = unpack_bf16x2(u.x); acc[0] += t.x; acc[1] += t.y;
-      t = unpack_bf16x2(u.y); acc[2] += t.x; acc[3] += t.y;
-      t = unpack_bf16x2(u.z); acc[4] += t.x; acc[5] += t.y;
-      t = unpack_bf16x2(u.w); acc[6] += t.x; acc[7] += t.y;
-      *reinterpret_cast<uint4*>(pp) = make_uint4(0, 0, 0, 0);
+    for (int s = side; s <= last_side; ++s) {
+      for (int k = 0; k < pad; ++k) {
+        const int prow = s ? T + pad + k : k;
+        __nv_bfloat16* pp = G + (b * Tp + prow) * ld + c;
+        uint4 u = *reinterpret_cast<const uint4*>(pp);
+        float2 t;
+        t = unpack_bf16x2(u.x); acc[0] += t.x; acc[1] += t.y;
+        t = unpack_bf16x2(u.y); acc[2] += t.x; acc[3] += t.y;
+        t = unpack_bf16x2(u.z); acc[4] += t.x; acc[5] += t.y;
+        t = unpack_bf16x2(u.w); acc[6] += t.x; acc[7] += t.y;
+        *reinterpret_cast<uint4*>(pp) = make_uint4(0, 0, 0, 0);
+      }
     }
     *reinterpret_cast<uint4*>(G + (b * Tp + edge) * ld + c) =
         make_uint4(pack_bf16x2(acc[0], acc[1]), pack_bf16x2(acc[2], acc[3]), pack_bf16x2(acc[4], acc[5]), pack_bf16x2(acc[6], acc[7]));
@@ -299,8 +304,9 @@ conv_w_to_dgrad_kernel(const float* __restrict__ w, int cout, int cin, int kt, i
 extern "C" int ibm_replicate_pad_rows(void* X, int64_t ld, int64_t n_win, int32_t T, int32_t pad, int32_t cols, void* stream) {
   using namespace ibm;
   IBM_CHECK_ARCH();
-  IBM_CHECK_ARG(X && n_win > 0 && T > 0 && pad > 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0 && ld >= cols && aligned16(X),
+  IBM_CHECK_ARG(X && n_win > 0 && T > 0 && pad >= 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0 && ld >= cols && aligned16(X),
                 "replicate_pad_rows: bad argument (cols and ld must be multiples of 8)");
+  if (pad == 0) return IBM_OK;                                  // kernel size 1: no pad rows
   replicate_pad_kernel<<<ew_grid(n_win * 2 * pad * (cols / 8)), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       static_cast<__nv_bfloat16*>(X), ld, n_win, T, pad, cols / 8);
   IBM_LAUNCH_CHECK();
@@ -310,8 +316,9 @@ extern "C" int ibm_replicate_pad_rows(void* X, int64_t ld, int64_t n_win, int32_
 extern "C" int ibm_fold_pad_rows(void* G, int64_t ld, int64_t n_win, int32_t T, int32_t pad, int32_t cols, void* stream) {
   using namespace ibm;
   IBM_CHECK_ARCH();
-  IBM_CHECK_ARG(G && n_win > 0 && T > 0 && pad > 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0 && ld >= cols && aligned16(G),
+  IBM_CHECK_ARG(G && n_win > 0 && T > 0 && pad >= 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0 && ld >= cols && aligned16(G),
                 "fold_pad_rows: bad argument (cols and ld must be multiples of 8)");
+  if (pad == 0) return IBM_OK;                                  // kernel size 1: no pad rows
   fold_pad_kernel<<<ew_grid(n_win * 2 * (cols / 8)), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       static_cast<__nv_bfloat16*>(G), ld, n_win, T, pad, cols / 8);
   IBM_LAUNCH_CHECK();
