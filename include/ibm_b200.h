@@ -366,6 +366,14 @@ int ibm_optimizer_step(int32_t kind, float* param, const float* grad, float* sta
 int ibm_optimizer_step_dev(int32_t kind, float* param, const float* grad, float* state0, float* state1,
                            void* param_bf16, int64_t n, float lr, float grad_scale, const int64_t* step_dev,
                            void* stream);
+/* Builder-owned (DESIGN.md §0; NOT in the reference): the same step, and in the same pass an exponential moving average of the
+ * updated parameters in the fp32 arena `ema` (same offsets as param, 16-byte aligned):
+ *   d_n = min(ema_decay, (1 + n) / (10 + n))   (double; n = the 1-based step count)
+ *   ema <- ema + (float)(1 - d_n) * (param - ema)
+ * 0 < ema_decay < 1.  n = step, or *step_dev when step_dev != NULL (graph-replayed steps). */
+int ibm_optimizer_step_ema(int32_t kind, float* param, const float* grad, float* state0, float* state1,
+                           void* param_bf16, float* ema, int64_t n, float lr, float grad_scale, float ema_decay,
+                           int64_t step, const int64_t* step_dev, void* stream);
 /* *counter_dev += inc (one thread): the device-resident step counter of graph-replayed training steps. */
 int ibm_counter_add(int64_t* counter_dev, int64_t inc, void* stream);
 

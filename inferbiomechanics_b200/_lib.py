@@ -63,6 +63,7 @@ SIGNATURES = {
     "ibm_attention_bwd_long": [P, _i64, P, _i64, P, _i64, P, _i64, P, _i64, P, _i64, P, _i64, P, _i64, _i64, _i32, _i32, _i32, _i32, _f,
                                P, P, P, P],
     "ibm_optimizer_step_dev": [_i32, P, P, P, P, P, _i64, _f, _f, P, P],
+    "ibm_optimizer_step_ema": [_i32, P, P, P, P, P, P, _i64, _f, _f, _f, _i64, P, P],
     "ibm_counter_add": [P, _i64, P],
     "ibm_optimizer_step": [_i32, P, P, P, P, P, _i64, _f, _f, _i64, P],
     "ibm_device_check": [_i32],

@@ -85,7 +85,10 @@ class AbstractCommand:
         first_linear = min(int(k.split('.')[1]) for k, v in zip(keys, sd.values()) if k.endswith('.weight') and v.dim() == 2)
         return bn, first_linear - int(bn) == 1
 
-    def load_latest_checkpoint(self, model, optimizer=None, checkpoint_dir="../checkpoints"):
+    def load_latest_checkpoint(self, model, optimizer=None, checkpoint_dir="../checkpoints", *, state_key="model_state_dict"):
+        """Loads the newest ``epoch_{e}_batch_{i}.pt`` into ``model`` (and ``optimizer``); returns (epoch, batch), or (-1, 0)
+        if there is none.  ``state_key='ema_state_dict'`` loads the weight average ``train --ema-decay`` saved instead of
+        the trained weights; a checkpoint without that entry is a ValueError."""
         if not os.path.exists(checkpoint_dir):
             print("Checkpoint directory does not exist!")
             return -1, 0
@@ -98,7 +101,9 @@ class AbstractCommand:
         latest_checkpoint = os.path.join(checkpoint_dir, checkpoints[-1])
         logging.info(f"{latest_checkpoint=}")
         checkpoint = torch.load(latest_checkpoint, map_location="cpu")
-        sd = checkpoint['model_state_dict']
+        if state_key not in checkpoint:
+            raise ValueError(f"{latest_checkpoint} holds no {state_key!r} (was it trained with --ema-decay?)")
+        sd = checkpoint[state_key]
         if all(k.startswith('module.') for k in sd):
             sd = {k[len('module.'):]: v for k, v in sd.items()}
         model.load_state_dict(sd)

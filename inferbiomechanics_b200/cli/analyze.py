@@ -66,6 +66,9 @@ class AnalyzeCommand(AbstractCommand):
                         help='Reverse sampler for --model-type diffusion: the ancestral DDPM chain or few-step DDIM.')
         sp.add_argument('--eta', type=float, default=0.0,
                         help='DDIM noise scale in [0, 1] (0: deterministic given x_T; 1: respaced ancestral sampling).')
+        sp.add_argument('--ema', action='store_true', default=False,
+                        help="Evaluate the checkpoint's EMA weights (ema_state_dict, written by train --ema-decay) instead of "
+                             "the trained ones.")
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'analyze':
@@ -86,7 +89,7 @@ class AnalyzeCommand(AbstractCommand):
                                dropout=args.dropout or dropout, dropout_prob=0.0,
                                root_history_len=root_history_len, output_data_format=args.output_data_format,
                                device=str(device)).to(device)
-        self.load_latest_checkpoint(model, checkpoint_dir=checkpoint_dir)
+        self.load_latest_checkpoint(model, checkpoint_dir=checkpoint_dir, state_key='ema_state_dict' if args.ema else 'model_state_dict')
         model.eval()
         native = model_type == 'feedforward'
         trainer = Trainer(model, args=args) if native else None

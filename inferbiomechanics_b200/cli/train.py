@@ -12,6 +12,7 @@ Conscious fixes of reference defects that stop it running (SURVEY §0.4): ``DEV`
 from __future__ import annotations
 
 import argparse
+import contextlib
 import logging
 import os
 from typing import List
@@ -156,6 +157,10 @@ class TrainCommand(AbstractCommand):
         sp.add_argument('--dev-sampling-steps', type=int, default=0,
                         help='--model-type diffusion: score the dev set before each epoch on samples of this many DDIM steps '
                              '(eta = 0); 0 skips the dev pass of the denoiser.')
+        sp.add_argument('--ema-decay', type=float, default=0.0,
+                        help='Keep an exponential moving average of the weights with this decay (e.g. 0.999; warm-up '
+                             'min(decay, (1 + n) / (10 + n)) at step n), evaluate the dev set with it and save it in the '
+                             'checkpoints as ema_state_dict; 0 keeps none.')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'train':
@@ -164,6 +169,8 @@ class TrainCommand(AbstractCommand):
             raise NotImplementedError("--compute-report needs nimblephysics inverse dynamics (RegressionLossEvaluator.py:265-286)")
         if args.dev_sampling_steps < 0:
             raise ValueError(f"--dev-sampling-steps must be >= 0, got {args.dev_sampling_steps}")
+        if not 0.0 <= args.ema_decay < 1.0:
+            raise ValueError(f"--ema-decay must be in [0, 1), got {args.ema_decay}")
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
         root_history_len = 10
@@ -195,7 +202,7 @@ class TrainCommand(AbstractCommand):
 
         native = model_type in ('feedforward', 'groundlink', 'diffusion')
         if native:
-            trainer = Trainer(model, opt_type=args.opt_type, lr=args.learning_rate, args=args, seed=1234)
+            trainer = Trainer(model, opt_type=args.opt_type, lr=args.learning_rate, args=args, seed=1234, ema_decay=args.ema_decay)
             optimizer = None
         else:
             if world > 1:
@@ -208,6 +215,11 @@ class TrainCommand(AbstractCommand):
                                                           optimizer=_TrainerOptimizer(trainer) if native else optimizer)
         if native and epoch_checkpoint >= 0:
             trainer.arena.sync_shadow(force=True)        # parameters were replaced under the engine
+            if trainer.ema is not None:
+                # the average resumes from the checkpoint, or starts at the loaded weights if that run kept none
+                ck = torch.load(self.latest_checkpoint_path(checkpoint_dir), map_location="cpu")
+                trainer.load_ema_state_dict(ck.get('ema_state_dict'))
+        use_ema = native and trainer.ema is not None
 
         train_batches = WindowStore.batches(train_store.shard(rank, world), args.batch_size)
         dev_batches = WindowStore.batches(dev_store.shard(rank, world), args.batch_size)
@@ -220,7 +232,7 @@ class TrainCommand(AbstractCommand):
 
         for epoch in range(epoch_checkpoint + 1, args.epochs):
             print(f'[{rank=}] Evaluating Dev Set Before Epoch {epoch}')
-            with torch.no_grad():
+            with torch.no_grad(), (trainer.ema_weights() if use_ema else contextlib.nullcontext()):
                 model.eval()
                 if model_type != 'diffusion' or dev_diffusion is not None:
                     for i, idx in enumerate(dev_batches):
@@ -234,7 +246,7 @@ class TrainCommand(AbstractCommand):
                             dev_ev(inputs, model(inputs), label_dict(dev_store, idx), [], [], args)
                         if (i + 1) % 100 == 0 or i == len(dev_batches) - 1:
                             print('  - Dev Batch ' + str(i + 1) + '/' + str(len(dev_batches)))
-                print(f'[{rank=}] Dev Set Evaluation: ')
+                print(f'[{rank=}] Dev Set Evaluation' + (' (EMA weights)' if use_ema else '') + ': ')
                 print_all_ranks_report(dev_log.ev if native else dev_ev, args, rank, world, device)
                 (dev_log if native else dev_ev).print_report(args, log_to_wandb=log_to_wandb)
             if world > 1:
@@ -259,9 +271,12 @@ class TrainCommand(AbstractCommand):
                     if rank == 0:                              # avoid redundant saving across processes
                         model_path = f"{checkpoint_dir}/epoch_{epoch}_batch_{i}.pt"
                         os.makedirs(os.path.dirname(model_path), exist_ok=True)
-                        torch.save({'epoch': epoch, 'model_state_dict': model.state_dict(),
-                                    'optimizer_state_dict': optimizer.state_dict() if optimizer is not None else
-                                    trainer.optimizer_state_dict()}, model_path)
+                        ck = {'epoch': epoch, 'model_state_dict': model.state_dict(),
+                              'optimizer_state_dict': optimizer.state_dict() if optimizer is not None else
+                              trainer.optimizer_state_dict()}
+                        if use_ema:
+                            ck['ema_state_dict'] = trainer.ema_state_dict()
+                        torch.save(ck, model_path)
             logging.info('-' * 80)
             logging.info(f'[{rank=}] Epoch {epoch}/{args.epochs} Training Set Evaluation: ')
             logging.info('-' * 80)

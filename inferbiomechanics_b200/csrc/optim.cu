@@ -1,7 +1,7 @@
 // Fused optimizer step over the flat fp32 parameter arena.  One launch updates parameters and
 // optimizer state in place, applies the data-parallel 1/world_size gradient scale, and refreshes
 // the bf16 shadow weights the tcgen05 GEMMs read.  HBM-bound (RMSprop: 12 B read + 10 B written
-// per parameter).
+// per parameter; an exponential moving average of the weights adds 4 B read + 4 B written).
 //
 // Replaces torch.optim.{RMSprop,Adam,SGD,Adagrad,Adadelta,Adamax}(lr) with torch defaults as
 // constructed at /root/reference/src/cli/train.py:183-197 and stepped at :284.
@@ -15,7 +15,16 @@ struct OptArgs {
   float lr, gscale;
   float bc1, bc2_sqrt;   // Adam / Adamax bias corrections for this step
   const long long* step_dev;   // optional device-resident step count (CUDA-graph replays): the corrections are derived from it
+  float* ema;            // EMA instantiation only: fp32 arena with the parameters' offsets
+  double ema_decay;      // the EMA's decay cap
+  float ema_w;           // 1 - d_n of this step (derived from step_dev when given)
 };
+
+// torch_ema's use_num_updates warm-up: d_n = min(decay, (1 + n) / (10 + n)), n = the 1-based step count, in double
+__host__ __device__ inline float ema_weight(double decay, double n) {
+  const double d = fmin(decay, (1.0 + n) / (10.0 + n));
+  return (float)(1.0 - d);
+}
 
 template <int KIND>
 __device__ __forceinline__ void opt_update(float& p, float g, float& s0, float& s1, const OptArgs& a) {
@@ -44,7 +53,9 @@ __device__ __forceinline__ void opt_update(float& p, float g, float& s0, float& 
   }
 }
 
-template <int KIND>
+__device__ __forceinline__ float ema_update(float e, float p, float w) { return fmaf(w, p - e, e); }
+
+template <int KIND, bool EMA>
 __global__ void __launch_bounds__(kThreads)
 optimizer_kernel(float* __restrict__ param, const float* __restrict__ grad, float* __restrict__ st0,
                  float* __restrict__ st1, __nv_bfloat16* __restrict__ pb, long long n, OptArgs a) {
@@ -62,6 +73,15 @@ optimizer_kernel(float* __restrict__ param, const float* __restrict__ grad, floa
       a.bc2_sqrt = s_bc[1];
     }
   }
+  if constexpr (EMA) {
+    if (a.step_dev != nullptr) {
+      __shared__ float s_w;
+      if (threadIdx.x == 0) s_w = ema_weight(a.ema_decay, (double)__ldg(a.step_dev));
+      __syncthreads();
+      a.ema_w = s_w;
+    }
+  }
+  float* __restrict__ ema = a.ema;
   const long long n4 = n >> 2;
   const long long stride = (long long)gridDim.x * blockDim.x;
   constexpr bool kS0 = KIND != 2, kS1 = (KIND == 1 || KIND == 4 || KIND == 5);
@@ -78,6 +98,12 @@ optimizer_kernel(float* __restrict__ param, const float* __restrict__ grad, floa
     if (kS0) *reinterpret_cast<float4*>(st0 + 4 * i) = s0;
     if (kS1) *reinterpret_cast<float4*>(st1 + 4 * i) = s1;
     if (pb) *reinterpret_cast<uint2*>(pb + 4 * i) = make_uint2(pack_bf16x2(p.x, p.y), pack_bf16x2(p.z, p.w));
+    if constexpr (EMA) {
+      float4 e = *reinterpret_cast<const float4*>(ema + 4 * i);
+      e = make_float4(ema_update(e.x, p.x, a.ema_w), ema_update(e.y, p.y, a.ema_w), ema_update(e.z, p.z, a.ema_w),
+                      ema_update(e.w, p.w, a.ema_w));
+      *reinterpret_cast<float4*>(ema + 4 * i) = e;
+    }
   }
   for (long long i = (n4 << 2) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     float p = param[i], s0 = kS0 ? st0[i] : 0.f, s1 = kS1 ? st1[i] : 0.f;
@@ -86,17 +112,32 @@ optimizer_kernel(float* __restrict__ param, const float* __restrict__ grad, floa
     if (kS0) st0[i] = s0;
     if (kS1) st1[i] = s1;
     if (pb) pb[i] = __float2bfloat16_rn(p);
+    if constexpr (EMA) ema[i] = ema_update(ema[i], p, a.ema_w);
+  }
+}
+
+template <bool EMA>
+static void launch_optimizer(int32_t kind, int grid, cudaStream_t s, float* param, const float* grad, float* state0, float* state1,
+                             __nv_bfloat16* pb, long long n, const OptArgs& a) {
+  switch (kind) {
+    case 0: optimizer_kernel<0, EMA><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
+    case 1: optimizer_kernel<1, EMA><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
+    case 2: optimizer_kernel<2, EMA><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
+    case 3: optimizer_kernel<3, EMA><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
+    case 4: optimizer_kernel<4, EMA><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
+    default: optimizer_kernel<5, EMA><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
   }
 }
 
 }  // namespace ibm
 
 static int optimizer_step_impl(int32_t kind, float* param, const float* grad, float* state0, float* state1, void* param_bf16,
-                               int64_t n, float lr, float grad_scale, int64_t step, const int64_t* step_dev, void* stream);
+                               float* ema, int64_t n, float lr, float grad_scale, float ema_decay, int64_t step,
+                               const int64_t* step_dev, void* stream);
 
 extern "C" int ibm_optimizer_step(int32_t kind, float* param, const float* grad, float* state0, float* state1,
                                   void* param_bf16, int64_t n, float lr, float grad_scale, int64_t step, void* stream) {
-  return optimizer_step_impl(kind, param, grad, state0, state1, param_bf16, n, lr, grad_scale, step, nullptr, stream);
+  return optimizer_step_impl(kind, param, grad, state0, state1, param_bf16, nullptr, n, lr, grad_scale, 0.f, step, nullptr, stream);
 }
 
 extern "C" int ibm_optimizer_step_dev(int32_t kind, float* param, const float* grad, float* state0, float* state1,
@@ -105,11 +146,23 @@ extern "C" int ibm_optimizer_step_dev(int32_t kind, float* param, const float* g
     ibm::set_error("optimizer_step_dev: null step counter");
     return IBM_E_ARG;
   }
-  return optimizer_step_impl(kind, param, grad, state0, state1, param_bf16, n, lr, grad_scale, 1, step_dev, stream);
+  return optimizer_step_impl(kind, param, grad, state0, state1, param_bf16, nullptr, n, lr, grad_scale, 0.f, 1, step_dev, stream);
+}
+
+extern "C" int ibm_optimizer_step_ema(int32_t kind, float* param, const float* grad, float* state0, float* state1,
+                                      void* param_bf16, float* ema, int64_t n, float lr, float grad_scale, float ema_decay,
+                                      int64_t step, const int64_t* step_dev, void* stream) {
+  if (ema == nullptr) {
+    ibm::set_error("optimizer_step_ema: null EMA arena");
+    return IBM_E_ARG;
+  }
+  return optimizer_step_impl(kind, param, grad, state0, state1, param_bf16, ema, n, lr, grad_scale, ema_decay,
+                             step_dev ? 1 : step, step_dev, stream);
 }
 
 static int optimizer_step_impl(int32_t kind, float* param, const float* grad, float* state0, float* state1, void* param_bf16,
-                               int64_t n, float lr, float grad_scale, int64_t step, const int64_t* step_dev, void* stream) {
+                               float* ema, int64_t n, float lr, float grad_scale, float ema_decay, int64_t step,
+                               const int64_t* step_dev, void* stream) {
   using namespace ibm;
   IBM_CHECK_ARCH();
   IBM_CHECK_ARG(kind >= 0 && kind <= 5, "optimizer_step: unknown optimizer kind %d", kind);
@@ -117,27 +170,28 @@ static int optimizer_step_impl(int32_t kind, float* param, const float* grad, fl
   IBM_CHECK_ARG(kind == 2 || state0, "optimizer_step: state0 required");
   IBM_CHECK_ARG(!(kind == 1 || kind == 4 || kind == 5) || state1, "optimizer_step: state1 required");
   IBM_CHECK_ARG(aligned16(param) && aligned16(grad) && (!state0 || aligned16(state0)) && (!state1 || aligned16(state1)) &&
-                    (!param_bf16 || (reinterpret_cast<uintptr_t>(param_bf16) % 8 == 0)),
+                    (!ema || aligned16(ema)) && (!param_bf16 || (reinterpret_cast<uintptr_t>(param_bf16) % 8 == 0)),
                 "optimizer_step: arenas must be 16-byte aligned");
+  IBM_CHECK_ARG(!ema || (ema_decay > 0.f && ema_decay < 1.f), "optimizer_step: EMA decay must be in (0, 1), got %g",
+                (double)ema_decay);
   OptArgs a;
   a.lr = lr;
   a.gscale = grad_scale;
   a.bc1 = (float)(1.0 - pow(0.9, (double)step));
   a.bc2_sqrt = (float)sqrt(1.0 - pow(0.999, (double)step));
   a.step_dev = reinterpret_cast<const long long*>(step_dev);
+  a.ema = ema;
+  a.ema_decay = (double)ema_decay;
+  a.ema_w = ema_weight(a.ema_decay, (double)step);
   long long need = ceil_div(n / 4 + 1, kThreads);
   long long cap = (long long)sm_count() * 16;
   const int grid = (int)(need < cap ? need : cap);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   auto* pb = static_cast<__nv_bfloat16*>(param_bf16);
-  switch (kind) {
-    case 0: optimizer_kernel<0><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
-    case 1: optimizer_kernel<1><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
-    case 2: optimizer_kernel<2><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
-    case 3: optimizer_kernel<3><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
-    case 4: optimizer_kernel<4><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
-    default: optimizer_kernel<5><<<grid, kThreads, 0, s>>>(param, grad, state0, state1, pb, n, a); break;
-  }
+  if (ema)
+    launch_optimizer<true>(kind, grid, s, param, grad, state0, state1, pb, n, a);
+  else
+    launch_optimizer<false>(kind, grid, s, param, grad, state0, state1, pb, n, a);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }

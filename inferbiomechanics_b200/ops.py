@@ -333,8 +333,17 @@ def pack_labels(raw, nb, win_row0, contact_idx, mass, F, stride, last_only, out_
 
 
 # ---- optimizer ----------------------------------------------------------------------------------------
-def optimizer_step(kind: str, param, grad, state0, state1, param_bf16, lr, grad_scale, step, step_dev=None):
-    """``step_dev`` (device int64[1]) replaces the by-value 1-based step count (graph-replayed steps)."""
+def optimizer_step(kind: str, param, grad, state0, state1, param_bf16, lr, grad_scale, step, step_dev=None, ema=None,
+                   ema_decay=0.0):
+    """``step_dev`` (device int64[1]) replaces the by-value 1-based step count (graph-replayed steps).  ``ema`` (fp32, the
+    parameters' layout): also updates this exponential moving average of the parameters in the same pass, decay
+    min(``ema_decay``, (1 + n) / (10 + n)) at step n."""
+    if ema is not None:
+        if ema.numel() != param.numel() or ema.dtype != torch.float32:
+            raise ValueError(f"EMA arena must be fp32 with {param.numel()} elements, got {ema.dtype} x {ema.numel()}")
+        call("ibm_optimizer_step_ema", _lib.OPT_KIND[kind], _p(param), _p(grad), _p(state0), _p(state1), _p(param_bf16), _p(ema),
+             param.numel(), lr, grad_scale, ema_decay, step, _p(step_dev), stream_ptr())
+        return
     if step_dev is not None:
         call("ibm_optimizer_step_dev", _lib.OPT_KIND[kind], _p(param), _p(grad), _p(state0), _p(state1), _p(param_bf16), param.numel(),
              lr, grad_scale, _p(step_dev), stream_ptr())

@@ -17,9 +17,10 @@ drop-in classes remain usable with the reference's own autograd loop; this is th
 from __future__ import annotations
 
 import argparse
+import contextlib
 import gc
 import os
-from typing import Dict, List, Optional
+from typing import Dict, Iterator, List, Optional
 
 import torch
 
@@ -57,7 +58,9 @@ def _time_kernel(fn, iters: int = 20) -> float:
 
 class Trainer:
     def __init__(self, model, opt_type: str = "rmsprop", lr: float = 1e-4, args: Optional[argparse.Namespace] = None,
-                 diffusion: Optional[GaussianDiffusion] = None, bucket_mb: float = 8.0, seed: int = 0):
+                 diffusion: Optional[GaussianDiffusion] = None, bucket_mb: float = 8.0, seed: int = 0, ema_decay: float = 0.0):
+        if not 0.0 <= ema_decay < 1.0:
+            raise ValueError(f"ema_decay must be in [0, 1) (0 = no EMA), got {ema_decay}")
         self.model = model
         self.eng = model.engine()
         self.arena = model.arena
@@ -87,6 +90,11 @@ class Trainer:
         # DDP constructor semantics: everyone starts from rank 0's parameters (train.py:175)
         self.bucketer.broadcast_(self.arena.master)
         self.arena.sync_shadow(force=True)
+        # exponential moving average of the weights, updated by the optimizer kernel: taken after the broadcast, it stays
+        # identical across data-parallel ranks because their masters are bit-identical after every step
+        self.ema_decay = float(ema_decay)
+        self.ema: Optional[torch.Tensor] = self.arena.master.clone() if ema_decay > 0 else None
+        self._in_ema = False
         # device-resident 1-based step counter: incremented by a one-thread kernel at the start of every step, read by the
         # dropout kernels (Philox offset) and the optimizer kernel (Adam / Adamax bias correction), so that a captured step
         # can be replayed although those values change from step to step
@@ -241,8 +249,73 @@ class Trainer:
     def optimizer_step(self) -> None:
         self.step_count += 1
         ops.optimizer_step(self.opt_type, self.arena.master, self.arena.grad, self.state0, self.state1, self.arena.shadow,
-                           self.lr, 1.0 / self.world, self.step_count, step_dev=self.step_dev)
+                           self.lr, 1.0 / self.world, self.step_count, step_dev=self.step_dev, ema=self.ema,
+                           ema_decay=self.ema_decay)
         self.arena.mark_shadow_fresh()
+
+    # ---- exponential moving average of the weights -------------------------------------------------------------------
+    def _require_ema(self) -> None:
+        if self.ema is None:
+            raise RuntimeError("this Trainer keeps no EMA of the weights (construct it with ema_decay > 0)")
+
+    def ema_state_dict(self) -> dict:
+        """``model.state_dict()``'s keys with the parameters taken from the EMA arena and the buffers (BatchNorm running
+        statistics) copied from the model, so ``model.load_state_dict`` of any instance of the class accepts it."""
+        self._require_ema()
+        out = {}
+        for k, v in self.model.state_dict().items():
+            if k in self.arena.offsets:
+                o, n = self.arena.offsets[k]
+                out[k] = self.ema[o:o + n].view(v.shape).clone()
+            else:
+                out[k] = v.clone()
+        return out
+
+    def load_ema_state_dict(self, sd: Optional[dict]) -> None:
+        """Inverse of ``ema_state_dict``: the parameters' entries go into the EMA arena (buffers are the model's own).
+        ``None`` restarts the average at the current weights (a resumed run whose checkpoint holds no EMA)."""
+        self._require_ema()
+        if sd is None:
+            self.ema.copy_(self.arena.master)
+            return
+        if all(k.startswith("module.") for k in sd):
+            sd = {k[len("module."):]: v for k, v in sd.items()}
+        keys = self.model.state_dict().keys()
+        missing = [k for k in self.arena.names if k not in sd]
+        unexpected = [k for k in sd if k not in keys]
+        if missing or unexpected:
+            raise ValueError(f"EMA state dict does not match the model: missing {missing}, unexpected {unexpected}")
+        for name in self.arena.names:
+            o, n = self.arena.offsets[name]
+            if sd[name].numel() != n:
+                raise ValueError(f"EMA entry {name} has {sd[name].numel()} elements, the parameter {n}")
+            self.ema[o:o + n].copy_(sd[name].reshape(-1))
+
+    def _swap_ema(self) -> None:
+        """Exchanges the contents (never the storage: captured graphs hold the pointers) of the masters and the EMA arena,
+        then re-derives the bf16 shadow, the padded copies and, through the version bump, every cache keyed on
+        ``ParamArena.version``.  Parameters are views re-pointed into the masters, so a copy into the masters does not move
+        their ``_version``: the bump is what makes the Groundlink conv layouts and the denoiser's time-MLP table refresh."""
+        tmp = self.arena.master.clone()
+        self.arena.master.copy_(self.ema)
+        self.ema.copy_(tmp)
+        self.arena.sync_shadow(force=True)
+        self.arena.bump_version()
+
+    @contextlib.contextmanager
+    def ema_weights(self) -> Iterator[None]:
+        """Evaluates (``eval_step``, the model's forward, sampling) with the EMA weights in the masters; the trained weights
+        are back on exit."""
+        self._require_ema()
+        if self._in_ema:
+            raise RuntimeError("already inside ema_weights()")
+        self._in_ema = True
+        self._swap_ema()
+        try:
+            yield
+        finally:
+            self._swap_ema()
+            self._in_ema = False
 
     # ---- optimizer state in torch.optim's own state_dict layout (checkpoints, train.py:270-278) -----------------------
     _OPT_CLASS = {"adagrad": "Adagrad", "adam": "Adam", "sgd": "SGD", "rmsprop": "RMSprop", "adadelta": "Adadelta", "adamax": "Adamax"}
