@@ -221,15 +221,18 @@ int ibm_add_time_pos_bwd(const void* dh_bf16, int64_t ld, void* dtemb_bf16, int6
  *   A: bf16, logical [M,K]. a_mn_major==0: stored row-major [M,K] (ld=lda).
  *                           a_mn_major==1: stored row-major [K,M] (ld=lda)  (i.e. A^T in memory).
  *   B: bf16, logical [N,K]. b_mn_major likewise ([N,K] vs [K,N] in memory).
- *   bias: fp32[N] or NULL.  act: IBM_ACT_* applied to (acc + bias).
- *   aux: bf16 [M,N] (ld=ldaux) or NULL; aux_mode 1: out = act(acc+bias) + aux   (residual)
+ *   bias: fp32[N], 16-byte aligned, or NULL.  act: IBM_ACT_* applied to (acc + bias).
+ *   aux: bf16 [M,N] (ld=ldaux) or NULL; aux_mode 1: out = act(acc+bias) + aux   (residual; act none/relu/elu)
  *                                        aux_mode 2: out = (acc+bias) * act'(aux) (aux = saved
- *                                        activation OUTPUT; dgrad through relu/sigmoid/tanh/elu)
+ *                                        activation OUTPUT; dgrad through none/relu/sigmoid/tanh/elu)
+ *   Other act with aux, and any act with mask_mode 2, are rejected (IBM_E_ARG).
  *   out: out_dtype IBM_BF16 | IBM_F32, row-major [M,N] (ld=ldd).
  *   accumulate!=0 (requires IBM_F32 out, no act/aux): D += A·B^T via TMA reduce-add; the K range is
  *   split over `split_k` CTAs (weight gradients: K = tokens).  split_k<=0 ⇒ chosen by the library.
  *   taps>1: A rows are shifted by tap index: K is taps*K_tap, k-block kb reads A rows
- *   m + (kb / kb_per_tap) (implicit-GEMM temporal convolution, Groundlink.py:41).
+ *   m + (kb / kb_per_tap) (implicit-GEMM temporal convolution, Groundlink.py:41).  B holds taps blocks of
+ *   round_up(K_tap, 64) k: tap j's weights start at k = j * round_up(K_tap, 64) (B is [N, taps*round_up(K_tap, 64)],
+ *   or its transpose when MN-major).
  *   colsum_out: NULL, or fp32[N] that the column sums of the bf16 output (rows < M, as rounded) are
  *   ADDED to by the epilogue: when D is the gradient w.r.t. a layer's pre-activation this is that
  *   layer's bias gradient (nn.Linear bias, TransformerBaseline.py:15) without another pass over D.

@@ -602,7 +602,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           if (kAux) {
             epi_dispatch_aux<PT>(v, smem_u32(my_aux + xb * kWarpStage + lane * 128), rsw, args.act, args.aux_mode, kAuxRegs ? ax : nullptr);
           } else {
-            epi_dispatch_plain<PT>(v, args.act);
+            // fp32 aux_mode 2 (below): (acc + bias) * act'(aux), no act; bf16 kernels without kAux never see aux
+            if (!kOutF32 || args.aux_mode != 2) epi_dispatch_plain<PT>(v, args.act);
             if constexpr (!kOutF32) {
               if (mask_mode == 1) {
                 // the sign pattern of the (post-activation) outputs: what the dgrad of this layer needs instead of the
@@ -805,6 +806,12 @@ extern "C" int ibm_gemm_bf16(const void* A, int64_t lda, int32_t a_mn_major, con
   IBM_CHECK_ARG(act >= 0 && act <= IBM_ACT_SILU, "gemm: bad activation %d", act);
   IBM_CHECK_ARG(aux_mode >= 0 && aux_mode <= 2 && (aux_mode == 0 || aux != nullptr), "gemm: bad aux mode");
   IBM_CHECK_ARG(aux_mode == 0 || (ldaux % 8 == 0 && aligned16(aux)), "gemm: aux must be 16-byte aligned with ld %% 8 == 0");
+  // the epilogues instantiated for aux: the residual add after none / relu / elu, and every derivative that follows from
+  // the activation's output (SiLU's does not)
+  IBM_CHECK_ARG(aux_mode != 1 || act == IBM_ACT_NONE || act == IBM_ACT_RELU || act == IBM_ACT_ELU,
+                "gemm: aux_mode 1 (residual) supports act none, relu or elu, got %d", act);
+  IBM_CHECK_ARG(aux_mode != 2 || act != IBM_ACT_SILU, "gemm: aux_mode 2 needs act' from the activation output: not silu");
+  IBM_CHECK_ARG(bias == nullptr || aligned16(bias), "gemm: bias must be 16-byte aligned");
   IBM_CHECK_ARG(!accumulate || (out_dtype == IBM_F32 && act == IBM_ACT_NONE && aux_mode == 0 && bias == nullptr),
                 "gemm: accumulate mode needs fp32 output and a plain epilogue");
   IBM_CHECK_ARG(colsum_out == nullptr || (out_dtype == IBM_BF16 && !accumulate), "gemm: colsum_out needs a bf16 output");
@@ -812,6 +819,7 @@ extern "C" int ibm_gemm_bf16(const void* A, int64_t lda, int32_t a_mn_major, con
   IBM_CHECK_ARG(mask_mode == 0 || (mask != nullptr && out_dtype == IBM_BF16 && !accumulate && aux_mode == 0 && N % 64 == 0 &&
                                    ldmask % 8 == 0 && ldmask * 8 >= N && (reinterpret_cast<uintptr_t>(mask) & 7) == 0),
                 "gemm: sign bitmask needs a bf16 output without aux, N %% 64 == 0 and an 8-byte aligned mask with ldmask %% 8 == 0");
+  IBM_CHECK_ARG(mask_mode != 2 || act == IBM_ACT_NONE, "gemm: mask_mode 2 gates acc + bias: act must be none");
   if (taps < 1) taps = 1;
   IBM_CHECK_ARG(taps == 1 || (!a_mn_major && K % taps == 0 && (K / taps) % 8 == 0), "gemm: taps needs K-major A and K/taps %% 8 == 0");
 
@@ -897,7 +905,8 @@ extern "C" int ibm_gemm_bf16(const void* A, int64_t lda, int32_t a_mn_major, con
     pf_aux = (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 0;
   }
   args.pf_aux = pf_aux;
-  // With taps the B operand is [N, taps * kb_per_tap * 64] (each tap's K padded to whole k blocks).
+  // With taps the B operand is [N, taps * kb_per_tap * 64] (each tap's K padded to whole k blocks; [taps * kb_per_tap * 64, N]
+  // when MN-major).
   const int64_t Kb = taps == 1 ? K : (int64_t)args.kb_total * BLOCK_K;
 
   CUtensorMap ta, tb, td;
@@ -906,7 +915,7 @@ extern "C" int ibm_gemm_bf16(const void* A, int64_t lda, int32_t a_mn_major, con
   else rc = make_map(&ta, A, false, M, K, lda, 64, BLOCK_K);
   if (rc) return rc;
   if (!args.b_mn) rc = make_map(&tb, B, false, Kb, N, ldb, BLOCK_K, (uint32_t)(bn / cg));
-  else rc = make_map(&tb, B, false, N, K, ldb, 64, BLOCK_K);
+  else rc = make_map(&tb, B, false, N, Kb, ldb, 64, BLOCK_K);
   if (rc) return rc;
   const bool f32 = out_dtype == IBM_F32;
   rc = make_map(&td, D, f32, N, M, ldd, f32 ? 32 : 64, 32);           // one epilogue warp's 32-row tile

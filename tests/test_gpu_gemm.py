@@ -50,7 +50,7 @@ def _check(out, ref, bf16_out, what):
     (6, 24, 40, "tanh", False),
     (200, 8, 64, "none", False),
     (200, 12, 64, "none", True),
-    (5000, 512, 1472, "sigmoid", False),     # supertile (two column tiles per work item), bf16 and fp32 outputs
+    (5000, 512, 1472, "sigmoid", False),     # K >= 1024 but 20 row blocks x 1 column-tile pair < 148: single column tiles
     (777, 1000, 2048, "none", True),
     (70000, 512, 1024, "relu", False),
     (40000, 1536, 512, "none", False),       # >= 148 row blocks, K <= 512 (also the A-stationary schedule when IBM_GEMM_AS=1)
@@ -76,8 +76,9 @@ def test_gemm_forward(M, N, K, act, out_f32):
         assert torch.all(out[:, n_touched:].float() == 7.0)
 
 
+# of the K >= 1024 shapes only (20000, 1024, 1536) has enough work items for two-tile supertiles
 @pytest.mark.parametrize("M,N,K", [(515, 512, 256), (300, 200, 128), (40000, 512, 512), (1000, 2048, 512),
-                                   (3000, 512, 2048), (20000, 1024, 1536), (300, 504, 1024)])     # K >= 1024: two-tile supertiles
+                                   (3000, 512, 2048), (20000, 1024, 1536), (300, 504, 1024)])
 def test_gemm_residual_and_dact(M, N, K):
     from inferbiomechanics_b200 import ops
     A, B = _mk(M, K, K, 4), _mk(N, K, K, 5, 1.0 / math.sqrt(K))
