@@ -377,6 +377,33 @@ int ibm_optimizer_step_dev(int32_t kind, float* param, const float* grad, float*
 int ibm_optimizer_step_ema(int32_t kind, float* param, const float* grad, float* state0, float* state1,
                            void* param_bf16, float* ema, int64_t n, float lr, float grad_scale, float ema_decay,
                            int64_t step, const int64_t* step_dev, void* stream);
+/* Builder-owned (DESIGN.md §0; NOT in the reference): global gradient norm and clip coefficient of
+ * torch.nn.utils.clip_grad_norm_(params, max_norm) over the flat fp32 gradient arena (16-byte aligned):
+ *   total = grad_scale * ||grad||_2   (fp64 per thread and per block, deterministic last-block reduction, rounded to fp32)
+ *   coef  = min(1, max_norm / (total + 1e-6))   (fp32, as torch; a NaN total gives a NaN coefficient)
+ * out = {total, coef} (device float[2]).  The norm covers the whole arena, so the alignment padding between parameters
+ * must be zero, which it is when the arena is cleared as a whole before backward and nothing writes the padding.
+ * Workspace, caller-owned: partials = 1024 doubles, counter = one uint32 that is zero before the first call (the kernel
+ * resets it).  record (nullable, device double[3]): += {total, 1, coef < 1 ? 1 : 0}, a running sum for reports.
+ * No allocation, host synchronisation or host read: the call can be captured in a CUDA graph.  Two calls on the same
+ * arena and device give bit-identical outputs; max_norm > 0. */
+int ibm_grad_clip_coef(const float* grad, int64_t n, float grad_scale, float max_norm, float* out, double* partials,
+                       uint32_t* counter, double* record, void* stream);
+/* Builder-owned (DESIGN.md §0; NOT in the reference): ibm_optimizer_step_ema with `ema` nullable, a clip coefficient and a
+ * learning-rate schedule, both applied on the device so that a captured step replays with the values of its own step:
+ *   gradient = (grad * grad_scale) * clip[1]   (clip: the float[2] of ibm_grad_clip_coef, or NULL for no clipping)
+ *   lr_n     = (float)((double)lr * lambda(n)), n = the 1-based step (step, or *step_dev when step_dev != NULL), with
+ *     lambda(n) = n / W                                    for W > 0 and n <= W   (linear warm-up, W = warmup_steps)
+ *               = 1                                        after the warm-up, sched 0 (constant)
+ *               = r + (1 - r) (1 + cos(pi p)) / 2          after the warm-up, sched 1 (cosine), r = lr_min / lr,
+ *                 p = clamp((n - W) / (S - W), 0, 1), S = total_steps
+ * lr_n is the rate torch.optim.lr_scheduler.LambdaLR(opt, lambda s: lambda(s + 1)) hands to the optimizer's n-th step().
+ * warmup_steps >= 0; sched 1 needs total_steps > warmup_steps; 0 <= lr_min <= lr.  With clip[1] == 1 and lambda == 1 the
+ * update is bit-identical to ibm_optimizer_step_dev / _ema (both factors multiply by exactly 1). */
+int ibm_optimizer_step_sched(int32_t kind, float* param, const float* grad, float* state0, float* state1,
+                             void* param_bf16, float* ema, int64_t n, float lr, float grad_scale, float ema_decay,
+                             int64_t step, const int64_t* step_dev, const float* clip, int32_t sched,
+                             int64_t warmup_steps, int64_t total_steps, float lr_min, void* stream);
 /* *counter_dev += inc (one thread): the device-resident step counter of graph-replayed training steps. */
 int ibm_counter_add(int64_t* counter_dev, int64_t inc, void* stream);
 

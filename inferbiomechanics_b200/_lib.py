@@ -64,6 +64,8 @@ SIGNATURES = {
                                P, P, P, P],
     "ibm_optimizer_step_dev": [_i32, P, P, P, P, P, _i64, _f, _f, P, P],
     "ibm_optimizer_step_ema": [_i32, P, P, P, P, P, P, _i64, _f, _f, _f, _i64, P, P],
+    "ibm_grad_clip_coef": [P, _i64, _f, _f, P, P, P, P, P],
+    "ibm_optimizer_step_sched": [_i32, P, P, P, P, P, P, _i64, _f, _f, _f, _i64, P, P, _i32, _i64, _i64, _f, P],
     "ibm_counter_add": [P, _i64, P],
     "ibm_optimizer_step": [_i32, P, P, P, P, P, _i64, _f, _f, _i64, P],
     "ibm_device_check": [_i32],

@@ -25,7 +25,7 @@ from ..data.window_store import WindowStore
 from ..diffusion import GaussianDiffusion
 from ..keys import LOSS_QUANTITIES, MODEL_INPUT_ORDER
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
-from ..trainer import Trainer
+from ..trainer import LR_SCHEDULES, Trainer, check_clip_sched
 from . import _data
 from .abstract_command import AbstractCommand
 
@@ -161,6 +161,15 @@ class TrainCommand(AbstractCommand):
                         help='Keep an exponential moving average of the weights with this decay (e.g. 0.999; warm-up '
                              'min(decay, (1 + n) / (10 + n)) at step n), evaluate the dev set with it and save it in the '
                              'checkpoints as ema_state_dict; 0 keeps none.')
+        sp.add_argument('--clip-grad-norm', type=float, default=0.0,
+                        help='Scale the gradient down to this global L2 norm when it is larger (torch.nn.utils.clip_grad_norm_); '
+                             'each training report adds the mean pre-clip norm and the number of clipped steps. 0 = off.')
+        sp.add_argument('--lr-warmup-steps', type=int, default=0,
+                        help='Raise the learning rate linearly from lr / W to lr over the first W optimizer steps (0 = off).')
+        sp.add_argument('--lr-schedule', type=str, default='constant', choices=list(LR_SCHEDULES),
+                        help='Learning rate after the warm-up: constant, or a cosine decay to --lr-min at the last step of '
+                             'the run (epochs x batches per epoch).')
+        sp.add_argument('--lr-min', type=float, default=0.0, help='Final learning rate of the cosine schedule.')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'train':
@@ -171,6 +180,8 @@ class TrainCommand(AbstractCommand):
             raise ValueError(f"--dev-sampling-steps must be >= 0, got {args.dev_sampling_steps}")
         if not 0.0 <= args.ema_decay < 1.0:
             raise ValueError(f"--ema-decay must be in [0, 1), got {args.ema_decay}")
+        # the cosine's length (epochs x batches per epoch) is checked once the training store is open
+        check_clip_sched(args.learning_rate, args.clip_grad_norm, args.lr_warmup_steps, 'constant', args.lr_min, None, flag='--')
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
         root_history_len = 10
@@ -200,9 +211,21 @@ class TrainCommand(AbstractCommand):
             logging.error('Invalid optimizer type: ' + args.opt_type)
             assert (False)
 
+        train_batches = WindowStore.batches(train_store.shard(rank, world), args.batch_size)
+        dev_batches = WindowStore.batches(dev_store.shard(rank, world), args.batch_size)
+        if args.max_batches:
+            train_batches, dev_batches = train_batches[:args.max_batches], dev_batches[:args.max_batches]
+
         native = model_type in ('feedforward', 'groundlink', 'diffusion')
         if native:
-            trainer = Trainer(model, opt_type=args.opt_type, lr=args.learning_rate, args=args, seed=1234, ema_decay=args.ema_decay)
+            # every rank holds an equal-sized shard, so every rank runs the same number of steps
+            total_steps = args.epochs * len(train_batches) if args.lr_schedule == 'cosine' else None
+            if total_steps is not None and total_steps <= args.lr_warmup_steps:
+                raise ValueError(f"--lr-schedule cosine needs more steps than --lr-warmup-steps ({args.lr_warmup_steps}); "
+                                 f"the run has {total_steps} ({args.epochs} epochs x {len(train_batches)} batches)")
+            trainer = Trainer(model, opt_type=args.opt_type, lr=args.learning_rate, args=args, seed=1234, ema_decay=args.ema_decay,
+                              clip_grad_norm=args.clip_grad_norm, lr_warmup_steps=args.lr_warmup_steps,
+                              lr_schedule=args.lr_schedule, lr_min=args.lr_min, total_steps=total_steps)
             optimizer = None
         else:
             if world > 1:
@@ -220,11 +243,8 @@ class TrainCommand(AbstractCommand):
                 ck = torch.load(self.latest_checkpoint_path(checkpoint_dir), map_location="cpu")
                 trainer.load_ema_state_dict(ck.get('ema_state_dict'))
         use_ema = native and trainer.ema is not None
+        clipping = native and args.clip_grad_norm > 0
 
-        train_batches = WindowStore.batches(train_store.shard(rank, world), args.batch_size)
-        dev_batches = WindowStore.batches(dev_store.shard(rank, world), args.batch_size)
-        if args.max_batches:
-            train_batches, dev_batches = train_batches[:args.max_batches], dev_batches[:args.max_batches]
         train_log, dev_log = _ResultLog('train'), _ResultLog(DEV)
         train_ev, dev_ev = RegressionLossEvaluator(None, 'train', device=device), RegressionLossEvaluator(None, DEV, device=device)
         # the denoiser is evaluated by reverse sampling, as in analyze: a few DDIM steps per dev batch, or no dev pass
@@ -268,6 +288,10 @@ class TrainCommand(AbstractCommand):
                 if (i + 1) % 1000 == 0 or i == len(train_batches) - 1:
                     logging.info(f'[{rank=}] Batch {i} Training Set Evaluation: ')
                     (train_log if native else train_ev).print_report(args, reset=False)
+                    if clipping:
+                        st = trainer.grad_norm_stats()
+                        print(f'[{rank=}] Gradient norm before clipping: mean {st["mean_norm"]:.6g} over {st["steps"]} steps, '
+                              f'{st["clipped"]} clipped (max norm {args.clip_grad_norm:g})')
                     if rank == 0:                              # avoid redundant saving across processes
                         model_path = f"{checkpoint_dir}/epoch_{epoch}_batch_{i}.pt"
                         os.makedirs(os.path.dirname(model_path), exist_ok=True)

@@ -333,14 +333,57 @@ def pack_labels(raw, nb, win_row0, contact_idx, mass, F, stride, last_only, out_
 
 
 # ---- optimizer ----------------------------------------------------------------------------------------
+LR_SCHEDULES = {"constant": 0, "cosine": 1}
+
+
+class GradClipWorkspace:
+    """Device buffers of ``grad_clip_coef``: ``out`` = {pre-clip total norm, clip coefficient} (fp32[2]), the per-block
+    partials and the last-block counter, and ``record`` = {sum of totals, steps, clipped steps} (fp64[3]) for reports."""
+
+    def __init__(self, device):
+        self.out = torch.zeros(2, dtype=torch.float32, device=device)
+        self.partials = torch.zeros(1024, dtype=torch.float64, device=device)
+        self.counter = torch.zeros(1, dtype=torch.int32, device=device)
+        self.record = torch.zeros(3, dtype=torch.float64, device=device)
+
+
+def grad_clip_coef(grad, max_norm, grad_scale=1.0, ws: Optional[GradClipWorkspace] = None, record=True) -> torch.Tensor:
+    """torch.nn.utils.clip_grad_norm_'s total norm and clip coefficient of ``grad_scale * grad`` (a flat fp32 arena) into
+    ``ws.out`` = {total, min(1, max_norm / (total + 1e-6))}, on the device, without a host synchronisation; with ``record``
+    also accumulates ``ws.record``.  Returns ``ws.out``."""
+    _require_cuda(grad)
+    if grad.dtype != torch.float32 or not grad.is_contiguous():
+        raise ValueError(f"gradient arena must be contiguous fp32, got {grad.dtype}")
+    ws = ws or GradClipWorkspace(grad.device)
+    call("ibm_grad_clip_coef", _p(grad), grad.numel(), grad_scale, max_norm, _p(ws.out), _p(ws.partials), _p(ws.counter),
+         _p(ws.record) if record else None, stream_ptr())
+    return ws.out
+
+
 def optimizer_step(kind: str, param, grad, state0, state1, param_bf16, lr, grad_scale, step, step_dev=None, ema=None,
-                   ema_decay=0.0):
+                   ema_decay=0.0, clip=None, schedule=None, warmup_steps=0, total_steps=0, lr_min=0.0):
     """``step_dev`` (device int64[1]) replaces the by-value 1-based step count (graph-replayed steps).  ``ema`` (fp32, the
     parameters' layout): also updates this exponential moving average of the parameters in the same pass, decay
-    min(``ema_decay``, (1 + n) / (10 + n)) at step n."""
+    min(``ema_decay``, (1 + n) / (10 + n)) at step n.
+
+    ``clip`` (device fp32[2] from ``grad_clip_coef``) multiplies the averaged gradient by its clip coefficient; ``schedule``
+    ('constant' or 'cosine') scales ``lr`` at step n by the warm-up / cosine factor of ibm_b200.h, from ``warmup_steps``,
+    ``total_steps`` and ``lr_min``.  Either one selects the scheduled kernel; with neither the call is the plain step."""
     if ema is not None:
         if ema.numel() != param.numel() or ema.dtype != torch.float32:
             raise ValueError(f"EMA arena must be fp32 with {param.numel()} elements, got {ema.dtype} x {ema.numel()}")
+    if clip is not None or schedule is not None:
+        if schedule is None:
+            schedule = "constant"
+        if schedule not in LR_SCHEDULES:
+            raise ValueError(f"unknown learning-rate schedule {schedule!r}; expected one of {sorted(LR_SCHEDULES)}")
+        if clip is not None and (clip.dtype != torch.float32 or clip.numel() < 2):
+            raise ValueError("clip must be the fp32[2] {total, coefficient} of grad_clip_coef")
+        call("ibm_optimizer_step_sched", _lib.OPT_KIND[kind], _p(param), _p(grad), _p(state0), _p(state1), _p(param_bf16),
+             _p(ema), param.numel(), lr, grad_scale, ema_decay if ema is not None else 0.0, step, _p(step_dev), _p(clip),
+             LR_SCHEDULES[schedule], int(warmup_steps), int(total_steps), lr_min, stream_ptr())
+        return
+    if ema is not None:
         call("ibm_optimizer_step_ema", _lib.OPT_KIND[kind], _p(param), _p(grad), _p(state0), _p(state1), _p(param_bf16), _p(ema),
              param.numel(), lr, grad_scale, ema_decay, step, _p(step_dev), stream_ptr())
         return

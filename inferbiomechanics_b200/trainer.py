@@ -19,6 +19,7 @@ from __future__ import annotations
 import argparse
 import contextlib
 import gc
+import math
 import os
 from typing import Dict, Iterator, List, Optional
 
@@ -56,11 +57,51 @@ def _time_kernel(fn, iters: int = 20) -> float:
     return e0.elapsed_time(e1) / iters
 
 
+LR_SCHEDULES = tuple(ops.LR_SCHEDULES)                # the kernel's schedule codes, in the order of their values
+
+
+def lr_lambda(n: int, warmup_steps: int, schedule: str, total_steps: int, lr_ratio: float) -> float:
+    """Learning-rate factor of the 1-based step n, the host twin of the optimizer kernel's (include/ibm_b200.h,
+    ibm_optimizer_step_sched): n / W during a warm-up of W steps, then 1 (constant) or a cosine from 1 down to
+    ``lr_ratio`` = lr_min / lr at step ``total_steps``.  ``LambdaLR(opt, lambda s: lr_lambda(s + 1, ...))`` hands the
+    optimizer's n-th step() lr * lr_lambda(n)."""
+    if warmup_steps > 0 and n <= warmup_steps:
+        return n / warmup_steps
+    if schedule == "constant":
+        return 1.0
+    p = min(max((n - warmup_steps) / (total_steps - warmup_steps), 0.0), 1.0)
+    return lr_ratio + (1.0 - lr_ratio) * (0.5 * (1.0 + math.cos(math.pi * p)))
+
+
+def check_clip_sched(lr: float, clip_grad_norm: float, lr_warmup_steps: int, lr_schedule: str, lr_min: float,
+                     total_steps: Optional[int], flag: str = "") -> None:
+    """ValueError for settings the scheduled optimizer cannot run; ``flag`` = '--' names the CLI flags instead."""
+    def name(k):
+        return f"--{k.replace('_', '-')}" if flag else k
+    if not clip_grad_norm >= 0.0:
+        raise ValueError(f"{name('clip_grad_norm')} must be >= 0 (0 = no clipping), got {clip_grad_norm}")
+    if lr_warmup_steps < 0:
+        raise ValueError(f"{name('lr_warmup_steps')} must be >= 0, got {lr_warmup_steps}")
+    if lr_schedule not in LR_SCHEDULES:
+        raise ValueError(f"{name('lr_schedule')} must be one of {LR_SCHEDULES}, got {lr_schedule!r}")
+    if not lr_min >= 0.0:
+        raise ValueError(f"{name('lr_min')} must be >= 0, got {lr_min}")
+    if lr_min > lr:
+        raise ValueError(f"{name('lr_min')} ({lr_min}) must not exceed the learning rate ({lr})")
+    if total_steps is not None and total_steps < 0:
+        raise ValueError(f"total_steps must be >= 0, got {total_steps}")
+    if lr_schedule == "cosine" and (total_steps is None or total_steps <= lr_warmup_steps):
+        raise ValueError(f"the cosine schedule needs total_steps > {name('lr_warmup_steps')} ({lr_warmup_steps}), got {total_steps}")
+
+
 class Trainer:
     def __init__(self, model, opt_type: str = "rmsprop", lr: float = 1e-4, args: Optional[argparse.Namespace] = None,
-                 diffusion: Optional[GaussianDiffusion] = None, bucket_mb: float = 8.0, seed: int = 0, ema_decay: float = 0.0):
+                 diffusion: Optional[GaussianDiffusion] = None, bucket_mb: float = 8.0, seed: int = 0, ema_decay: float = 0.0,
+                 clip_grad_norm: float = 0.0, lr_warmup_steps: int = 0, lr_schedule: str = "constant", lr_min: float = 0.0,
+                 total_steps: Optional[int] = None):
         if not 0.0 <= ema_decay < 1.0:
             raise ValueError(f"ema_decay must be in [0, 1) (0 = no EMA), got {ema_decay}")
+        check_clip_sched(lr, clip_grad_norm, lr_warmup_steps, lr_schedule, lr_min, total_steps)
         self.model = model
         self.eng = model.engine()
         self.arena = model.arena
@@ -95,6 +136,13 @@ class Trainer:
         self.ema_decay = float(ema_decay)
         self.ema: Optional[torch.Tensor] = self.arena.master.clone() if ema_decay > 0 else None
         self._in_ema = False
+        # global-norm gradient clipping and the learning-rate schedule, both evaluated on the device by the optimizer kernel
+        # from the device step counter, so captured steps replay with the values of their own step
+        self.clip_grad_norm = float(clip_grad_norm)
+        self.lr_warmup_steps, self.lr_schedule, self.lr_min = int(lr_warmup_steps), lr_schedule, float(lr_min)
+        self.total_steps = int(total_steps) if total_steps is not None else 0
+        self.scheduled = self.lr_warmup_steps > 0 or lr_schedule != "constant"
+        self._clip_ws = ops.GradClipWorkspace(dev) if self.clip_grad_norm > 0 else None
         # device-resident 1-based step counter: incremented by a one-thread kernel at the start of every step, read by the
         # dropout kernels (Philox offset) and the optimizer kernel (Adam / Adamax bias correction), so that a captured step
         # can be replayed although those values change from step to step
@@ -174,7 +222,8 @@ class Trainer:
         return graphs
 
     def _train_step_graphed(self, store: WindowStore, idx: torch.Tensor) -> torch.Tensor:
-        key = (id(store), idx.numel(), self.lr, self.model.training)     # launch arguments baked into the captured step
+        # launch arguments baked into the captured step: the schedule's parameters, never a per-step learning rate
+        key = (id(store), idx.numel(), self.lr, self.model.training, self._clip_sched_key())
         g = self._graphs.get(key)
         if g is None:
             if len(self._graphs) >= 8:
@@ -247,11 +296,45 @@ class Trainer:
         return result
 
     def optimizer_step(self) -> None:
+        """After ``bucketer.finish()``, on the compute stream: the gradient arena holds the allreduced sum.  With clipping on,
+        the norm kernel reads it first and the scheduled optimizer applies the coefficient it wrote."""
         self.step_count += 1
-        ops.optimizer_step(self.opt_type, self.arena.master, self.arena.grad, self.state0, self.state1, self.arena.shadow,
-                           self.lr, 1.0 / self.world, self.step_count, step_dev=self.step_dev, ema=self.ema,
-                           ema_decay=self.ema_decay)
+        if self._clip_ws is None and not self.scheduled:
+            ops.optimizer_step(self.opt_type, self.arena.master, self.arena.grad, self.state0, self.state1, self.arena.shadow,
+                               self.lr, 1.0 / self.world, self.step_count, step_dev=self.step_dev, ema=self.ema,
+                               ema_decay=self.ema_decay)
+        else:
+            clip = None
+            if self._clip_ws is not None:
+                clip = ops.grad_clip_coef(self.arena.grad, self.clip_grad_norm, 1.0 / self.world, self._clip_ws)
+            ops.optimizer_step(self.opt_type, self.arena.master, self.arena.grad, self.state0, self.state1, self.arena.shadow,
+                               self.lr, 1.0 / self.world, self.step_count, step_dev=self.step_dev, ema=self.ema,
+                               ema_decay=self.ema_decay, clip=clip, schedule=self.lr_schedule,
+                               warmup_steps=self.lr_warmup_steps, total_steps=self.total_steps, lr_min=self.lr_min)
         self.arena.mark_shadow_fresh()
+
+    # ---- gradient clipping and learning-rate schedule ----------------------------------------------------------------
+    def _clip_sched_key(self) -> Optional[tuple]:
+        if self._clip_ws is None and not self.scheduled:
+            return None
+        return (self.clip_grad_norm, self.lr_warmup_steps, self.lr_schedule, self.total_steps, self.lr_min)
+
+    def current_lr(self) -> float:
+        """The learning rate the next step applies (the optimizer kernel derives the same value on the device)."""
+        if not self.scheduled:
+            return self.lr
+        return self.lr * lr_lambda(self.step_count + 1, self.lr_warmup_steps, self.lr_schedule, self.total_steps,
+                                   self.lr_min / self.lr if self.lr > 0 else 0.0)
+
+    def grad_norm_stats(self, reset: bool = True) -> dict:
+        """Mean pre-clip global gradient norm, the number of clipped steps and the number of steps since the last reset:
+        one read of the device record (a synchronisation), meant for report time."""
+        if self._clip_ws is None:
+            raise RuntimeError("this Trainer does not clip gradients (construct it with clip_grad_norm > 0)")
+        total, steps, clipped = self._clip_ws.record.tolist()
+        if reset:
+            self._clip_ws.record.zero_()
+        return {"mean_norm": total / steps if steps else float("nan"), "clipped": int(clipped), "steps": int(steps)}
 
     # ---- exponential moving average of the weights -------------------------------------------------------------------
     def _require_ema(self) -> None:
@@ -341,6 +424,13 @@ class Trainer:
         elif self.step_count > 0:                                    # SGD without momentum keeps no tensors
             sd["state"] = {i: {"momentum_buffer": None} for i in range(len(self.arena.names))}
         sd["ibm_b200"] = {"opt_type": self.opt_type, "step": self.step_count}
+        if self.scheduled:
+            # what a torch optimizer's group holds after optimizer.step(); scheduler.step() under LambdaLR
+            sd["param_groups"][0]["lr"] = self.current_lr()
+            sd["param_groups"][0]["initial_lr"] = self.lr
+        if self._clip_sched_key() is not None:
+            sd["ibm_b200"].update(clip_grad_norm=self.clip_grad_norm, lr_warmup_steps=self.lr_warmup_steps,
+                                  lr_schedule=self.lr_schedule, lr_min=self.lr_min, total_steps=self.total_steps)
         return sd
 
     def load_optimizer_state_dict(self, sd: dict) -> None:
