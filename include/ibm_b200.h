@@ -197,6 +197,26 @@ int ibm_ddpm_respaced_step(const float* x0_hat, int64_t x0_ld, const float* x_t,
                            int64_t bf16_ld, uint64_t seed, uint64_t offset, int32_t* t_next_dev,
                            const int32_t* t_succ, void* stream);
 
+/* Classifier-free guidance (DESIGN.md D-1).  One step of ibm_ddpm_posterior_step (t_succ == NULL) or
+ * ibm_ddpm_respaced_step (t_succ != NULL) on a guided prediction: x0_hat holds 2M rows (leading dim
+ * x0_ld), rows 0..M-1 conditional (c) and rows M..2M-1 unconditional (u), combined per element in fp32 as
+ * fmaf(guidance_scale, c - u, u) before the unchanged update, [t>0] noise gate and Philox counter
+ * offset + t.  x_t / z / x_prev: fp32 [M,30]; xprev_bf16 (optional) receives the bf16 rows twice, at
+ * rows m and M + m, so both halves of the next forward see the same x_t.  guidance_scale: finite, >= 0. */
+int ibm_ddpm_guided_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const float* z,
+                         const int32_t* t_dev, const float* coef_x0, const float* coef_xt,
+                         const float* sigma, int64_t M, float* x_prev, void* xprev_bf16,
+                         int64_t bf16_ld, uint64_t seed, uint64_t offset, int32_t* t_next_dev,
+                         const int32_t* t_succ, float guidance_scale, void* stream);
+
+/* Per-window condition dropout for classifier-free guidance training.  xc: bf16 [B*F, ld] (window b
+ * owns rows b*F .. b*F+F-1).  Window b is dropped iff word 0 of Philox4x32-10 draw b at (seed, offset)
+ * is below uint32(p * 2^32) (the keep rule of the dropout kernels); p >= 1 drops every window without
+ * drawing.  A dropped window gets +0 in columns col0 .. col0+ncols-1 of its F rows; no other byte is
+ * written.  keep_out (optional): uint8 [B], 1 = kept, 0 = dropped.  Requires 0 < p. */
+int ibm_cond_dropout(void* xc_bf16, int64_t ld, int64_t B, int32_t F, int32_t col0, int32_t ncols, float p,
+                     uint64_t seed, uint64_t offset, uint8_t* keep_out, void* stream);
+
 /* sinusoidal timestep embedding, bf16 [B, dim] (ld = dim): [sin(t w_k) | cos(t w_k)],
  * w_k = 10000^(-k/(dim/2)).  t: int32[B], or if t_is_scalar a single device int32 broadcast. */
 int ibm_timestep_embed(const int32_t* t, int32_t t_is_scalar, int64_t B, int32_t dim, void* out_bf16,

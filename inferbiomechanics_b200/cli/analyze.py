@@ -7,7 +7,8 @@ collective during the pass), keeps the per-batch fp32[40] results on the device 
 equal batch sizes keep the reference's mean-of-batch-means aggregate (RegressionLossEvaluator.py:383-387) exact.
 Per-window plots (matplotlib) and the names CSV are outside the hot path.  ``--model-type diffusion`` runs the
 reverse sampler per batch (``--sampler ddpm``: the 1000-step chain; ``ddim``: ``--sampling-steps`` respaced steps) and
-scores the sampled trajectories with the same evaluator.
+scores the sampled trajectories with the same evaluator; ``--guidance-scale`` samples it with classifier-free guidance, which
+needs a checkpoint trained with ``train --cond-drop-prob``.
 """
 from __future__ import annotations
 
@@ -19,7 +20,7 @@ import torch
 import torch.distributed as dist
 
 from .. import parallel
-from ..diffusion import GaussianDiffusion
+from ..diffusion import GaussianDiffusion, check_guidance_scale
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
 from ..trainer import Trainer
 from . import _data
@@ -69,6 +70,10 @@ class AnalyzeCommand(AbstractCommand):
         sp.add_argument('--ema', action='store_true', default=False,
                         help="Evaluate the checkpoint's EMA weights (ema_state_dict, written by train --ema-decay) instead of "
                              "the trained ones.")
+        sp.add_argument('--guidance-scale', type=float, default=1.0,
+                        help='--model-type diffusion: classifier-free guidance scale s (x0 = u + s (c - u)) with either '
+                             'sampler; 1 = no guidance, 0 = unconditional. s != 1 needs a checkpoint trained with '
+                             'train --cond-drop-prob > 0.')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'analyze':
@@ -77,6 +82,9 @@ class AnalyzeCommand(AbstractCommand):
             raise ValueError("--eta applies to --sampler ddim only")
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
+        guidance = args.guidance_scale
+        if guidance != 1.0:
+            self.check_guidance_checkpoint(model_type, guidance, checkpoint_dir)
         root_history_len = 10
         rank, world, local = parallel.init_from_env("nccl")
         torch.cuda.set_device(local)
@@ -115,9 +123,10 @@ class AnalyzeCommand(AbstractCommand):
                     if model_type == 'diffusion':
                         if args.sampler == 'ddim':
                             sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, ddim_steps=args.sampling_steps,
-                                             eta=args.eta)
+                                             eta=args.eta, guidance_scale=guidance)
                         else:
-                            sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, steps=args.sampling_steps)
+                            sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, steps=args.sampling_steps,
+                                             guidance_scale=guidance)
                         continue
                     inputs = input_dict(store, idx, model_type, args.stride, root_history_len)
                     ev(inputs, model(inputs), label_dict(store, idx), [], [], args)
@@ -136,10 +145,26 @@ class AnalyzeCommand(AbstractCommand):
                 src._results = [r for g in merged for r in g]
                 src._wm_results = list(src._results)
             if rank == 0:
-                print(f'{split} set evaluation ({n} windows):')
+                print(f'{split} set evaluation ({n} windows' + (f', guidance scale {guidance:g}' if guidance != 1.0 else '') + '):')
                 reports[split] = src.aggregate()
                 src.print_report(args, log_to_wandb=not args.no_wandb)
         if dist.is_initialized():
             dist.destroy_process_group()
         self.last_reports = reports
         return True
+
+    def check_guidance_checkpoint(self, model_type: str, guidance_scale: float, checkpoint_dir: str) -> None:
+        """ValueError unless guidance can run: a diffusion model, a finite scale >= 0 and a latest checkpoint whose optimizer
+        tag records cond_drop_prob > 0 (a denoiser never trained without its condition has no meaningful unconditional
+        prediction)."""
+        if model_type != 'diffusion':
+            raise ValueError("--guidance-scale applies to --model-type diffusion only")
+        check_guidance_scale(guidance_scale)
+        path = self.latest_checkpoint_path(checkpoint_dir)
+        if path is None:
+            raise ValueError(f"--guidance-scale {guidance_scale:g} needs a checkpoint trained with --cond-drop-prob > 0; "
+                             f"{checkpoint_dir} holds none")
+        tag = (torch.load(path, map_location="cpu").get('optimizer_state_dict') or {}).get('ibm_b200') or {}
+        if not tag.get('cond_drop_prob', 0.0) > 0.0:
+            raise ValueError(f"--guidance-scale {guidance_scale:g} needs a checkpoint trained with --cond-drop-prob > 0; "
+                             f"{path} records none")

@@ -25,7 +25,7 @@ from ..data.window_store import WindowStore
 from ..diffusion import GaussianDiffusion
 from ..keys import LOSS_QUANTITIES, MODEL_INPUT_ORDER
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
-from ..trainer import LR_SCHEDULES, Trainer, check_clip_sched
+from ..trainer import LR_SCHEDULES, Trainer, check_clip_sched, check_cond_drop
 from . import _data
 from .abstract_command import AbstractCommand
 
@@ -53,12 +53,14 @@ def label_dict(store: WindowStore, idx: torch.Tensor):
 
 
 def sample_and_score(diffusion, model, store: WindowStore, idx: torch.Tensor, ev: RegressionLossEvaluator, args, seed: int,
-                     *, steps=None, ddim_steps=None, eta: float = 0.0) -> None:
+                     *, steps=None, ddim_steps=None, eta: float = 0.0, guidance_scale: float = 1.0) -> None:
     """Reverse-sample the denoiser's trajectories for windows ``idx`` of ``store`` and score them with ``ev`` against the
     store's labels: the condition is the packed kinematics in the engine's concat buffer, x_T ~ Philox(``seed``), and
-    ``steps`` / ``ddim_steps`` / ``eta`` select the sampler as in ``GaussianDiffusion.sample``."""
+    ``steps`` / ``ddim_steps`` / ``eta`` select the sampler and ``guidance_scale`` the classifier-free guidance as in
+    ``GaussianDiffusion.sample``."""
     store.pack(idx, model.engine().input_layout(idx.numel(), store.F, False))
-    x0 = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta)
+    x0 = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
+                          guidance_scale=guidance_scale)
     if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
         x0 = x0[:, -1:]
     outputs = {k: x0[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, QUANTITY_CUTS)}
@@ -170,6 +172,10 @@ class TrainCommand(AbstractCommand):
                         help='Learning rate after the warm-up: constant, or a cosine decay to --lr-min at the last step of '
                              'the run (epochs x batches per epoch).')
         sp.add_argument('--lr-min', type=float, default=0.0, help='Final learning rate of the cosine schedule.')
+        sp.add_argument('--cond-drop-prob', type=float, default=0.0,
+                        help='--model-type diffusion: replace the kinematics of this fraction of the windows of every step by '
+                             'zeros (e.g. 0.1, as MDM), so the denoiser also learns the unconditional prediction that '
+                             'analyze --guidance-scale needs; recorded in the checkpoints. 0 = off.')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'train':
@@ -182,6 +188,7 @@ class TrainCommand(AbstractCommand):
             raise ValueError(f"--ema-decay must be in [0, 1), got {args.ema_decay}")
         # the cosine's length (epochs x batches per epoch) is checked once the training store is open
         check_clip_sched(args.learning_rate, args.clip_grad_norm, args.lr_warmup_steps, 'constant', args.lr_min, None, flag='--')
+        check_cond_drop(args.cond_drop_prob, args.model_type == 'diffusion', flag='--')
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
         root_history_len = 10
@@ -225,7 +232,8 @@ class TrainCommand(AbstractCommand):
                                  f"the run has {total_steps} ({args.epochs} epochs x {len(train_batches)} batches)")
             trainer = Trainer(model, opt_type=args.opt_type, lr=args.learning_rate, args=args, seed=1234, ema_decay=args.ema_decay,
                               clip_grad_norm=args.clip_grad_norm, lr_warmup_steps=args.lr_warmup_steps,
-                              lr_schedule=args.lr_schedule, lr_min=args.lr_min, total_steps=total_steps)
+                              lr_schedule=args.lr_schedule, lr_min=args.lr_min, total_steps=total_steps,
+                              cond_drop_prob=args.cond_drop_prob)
             optimizer = None
         else:
             if world > 1:

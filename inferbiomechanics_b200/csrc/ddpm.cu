@@ -64,15 +64,17 @@ q_sample_kernel(const float* __restrict__ x0, const float* __restrict__ eps, con
 // ---- posterior step --------------------------------------------------------------------------
 // One float2 per thread-iteration: 30 is even so a pair never straddles a row; x0_hat has its own
 // leading dimension (the head GEMM writes 32-float rows).  kSucc: the next timestep is t_succ[t]
-// (a respaced DDIM sequence) instead of t-1; the instantiation without it is the DDPM chain.
-template <bool kSucc>
+// (a respaced DDIM sequence) instead of t-1; the instantiation without it is the DDPM chain.  kGuided: x0h holds 2M
+// rows, conditional then unconditional, combined as u + s (c - u) (classifier-free guidance); the bf16 rows go to both
+// halves of the concat buffer.  gscale is the last parameter so the unguided instantiations keep their parameter offsets.
+template <bool kSucc, bool kGuided>
 __global__ void __launch_bounds__(kThreads)
 posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __restrict__ xt,
                  const float* __restrict__ z, const int32_t* __restrict__ t_dev, const float* __restrict__ c1t,
                  const float* __restrict__ c2t, const float* __restrict__ sig, long long M,
                  float* __restrict__ xprev, __nv_bfloat16* __restrict__ xp_bf16, long long bf16_ld,
                  uint64_t seed, uint64_t offset, int32_t* __restrict__ t_next,
-                 const int32_t* __restrict__ t_succ) {
+                 const int32_t* __restrict__ t_succ, float gscale) {
   const int tt = __ldg(t_dev);
   const float c1 = __ldg(c1t + tt), c2 = __ldg(c2t + tt);
   const float s = tt > 0 ? __ldg(sig + tt) : 0.f;
@@ -81,7 +83,12 @@ posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __
 #pragma unroll 2
   for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < npair; p += stride) {
     const long long m = p / 15, c = (p - m * 15) * 2;
-    const float2 a = *reinterpret_cast<const float2*>(x0h + m * x0_ld + c);
+    float2 a = *reinterpret_cast<const float2*>(x0h + m * x0_ld + c);
+    if (kGuided) {
+      const float2 u = *reinterpret_cast<const float2*>(x0h + (M + m) * x0_ld + c);
+      a.x = fmaf(gscale, a.x - u.x, u.x);
+      a.y = fmaf(gscale, a.y - u.y, u.y);
+    }
     const float2 x = *reinterpret_cast<const float2*>(xt + 2 * p);
     float2 n;
     if (z) n = *reinterpret_cast<const float2*>(z + 2 * p);
@@ -95,9 +102,49 @@ posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __
     r.y = fmaf(c1, a.y, c2 * x.y);
     if (tt > 0) { r.x = fmaf(s, n.x, r.x); r.y = fmaf(s, n.y, r.y); }
     if (xprev) *reinterpret_cast<float2*>(xprev + 2 * p) = r;
-    if (xp_bf16) *reinterpret_cast<uint32_t*>(xp_bf16 + m * bf16_ld + c) = pack_bf16x2(r.x, r.y);
+    if (xp_bf16) {
+      const uint32_t v = pack_bf16x2(r.x, r.y);
+      *reinterpret_cast<uint32_t*>(xp_bf16 + m * bf16_ld + c) = v;
+      if (kGuided) *reinterpret_cast<uint32_t*>(xp_bf16 + (M + m) * bf16_ld + c) = v;
+    }
   }
   if (t_next && blockIdx.x == 0 && threadIdx.x == 0) *t_next = kSucc ? __ldg(t_succ + tt) : tt - 1;
+}
+
+// ---- per-window condition dropout (classifier-free guidance training) -------------------------------------------------
+// One block per window (grid-stride): every thread derives the window's keep bit from word 0 of Philox draw b, so a kept
+// window costs one draw and no memory traffic.  A dropped window's F rows are cleared in 8-column groups: a group that lies
+// inside [col0, col0 + ncols) is one 16-byte store when the rows are 16-byte aligned (kVec), a group cut by the range edge
+// is stored element by element so neighbouring columns (x_t, pad) are never written.
+template <bool kVec>
+__global__ void __launch_bounds__(kThreads)
+cond_dropout_kernel(__nv_bfloat16* __restrict__ xc, long long ld, long long B, int F, int col0, int ncols,
+                    uint32_t thresh, int drop_all, uint64_t seed, uint64_t offset, uint8_t* __restrict__ keep_out) {
+  const int g0 = col0 >> 3, g1 = (col0 + ncols - 1) >> 3, col1 = col0 + ncols;
+  const int ng = g1 - g0 + 1;
+  const long long items = (long long)F * ng;
+  for (long long b = blockIdx.x; b < B; b += gridDim.x) {
+    bool drop = true;
+    if (!drop_all) {
+      const uint4 r = philox4x32_10(make_uint4((uint32_t)b, (uint32_t)(b >> 32), (uint32_t)offset, (uint32_t)(offset >> 32)),
+                                    make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+      drop = r.x < thresh;
+    }
+    if (keep_out && threadIdx.x == 0) keep_out[b] = drop ? 0 : 1;
+    if (!drop) continue;
+    __nv_bfloat16* base = xc + b * F * ld;
+    for (long long i = threadIdx.x; i < items; i += blockDim.x) {
+      const long long f = i / ng;
+      const int c = (g0 + (int)(i - f * ng)) << 3;
+      __nv_bfloat16* row = base + f * ld;
+      if (kVec && c >= col0 && c + 8 <= col1) {
+        *reinterpret_cast<uint4*>(row + c) = make_uint4(0u, 0u, 0u, 0u);
+      } else {
+        const int lo = c > col0 ? c : col0, hi = c + 8 < col1 ? c + 8 : col1;
+        for (int k = lo; k < hi; ++k) row[k] = __ushort_as_bfloat16((unsigned short)0);
+      }
+    }
+  }
 }
 
 // ---- sinusoidal timestep embedding -----------------------------------------------------------
@@ -308,9 +355,9 @@ extern "C" int ibm_ddpm_posterior_step(const float* x0_hat, int64_t x0_ld, const
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "posterior_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "posterior_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "posterior_step: bf16 ld must be even");
-  posterior_kernel<false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev, nullptr);
+      seed, offset, t_next_dev, nullptr, 0.f);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }
@@ -326,9 +373,56 @@ extern "C" int ibm_ddpm_respaced_step(const float* x0_hat, int64_t x0_ld, const 
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "respaced_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "respaced_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "respaced_step: bf16 ld must be even");
-  posterior_kernel<true><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<true, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev, t_succ);
+      seed, offset, t_next_dev, t_succ, 0.f);
+  IBM_LAUNCH_CHECK();
+  return IBM_OK;
+}
+
+extern "C" int ibm_ddpm_guided_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const float* z,
+                                    const int32_t* t_dev, const float* coef_x0, const float* coef_xt,
+                                    const float* sigma, int64_t M, float* x_prev, void* xprev_bf16, int64_t bf16_ld,
+                                    uint64_t seed, uint64_t offset, int32_t* t_next_dev, const int32_t* t_succ,
+                                    float guidance_scale, void* stream) {
+  using namespace ibm;
+  IBM_CHECK_ARCH();
+  IBM_CHECK_ARG(x0_hat && x_t && t_dev && coef_x0 && coef_xt && sigma, "guided_step: null argument");
+  IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "guided_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
+  IBM_CHECK_ARG(x_prev || xprev_bf16, "guided_step: no output requested");
+  IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "guided_step: bf16 ld must be even");
+  IBM_CHECK_ARG(guidance_scale >= 0.f && guidance_scale <= 3.402823466e38f, "guided_step: guidance scale must be finite and >= 0, got %g",
+                (double)guidance_scale);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  auto* xb = static_cast<__nv_bfloat16*>(xprev_bf16);
+  if (t_succ)
+    posterior_kernel<true, true><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
+                                                                        x_prev, xb, bf16_ld, seed, offset, t_next_dev, t_succ,
+                                                                        guidance_scale);
+  else
+    posterior_kernel<false, true><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
+                                                                         x_prev, xb, bf16_ld, seed, offset, t_next_dev, nullptr,
+                                                                         guidance_scale);
+  IBM_LAUNCH_CHECK();
+  return IBM_OK;
+}
+
+extern "C" int ibm_cond_dropout(void* xc_bf16, int64_t ld, int64_t B, int32_t F, int32_t col0, int32_t ncols, float p,
+                                uint64_t seed, uint64_t offset, uint8_t* keep_out, void* stream) {
+  using namespace ibm;
+  IBM_CHECK_ARCH();
+  IBM_CHECK_ARG(xc_bf16 && B > 0 && F > 0 && col0 >= 0 && ncols > 0 && (int64_t)col0 + ncols <= ld,
+                "cond_dropout: bad shape (B=%lld F=%d col0=%d ncols=%d ld=%lld)", (long long)B, F, col0, ncols, (long long)ld);
+  IBM_CHECK_ARG(p > 0.f, "cond_dropout: p must be > 0 (p = 0 drops nothing and launches nothing), got %g", (double)p);
+  const int drop_all = p >= 1.f;
+  const uint32_t thresh = drop_all ? 0u : (uint32_t)(p * 4294967296.0);   // the keep rule of dropout_kernel
+  const int grid = (int)(B < (int64_t)sm_count() * 16 ? B : (int64_t)sm_count() * 16);
+  auto* xc = static_cast<__nv_bfloat16*>(xc_bf16);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (ld % 8 == 0 && aligned16(xc_bf16))
+    cond_dropout_kernel<true><<<grid, kThreads, 0, s>>>(xc, ld, B, F, col0, ncols, thresh, drop_all, seed, offset, keep_out);
+  else
+    cond_dropout_kernel<false><<<grid, kThreads, 0, s>>>(xc, ld, B, F, col0, ncols, thresh, drop_all, seed, offset, keep_out);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }

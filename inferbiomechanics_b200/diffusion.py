@@ -13,9 +13,14 @@ The reverse loop runs the denoiser forward + one fused posterior kernel per step
 in device memory so two consecutive steps are captured once in a CUDA graph and replayed (sampling at
 512 windows/GPU is launch-bound otherwise).  Windows are independent: multi-GPU sampling shards them
 with no collective.
+
+Classifier-free guidance (Ho & Salimans 2022) with scale s != 1 runs the forward on 2B windows per step, the B conditioned
+ones and the same B with all-zero kinematics (the null condition the trainer's ``cond_drop_prob`` teaches), and one guided
+step kernel combines x0_hat = u + s (c - u) before the same update; s = 0 is unconditional sampling.
 """
 from __future__ import annotations
 
+import math
 from typing import Callable, Optional
 
 import numpy as np
@@ -54,6 +59,11 @@ def ddim_schedule(ddim_steps: int, eta: float = 0.0, num_timesteps: int = 1000, 
     out["succ"][ts] = succ
     out["ts"] = ts
     return out
+
+
+def check_guidance_scale(guidance_scale: float) -> None:
+    if not (math.isfinite(guidance_scale) and guidance_scale >= 0.0):
+        raise ValueError(f"guidance_scale must be finite and >= 0 (1 = no guidance, 0 = unconditional), got {guidance_scale}")
 
 
 def _check_schedule(T: int, steps: Optional[int], ddim_steps: Optional[int], eta: float) -> None:
@@ -115,17 +125,29 @@ class GaussianDiffusion:
     @torch.no_grad()
     def sample(self, model, B: int, *, x_T: Optional[torch.Tensor] = None, noise: Optional[Callable[[int], torch.Tensor]] = None,
                steps: Optional[int] = None, seed: int = 0, use_graph: bool = True, ddim_steps: Optional[int] = None,
-               eta: float = 0.0) -> torch.Tensor:
+               eta: float = 0.0, guidance_scale: float = 1.0) -> torch.Tensor:
         """Reverse-sample x_0 (B,F,30) for the kinematics already packed in model.engine().xc(B, False)
         (columns 30…).  ``noise(t)`` supplies z per step for parity tests; None ⇒ on-device Philox.
 
         ``ddim_steps=None``: the DDPM chain; ``steps`` < T runs only its first ``steps`` steps and returns x at timestep
         T - steps (a truncated chain, not a sample).  ``ddim_steps=S``: S-step DDIM with noise scale ``eta`` in [0, 1]
-        (``ddim_schedule``); eta = 0 draws no noise after x_T.  ``noise(t)`` is called with each timestep walked."""
+        (``ddim_schedule``); eta = 0 draws no noise after x_T.  ``noise(t)`` is called with each timestep walked.
+
+        ``guidance_scale`` s != 1: classifier-free guidance with either sampler.  The kinematics of xc(B) are copied into
+        the first half of xc(2B) and the second half gets the null condition (zeros); x_T goes into both halves, each step
+        runs the forward on 2B windows and the guided step kernel.  s = 1 runs the unguided loop, s = 0 samples
+        unconditionally.  The result depends on s only through the prediction: x_T and the noise are those of s = 1."""
         _check_schedule(self.T, steps, ddim_steps, eta)
+        check_guidance_scale(guidance_scale)
+        guided = guidance_scale != 1.0
         eng = model.engine()
         F, M = eng.F, B * eng.F
         xc = eng.xc(B, False)
+        if guided:
+            # rows 0..M-1 conditional, M..2M-1 the same windows with all-zero kinematics
+            xc2 = eng.xc(2 * B, False)
+            xc2[:M].copy_(xc)
+            ops.cond_dropout(xc2[M:], B, F, 30, eng.c_in, 1.0, 0, 0)
         if ddim_steps is None:
             sched = None
             ts = range(self.T - 1, self.T - 1 - (self.T if steps is None else steps), -1)
@@ -135,8 +157,9 @@ class GaussianDiffusion:
             tab = self.ddim_tables(ddim_steps, eta)
             ts = tab["ts"].tolist()
             coef_x0, coef_xt, sigma, succ = tab["coef_x0"], tab["coef_xt"], tab["sigma"], tab["succ"]
-        # the captured launches read the schedule's tables through baked-in pointers, so each schedule has its own graph
-        key = (id(model), B, sched)
+        # the captured launches read the schedule's tables through baked-in pointers, so each schedule has its own graph;
+        # the guidance scale is a baked launch argument
+        key = (id(model), B, sched) if not guided else (id(model), B, sched, float(guidance_scale))
         st = self._graphs.get(key)
         if st is None or st["model"] is not model:
             # the entry holds the model (its id() cannot be recycled while cached), the schedule's tables and, below, the
@@ -147,22 +170,29 @@ class GaussianDiffusion:
                       table_key=None, sched_tables=(coef_x0, coef_xt, sigma, succ))
             self._graphs[key] = st
         x, t_a, t_b = st["x"], st["t_a"], st["t_b"]
-        if x_T is None:
-            # x_T ~ N(0, I): the q_sample kernel with tables (0, 1) writes pure Philox noise (fp32 + bf16 rows)
-            zero = torch.zeros(B, F * 30, device=self.device)
-            ops.q_sample(zero, None, torch.zeros(B, dtype=torch.int32, device=self.device), torch.zeros(1, device=self.device),
-                         torch.ones(1, device=self.device), xt_f32=x.view(B, F * 30), xt_bf16=xc, bf16_ld=eng.ld_in, seed=seed,
-                         offset=1 << 40)
-        else:
-            x.copy_(x_T.reshape(M, 30))
-            ops.pack_inputs([x], M, F, out_bf16=xc, frame_stride=eng.ld_in, win_extra=0, col0=0)
+        # the halves of the guided buffer receive the same x_T (the same Philox seed and offset, or the same rows)
+        for rows in ((xc,) if not guided else (xc2[:M], xc2[M:])):
+            if x_T is None:
+                # x_T ~ N(0, I): the q_sample kernel with tables (0, 1) writes pure Philox noise (fp32 + bf16 rows)
+                zero = torch.zeros(B, F * 30, device=self.device)
+                ops.q_sample(zero, None, torch.zeros(B, dtype=torch.int32, device=self.device), torch.zeros(1, device=self.device),
+                             torch.ones(1, device=self.device), xt_f32=x.view(B, F * 30), xt_bf16=rows, bf16_ld=eng.ld_in,
+                             seed=seed, offset=1 << 40)
+            else:
+                x.copy_(x_T.reshape(M, 30))
+                ops.pack_inputs([x], M, F, out_bf16=rows, frame_stride=eng.ld_in, win_extra=0, col0=0)
         n_steps = len(ts)
         t_a.fill_(self.T - 1)
 
         def step(t_in, t_out, z):
-            x0_hat = eng.forward(B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
-            ops.posterior_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, x_prev=x, xprev_bf16=xc,
-                               bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ)
+            if not guided:
+                x0_hat = eng.forward(B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
+                ops.posterior_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, x_prev=x, xprev_bf16=xc,
+                                   bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ)
+                return
+            x0_hat = eng.forward(2 * B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
+            ops.guided_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, guidance_scale, x_prev=x, xprev_bf16=xc2,
+                            bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ)
 
         # DDPM runs an odd step count eagerly, as it always has; DDIM replays the graph for the even part of any S >= 2
         if noise is not None or not use_graph or (n_steps % 2 if sched is None else n_steps < 2):
@@ -202,7 +232,7 @@ class GaussianDiffusion:
     @torch.no_grad()
     def sample_windows(self, model, cond: torch.Tensor, *, batch: int = 512, steps: Optional[int] = None, seed: int = 0,
                        rank: Optional[int] = None, world: Optional[int] = None, ddim_steps: Optional[int] = None,
-                       eta: float = 0.0):
+                       eta: float = 0.0, guidance_scale: float = 1.0):
         """Reverse-sample GRF / CoP / torque / wrench trajectories for ``cond``: (N, F, C_in) fp32 packed kinematics of N
         windows (model concat order, FeedForward...py:97-108) in HOST memory (pinned for asynchronous copies).
 
@@ -211,9 +241,10 @@ class GaussianDiffusion:
         ``steps`` (default: the full schedule) CUDA-graph-replayed denoise steps, D2H copy of the trajectories — and returns
         ``(range, x0)`` with x0 a pinned host tensor (len(range), F, 30).  No collective; per-rank noise stream = seed + rank.
         The copies of batch i+1 / i-1 overlap the sampling of batch i (separate streams).  ``ddim_steps`` / ``eta`` select
-        DDIM sampling as in ``sample``."""
+        DDIM sampling and ``guidance_scale`` classifier-free guidance as in ``sample``."""
         from . import parallel
         _check_schedule(self.T, steps, ddim_steps, eta)
+        check_guidance_scale(guidance_scale)
         r, w = parallel.world()
         rank = r if rank is None else rank
         world = w if world is None else world
@@ -252,7 +283,8 @@ class GaussianDiffusion:
             packed[i & 1].record(main)
             if i + 1 < len(starts):
                 upload(i + 1)
-            x0 = self.sample(model, nb, steps=steps, seed=seed + rank + 7919 * i, ddim_steps=ddim_steps, eta=eta)
+            x0 = self.sample(model, nb, steps=steps, seed=seed + rank + 7919 * i, ddim_steps=ddim_steps, eta=eta,
+                             guidance_scale=guidance_scale)
             ready = torch.cuda.Event()
             ready.record(main)
             with torch.cuda.stream(down):

@@ -7,6 +7,11 @@ x0-prediction (MDM style): given packed kinematics c (B,F,C_in), a noisy 30-chan
 The encoder layers are the reference's ``TransformerLayer`` (post-LN, nn.MultiheadAttention, ReLU FFN;
 /root/reference/src/models/TransformerBaseline.py:8-38) at d=512, 8 heads, FFN 2048, 8 layers; the
 parameter containers below reproduce its ``state_dict`` keys so a reference layer's weights load.
+
+Classifier-free guidance (DESIGN.md D-1): the null condition is all-zero kinematics, so a model trained with
+``Trainer(cond_drop_prob=p)`` (``train --cond-drop-prob``) gives its unconditional prediction when ``forward`` is passed zero
+kinematics, and guided x0_hat = u + s (c - u) is two calls of this module.  No parameter is added: checkpoints trained either
+way have the same keys.
 """
 from __future__ import annotations
 

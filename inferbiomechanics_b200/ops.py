@@ -293,6 +293,25 @@ def posterior_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_p
              _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), stream_ptr())
 
 
+def guided_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, guidance_scale, x_prev=None, xprev_bf16=None,
+                bf16_ld=0, seed=0, offset=0, t_next=None, t_succ=None):
+    """``posterior_step`` on a classifier-free guided prediction: x0_hat holds 2M rows, conditional then unconditional,
+    combined in fp32 as u + guidance_scale (c - u); xprev_bf16 receives the bf16 rows at m and at M + m."""
+    call("ibm_ddpm_guided_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
+         _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), float(guidance_scale), stream_ptr())
+
+
+def cond_dropout(xc, B, F, col0, ncols, p, seed, offset, keep_out=None):
+    """Zeroes columns col0 .. col0+ncols-1 of the F rows of each dropped window of xc (bf16 [B*F, ld]); window b is dropped
+    iff word 0 of Philox draw b at (seed, offset) is below uint32(p * 2^32), every window at p = 1.  keep_out (uint8 [B]):
+    1 = kept.  p must lie in (0, 1]: p = 0 drops nothing, and callers launch nothing."""
+    if not 0.0 < p <= 1.0:
+        raise ValueError(f"condition dropout probability must lie in (0, 1], got {p}")
+    if keep_out is not None and (keep_out.dtype != torch.uint8 or keep_out.numel() < B):
+        raise ValueError(f"keep_out must be uint8 with at least {B} elements")
+    call("ibm_cond_dropout", _p(xc), xc.stride(0), B, F, col0, ncols, p, seed, offset, _p(keep_out), stream_ptr())
+
+
 def timestep_embed(t, out_bf16, dim, scalar=False):
     B = out_bf16.shape[0]
     call("ibm_timestep_embed", _p(t), int(scalar), B, dim, _p(out_bf16), stream_ptr())

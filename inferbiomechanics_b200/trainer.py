@@ -94,14 +94,28 @@ def check_clip_sched(lr: float, clip_grad_norm: float, lr_warmup_steps: int, lr_
         raise ValueError(f"the cosine schedule needs total_steps > {name('lr_warmup_steps')} ({lr_warmup_steps}), got {total_steps}")
 
 
+def check_cond_drop(cond_drop_prob: float, trains_by_diffusion: bool, flag: str = "") -> None:
+    """ValueError for a condition-dropout probability outside [0, 1], or a nonzero one for a model that does not train by
+    diffusion (only the denoiser has a condition to drop); ``flag`` = '--' names the CLI flag instead."""
+    name = "--cond-drop-prob" if flag else "cond_drop_prob"
+    if not 0.0 <= cond_drop_prob <= 1.0:
+        raise ValueError(f"{name} must lie in [0, 1] (0 = off), got {cond_drop_prob}")
+    if cond_drop_prob > 0.0 and not trains_by_diffusion:
+        raise ValueError(f"{name} applies to the diffusion denoiser only (classifier-free guidance)")
+
+
 class Trainer:
+    COND_DROP_SEED = 0x63666764         # Philox key constant of the condition-dropout masks
+    cond_drop_prob = 0.0
+
     def __init__(self, model, opt_type: str = "rmsprop", lr: float = 1e-4, args: Optional[argparse.Namespace] = None,
                  diffusion: Optional[GaussianDiffusion] = None, bucket_mb: float = 8.0, seed: int = 0, ema_decay: float = 0.0,
                  clip_grad_norm: float = 0.0, lr_warmup_steps: int = 0, lr_schedule: str = "constant", lr_min: float = 0.0,
-                 total_steps: Optional[int] = None):
+                 total_steps: Optional[int] = None, cond_drop_prob: float = 0.0):
         if not 0.0 <= ema_decay < 1.0:
             raise ValueError(f"ema_decay must be in [0, 1) (0 = no EMA), got {ema_decay}")
         check_clip_sched(lr, clip_grad_norm, lr_warmup_steps, lr_schedule, lr_min, total_steps)
+        check_cond_drop(cond_drop_prob, getattr(model, "trains_by_diffusion", False))
         self.model = model
         self.eng = model.engine()
         self.arena = model.arena
@@ -143,6 +157,11 @@ class Trainer:
         self.total_steps = int(total_steps) if total_steps is not None else 0
         self.scheduled = self.lr_warmup_steps > 0 or lr_schedule != "constant"
         self._clip_ws = ops.GradClipWorkspace(dev) if self.clip_grad_norm > 0 else None
+        # classifier-free guidance training: the denoiser's condition is zeroed for a random fraction of the windows of each
+        # step, Philox keyed by (COND_DROP_SEED ^ trainer seed) + rank and offset by the global step count, so every rank
+        # draws its own masks and a resumed run continues the sequence
+        self.cond_drop_prob = float(cond_drop_prob)
+        self._cond_drop_seed = (self.COND_DROP_SEED ^ ((seed * 0x9E3779B1) & 0x7FFFFFFF)) + self.rank
         # device-resident 1-based step counter: incremented by a one-thread kernel at the start of every step, read by the
         # dropout kernels (Philox offset) and the optimizer kernel (Adam / Adamax bias correction), so that a captured step
         # can be replayed although those values change from step to step
@@ -284,6 +303,9 @@ class Trainer:
             t.copy_(torch.randint(0, self.diffusion.T, (B,), device=t.device, generator=self._gen, dtype=torch.int32))
             xc, ld, _, _ = eng.input_layout(B, F, True)
             self.diffusion.q_sample(lab.view(B, -1), t, None, xt_bf16=xc, bf16_ld=ld, seed=self.seed + self.rank, offset=self.step_count)
+            if self.cond_drop_prob > 0.0:
+                # the null condition is all-zero kinematics; the in-projection's weight gradient reads the same zeroed rows
+                ops.cond_dropout(xc, B, F, 30, eng.c_in, self.cond_drop_prob, self._cond_drop_seed, self.step_count)
         Fo = lab.shape[1]
         outs = eng.quantity_views(eng.forward(B, F, True), B, F, Fo)
         labs, gviews = quantity_split(lab), eng.quantity_views(eng.dout(B, F), B, F, Fo)
@@ -431,6 +453,8 @@ class Trainer:
         if self._clip_sched_key() is not None:
             sd["ibm_b200"].update(clip_grad_norm=self.clip_grad_norm, lr_warmup_steps=self.lr_warmup_steps,
                                   lr_schedule=self.lr_schedule, lr_min=self.lr_min, total_steps=self.total_steps)
+        if self.cond_drop_prob > 0.0:
+            sd["ibm_b200"]["cond_drop_prob"] = self.cond_drop_prob
         return sd
 
     def load_optimizer_state_dict(self, sd: dict) -> None:
