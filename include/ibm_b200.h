@@ -217,6 +217,29 @@ int ibm_ddpm_guided_step(const float* x0_hat, int64_t x0_ld, const float* x_t, c
 int ibm_cond_dropout(void* xc_bf16, int64_t ld, int64_t B, int32_t F, int32_t col0, int32_t ncols, float p,
                      uint64_t seed, uint64_t offset, uint8_t* keep_out, void* stream);
 
+/* Builder-owned (DESIGN.md §3; NOT in the reference): probabilistic score of K sampled trajectories per window.
+ * draws: fp32 [K, B*F, 30] draw-major (draw k of window b, frame f at row k*B*F + b*F + f), the fp32 state
+ * GaussianDiffusion.sample returns for B*K windows whose conditions are K copies of the same B.  labels: fp32 [B, Fo, 30]
+ * (rows30); Fo = F scores every frame, Fo = 1 (last_frame) scores frame F-1 of each draw.  For each scored element with
+ * draws x_1..x_K and label y:
+ *   m    = (1/K) sum_k x_k                      (fp64 sum; written to mean_out fp32 [B, Fo, 30] as rounded)
+ *   s2   = 1/(K-1) sum_k (x_k - m)^2            (two-pass, from m)
+ *   pair = 1/(K(K-1)) sum_{i!=j} |x_i - x_j|    (mean pairwise distance: a per-component MDM MultiModality)
+ *   crps = (1/K) sum_k |x_k - y| - pair/2       (the fair CRPS, Ferro 2014: unbiased at every K)
+ *   se   = (m - y)^2
+ * CoP channels 0-2 (3-5) are scored only on rows whose label force triple 6-8 (9-11) passes the contact test of
+ * ibm_regression_loss_fwd at `threshold` (||f|| > threshold, bit for bit the same predicate); every other channel is scored
+ * on every row.  mean_out is written for every element.
+ * acc: fp64 [5, 30], caller-owned, row q channel c: += the batch's sum over scored elements of channel c of
+ *   q = 0 crps, 1 s2, 2 se, 3 pair, 4 the element count,
+ * so successive batches accumulate on the device.  Per-block partials and a last-arriving-block reduction in a fixed order:
+ * the same inputs on the same device give bit-identical accumulators.  Workspace, caller-owned: partials = 1024 * 150
+ * doubles, counter = one uint32 that is zero before the first call (the kernel resets it).  2 <= K <= 64: the kernel holds
+ * the K draws of an element in registers.  Buffers contiguous, fp32 ones 4-byte and fp64 ones 8-byte aligned.  No allocation
+ * or host synchronisation: the call can be captured in a CUDA graph. */
+int ibm_ensemble_score(const float* draws, int32_t K, int64_t B, int32_t F, const float* labels, int32_t Fo, float threshold,
+                       float* mean_out, double* acc, double* partials, uint32_t* counter, void* stream);
+
 /* sinusoidal timestep embedding, bf16 [B, dim] (ld = dim): [sin(t w_k) | cos(t w_k)],
  * w_k = 10000^(-k/(dim/2)).  t: int32[B], or if t_is_scalar a single device int32 broadcast. */
 int ibm_timestep_embed(const int32_t* t, int32_t t_is_scalar, int64_t B, int32_t dim, void* out_bf16,

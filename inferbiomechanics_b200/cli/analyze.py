@@ -8,7 +8,9 @@ equal batch sizes keep the reference's mean-of-batch-means aggregate (Regression
 Per-window plots (matplotlib) and the names CSV are outside the hot path.  ``--model-type diffusion`` runs the
 reverse sampler per batch (``--sampler ddpm``: the 1000-step chain; ``ddim``: ``--sampling-steps`` respaced steps) and
 scores the sampled trajectories with the same evaluator; ``--guidance-scale`` samples it with classifier-free guidance, which
-needs a checkpoint trained with ``train --cond-drop-prob``.
+needs a checkpoint trained with ``train --cond-drop-prob``.  ``--num-samples K`` (K >= 2) draws K samples per window: the
+evaluator scores their mean and an ``EnsembleScorer`` block (CRPS, spread, spread-skill ratio, pairwise distance) follows
+the report.
 """
 from __future__ import annotations
 
@@ -20,8 +22,9 @@ import torch
 import torch.distributed as dist
 
 from .. import parallel
-from ..diffusion import GaussianDiffusion, check_guidance_scale
+from ..diffusion import MAX_NUM_SAMPLES, GaussianDiffusion, check_guidance_scale
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
+from ..loss.ensemble import EnsembleScorer
 from ..trainer import Trainer
 from . import _data
 from .abstract_command import AbstractCommand
@@ -74,6 +77,10 @@ class AnalyzeCommand(AbstractCommand):
                         help='--model-type diffusion: classifier-free guidance scale s (x0 = u + s (c - u)) with either '
                              'sampler; 1 = no guidance, 0 = unconditional. s != 1 needs a checkpoint trained with '
                              'train --cond-drop-prob > 0.')
+        sp.add_argument('--num-samples', type=int, default=1,
+                        help=f'--model-type diffusion: samples drawn per window (1..{MAX_NUM_SAMPLES}).  K >= 2 scores the '
+                             'ensemble mean with the evaluator and adds CRPS, spread, spread-skill ratio and mean pairwise '
+                             'distance per quantity; each launch then samples batch-size // K windows x K draws.')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'analyze':
@@ -85,6 +92,10 @@ class AnalyzeCommand(AbstractCommand):
         guidance = args.guidance_scale
         if guidance != 1.0:
             self.check_guidance_checkpoint(model_type, guidance, checkpoint_dir)
+        K = args.num_samples
+        self.check_num_samples(model_type, K, args.batch_size)
+        # windows per launch: K draws each, so that every launch but the last holds the same number of windows
+        per_launch = args.batch_size // K
         root_history_len = 10
         rank, world, local = parallel.init_from_env("nccl")
         torch.cuda.set_device(local)
@@ -106,7 +117,7 @@ class AnalyzeCommand(AbstractCommand):
             import wandb
             wandb.init(project="addbiomechanics-baseline", config=dict(args.__dict__))
 
-        reports = {}
+        reports, ensemble_reports = {}, {}
         for split, seed in (('dev', 4321), ('train', 1234)):
             logging.info(f'## Loading {split} dataset:')
             store = _data.open_split(args, split, model_type, device, seed=seed)
@@ -114,19 +125,21 @@ class AnalyzeCommand(AbstractCommand):
             shard = parallel.contiguous_shard(n, rank, world)
             idx_all = torch.arange(shard.start, shard.stop, device=device)
             log, ev = _ResultLog(split), RegressionLossEvaluator(None, split, device=device)
+            scorer = EnsembleScorer(K, split, device=device) if K > 1 else None
             with torch.no_grad():
-                for i in range(0, idx_all.numel(), args.batch_size):
-                    idx = idx_all[i:i + args.batch_size]
+                for i in range(0, idx_all.numel(), per_launch):
+                    idx = idx_all[i:i + per_launch]
                     if native:
                         log.add(trainer.eval_step(store, idx))
                         continue
                     if model_type == 'diffusion':
+                        ens = dict(num_samples=K, scorer=scorer) if scorer is not None else {}
                         if args.sampler == 'ddim':
                             sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, ddim_steps=args.sampling_steps,
-                                             eta=args.eta, guidance_scale=guidance)
+                                             eta=args.eta, guidance_scale=guidance, **ens)
                         else:
                             sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, steps=args.sampling_steps,
-                                             guidance_scale=guidance)
+                                             guidance_scale=guidance, **ens)
                         continue
                     inputs = input_dict(store, idx, model_type, args.stride, root_history_len)
                     ev(inputs, model(inputs), label_dict(store, idx), [], [], args)
@@ -144,14 +157,33 @@ class AnalyzeCommand(AbstractCommand):
                 merged = [g[:int(c.item())] for g, c in zip(gathered, counts)]
                 src._results = [r for g in merged for r in g]
                 src._wm_results = list(src._results)
+            if scorer is not None:
+                scorer.merge(world)
             if rank == 0:
-                print(f'{split} set evaluation ({n} windows' + (f', guidance scale {guidance:g}' if guidance != 1.0 else '') + '):')
+                print(f'{split} set evaluation ({n} windows' + (f', guidance scale {guidance:g}' if guidance != 1.0 else '') +
+                      (f', ensemble mean of {K} samples' if scorer is not None else '') + '):')
                 reports[split] = src.aggregate()
                 src.print_report(args, log_to_wandb=not args.no_wandb)
+                if scorer is not None:
+                    ensemble_reports[split] = scorer.summary()
+                    scorer.print_report(args, log_to_wandb=not args.no_wandb, summary=ensemble_reports[split])
         if dist.is_initialized():
             dist.destroy_process_group()
         self.last_reports = reports
+        self.last_ensemble_reports = ensemble_reports
         return True
+
+    @staticmethod
+    def check_num_samples(model_type: str, num_samples: int, batch_size: int) -> None:
+        """ValueError unless ``--num-samples`` can run: 1 <= K <= 64, K >= 2 for the diffusion model only, K <= --batch-size
+        (each launch samples batch-size // K windows x K draws)."""
+        if not 1 <= num_samples <= MAX_NUM_SAMPLES:
+            raise ValueError(f"--num-samples must lie in [1, {MAX_NUM_SAMPLES}], got {num_samples}")
+        if num_samples > 1 and model_type != 'diffusion':
+            raise ValueError("--num-samples > 1 applies to --model-type diffusion only")
+        if num_samples > batch_size:
+            raise ValueError(f"--num-samples {num_samples} exceeds --batch-size {batch_size}: a launch samples batch-size // K "
+                             "windows x K draws")
 
     def check_guidance_checkpoint(self, model_type: str, guidance_scale: float, checkpoint_dir: str) -> None:
         """ValueError unless guidance can run: a diffusion model, a finite scale >= 0 and a latest checkpoint whose optimizer

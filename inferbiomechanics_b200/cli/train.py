@@ -47,24 +47,37 @@ def input_dict(store: WindowStore, idx: torch.Tensor, model_type: str, stride: i
 QUANTITY_CUTS = [(0, 6), (6, 12), (12, 18), (18, 30)]       # column ranges of the four loss quantities in a 30-wide row
 
 
+def quantity_dict(rows: torch.Tensor):
+    """The four loss quantities of (B, F, 30) rows30, as views."""
+    return {k: rows[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, QUANTITY_CUTS)}
+
+
 def label_dict(store: WindowStore, idx: torch.Tensor):
-    lab = store.labels(idx)
-    return {k: lab[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, QUANTITY_CUTS)}
+    return quantity_dict(store.labels(idx))
 
 
 def sample_and_score(diffusion, model, store: WindowStore, idx: torch.Tensor, ev: RegressionLossEvaluator, args, seed: int,
-                     *, steps=None, ddim_steps=None, eta: float = 0.0, guidance_scale: float = 1.0) -> None:
+                     *, steps=None, ddim_steps=None, eta: float = 0.0, guidance_scale: float = 1.0, num_samples: int = 1,
+                     scorer=None) -> None:
     """Reverse-sample the denoiser's trajectories for windows ``idx`` of ``store`` and score them with ``ev`` against the
     store's labels: the condition is the packed kinematics in the engine's concat buffer, x_T ~ Philox(``seed``), and
     ``steps`` / ``ddim_steps`` / ``eta`` select the sampler and ``guidance_scale`` the classifier-free guidance as in
-    ``GaussianDiffusion.sample``."""
+    ``GaussianDiffusion.sample``.  ``num_samples`` K >= 2 draws K samples per window: ``scorer`` (an ``EnsembleScorer`` for
+    K draws) accumulates their probabilistic scores and ``ev`` scores the ensemble mean."""
     store.pack(idx, model.engine().input_layout(idx.numel(), store.F, False))
+    if num_samples > 1:
+        if scorer is None or scorer.K != num_samples:
+            raise ValueError(f"num_samples={num_samples} needs an EnsembleScorer for {num_samples} draws")
+        draws = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
+                                 guidance_scale=guidance_scale, num_samples=num_samples)
+        labels = store.labels(idx)
+        ev({}, quantity_dict(scorer.score(draws, labels)), quantity_dict(labels), [], [], args)
+        return
     x0 = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
                           guidance_scale=guidance_scale)
     if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
         x0 = x0[:, -1:]
-    outputs = {k: x0[:, :, a:b] for k, (a, b) in zip(LOSS_QUANTITIES, QUANTITY_CUTS)}
-    ev({}, outputs, label_dict(store, idx), [], [], args)
+    ev({}, quantity_dict(x0), label_dict(store, idx), [], [], args)
 
 
 class _ResultLog:

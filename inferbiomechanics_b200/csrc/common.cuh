@@ -3,6 +3,7 @@
 
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -82,6 +83,23 @@ __device__ __forceinline__ float4 ld_stream_f4(const float* p) {
 }
 __device__ __forceinline__ void st_stream_f4(float* p, float4 v) {
   st_stream16(p, make_uint4(__float_as_uint(v.x), __float_as_uint(v.y), __float_as_uint(v.z), __float_as_uint(v.w)));
+}
+
+// The CoP contact test of the reference evaluator (mask_by_threes on the label force, threshold 10.0 at
+// RegressionLossEvaluator.py:205-209): ||f|| > thr, strict, the norm accumulated as (a*a + b*b) + c*c without FMA
+// contraction like the reference's fp32 torch.norm.  norm3_gt2 is the same predicate without the square root, with
+// thr2 = norm3_threshold_sq(thr) from the host; the loss and ensemble kernels share both so their contact decisions agree.
+__device__ __forceinline__ bool norm3_gt2(float a, float b, float c, float thr2) {
+  return __fadd_rn(__fadd_rn(__fmul_rn(a, a), __fmul_rn(b, b)), __fmul_rn(c, c)) > thr2;
+}
+// largest fp32 x with sqrtf(x) <= thr, so that (sqrtf(n2) > thr)  <=>  (n2 > x) bit for bit (sqrtf is correctly rounded and
+// monotonic, so this is exact); -1 for a negative threshold, which every norm exceeds
+static inline float norm3_threshold_sq(float thr) {
+  if (thr < 0.f) return -1.f;
+  float x = thr * thr;
+  while (sqrtf(nextafterf(x, INFINITY)) <= thr) x = nextafterf(x, INFINITY);
+  while (x > 0.f && sqrtf(x) > thr) x = nextafterf(x, -INFINITY);
+  return x;
 }
 
 // activations and their derivatives expressed through the activation OUTPUT y

@@ -56,10 +56,7 @@ __device__ __forceinline__ bool norm3_gt(float a, float b, float c, float thr) {
   float n2 = __fadd_rn(__fadd_rn(__fmul_rn(a, a), __fmul_rn(b, b)), __fmul_rn(c, c));
   return sqrtf(n2) > thr;
 }
-// same predicate without the square root: thr2 is computed on the host so that the two agree exactly
-__device__ __forceinline__ bool norm3_gt2(float a, float b, float c, float thr2) {
-  return __fadd_rn(__fadd_rn(__fmul_rn(a, a), __fmul_rn(b, b)), __fmul_rn(c, c)) > thr2;
-}
+// the same predicate without the square root is norm3_gt2 (common.cuh), shared with the ensemble kernel
 __device__ __forceinline__ bool force_mask(const float* f3, float thr) {
   return norm3_gt(__ldg(f3), __ldg(f3 + 1), __ldg(f3 + 2), thr);
 }
@@ -533,14 +530,7 @@ static int fill_params(LossParams& p, const void* const* h_out, const int64_t* o
   }
   for (int c = 0; c < 30; ++c) p.w[c] = w[c];
   p.B = B; p.F = F; p.thr = thr;
-  // largest fp32 x with sqrtf(x) <= thr (sqrtf is correctly rounded and monotonic, so this is exact)
-  float x = thr * thr;
-  if (thr < 0.f) x = -1.f;                       // every norm exceeds a negative threshold
-  else {
-    while (sqrtf(nextafterf(x, INFINITY)) <= thr) x = nextafterf(x, INFINITY);
-    while (x > 0.f && sqrtf(x) > thr) x = nextafterf(x, -INFINITY);
-  }
-  p.thr2 = x;
+  p.thr2 = norm3_threshold_sq(thr);
   return IBM_OK;
 }
 

@@ -66,6 +66,14 @@ def check_guidance_scale(guidance_scale: float) -> None:
         raise ValueError(f"guidance_scale must be finite and >= 0 (1 = no guidance, 0 = unconditional), got {guidance_scale}")
 
 
+MAX_NUM_SAMPLES = 64             # draws per window: the bound of the ensemble scoring kernel (ops.ENSEMBLE_MAX_DRAWS)
+
+
+def check_num_samples(num_samples: Optional[int]) -> None:
+    if num_samples is not None and not (isinstance(num_samples, int) and 1 <= num_samples <= MAX_NUM_SAMPLES):
+        raise ValueError(f"num_samples must be None or an int in [1, {MAX_NUM_SAMPLES}], got {num_samples!r}")
+
+
 def _check_schedule(T: int, steps: Optional[int], ddim_steps: Optional[int], eta: float) -> None:
     if steps is not None and ddim_steps is not None:
         raise ValueError("give either steps (a truncated DDPM chain) or ddim_steps (a respaced DDIM sequence), not both")
@@ -125,7 +133,7 @@ class GaussianDiffusion:
     @torch.no_grad()
     def sample(self, model, B: int, *, x_T: Optional[torch.Tensor] = None, noise: Optional[Callable[[int], torch.Tensor]] = None,
                steps: Optional[int] = None, seed: int = 0, use_graph: bool = True, ddim_steps: Optional[int] = None,
-               eta: float = 0.0, guidance_scale: float = 1.0) -> torch.Tensor:
+               eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None) -> torch.Tensor:
         """Reverse-sample x_0 (B,F,30) for the kinematics already packed in model.engine().xc(B, False)
         (columns 30…).  ``noise(t)`` supplies z per step for parity tests; None ⇒ on-device Philox.
 
@@ -136,9 +144,25 @@ class GaussianDiffusion:
         ``guidance_scale`` s != 1: classifier-free guidance with either sampler.  The kinematics of xc(B) are copied into
         the first half of xc(2B) and the second half gets the null condition (zeros); x_T goes into both halves, each step
         runs the forward on 2B windows and the guided step kernel.  s = 1 runs the unguided loop, s = 0 samples
-        unconditionally.  The result depends on s only through the prediction: x_T and the noise are those of s = 1."""
+        unconditionally.  The result depends on s only through the prediction: x_T and the noise are those of s = 1.
+
+        ``num_samples`` K (1..64): K independent draws per window.  The B packed conditions are copied into K consecutive
+        blocks of xc(B*K) and the loop above runs on B*K windows; the result is (K, B, F, 30), draw k of window b at row
+        k*B*F + b*F + f of the fp32 state (the layout ``ops.ensemble_score`` reads).  x_T and the noise are Philox draws indexed
+        by element, so the draws are independent and draw 0 starts from the x_T and noise of a call without ``num_samples``."""
         _check_schedule(self.T, steps, ddim_steps, eta)
         check_guidance_scale(guidance_scale)
+        check_num_samples(num_samples)
+        if num_samples is not None:
+            eng = model.engine()
+            src = eng.xc(B, False)
+            dst = eng.xc(B * num_samples, False)
+            M = src.shape[0]
+            for k in range(num_samples):
+                dst[k * M:(k + 1) * M].copy_(src)
+            x0 = self.sample(model, B * num_samples, x_T=x_T, noise=noise, steps=steps, seed=seed, use_graph=use_graph,
+                             ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale)
+            return x0.view(num_samples, B, eng.F, 30)
         guided = guidance_scale != 1.0
         eng = model.engine()
         F, M = eng.F, B * eng.F
@@ -232,7 +256,7 @@ class GaussianDiffusion:
     @torch.no_grad()
     def sample_windows(self, model, cond: torch.Tensor, *, batch: int = 512, steps: Optional[int] = None, seed: int = 0,
                        rank: Optional[int] = None, world: Optional[int] = None, ddim_steps: Optional[int] = None,
-                       eta: float = 0.0, guidance_scale: float = 1.0):
+                       eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None):
         """Reverse-sample GRF / CoP / torque / wrench trajectories for ``cond``: (N, F, C_in) fp32 packed kinematics of N
         windows (model concat order, FeedForward...py:97-108) in HOST memory (pinned for asynchronous copies).
 
@@ -241,10 +265,12 @@ class GaussianDiffusion:
         ``steps`` (default: the full schedule) CUDA-graph-replayed denoise steps, D2H copy of the trajectories — and returns
         ``(range, x0)`` with x0 a pinned host tensor (len(range), F, 30).  No collective; per-rank noise stream = seed + rank.
         The copies of batch i+1 / i-1 overlap the sampling of batch i (separate streams).  ``ddim_steps`` / ``eta`` select
-        DDIM sampling and ``guidance_scale`` classifier-free guidance as in ``sample``."""
+        DDIM sampling and ``guidance_scale`` classifier-free guidance as in ``sample``.  ``num_samples`` K: K draws per window
+        (``sample(..., num_samples=K)`` per batch, ``batch`` still counts windows) and x0 is (len(range), K, F, 30)."""
         from . import parallel
         _check_schedule(self.T, steps, ddim_steps, eta)
         check_guidance_scale(guidance_scale)
+        check_num_samples(num_samples)
         r, w = parallel.world()
         rank = r if rank is None else rank
         world = w if world is None else world
@@ -253,7 +279,8 @@ class GaussianDiffusion:
         N = cond.shape[0]
         assert tuple(cond.shape[1:]) == (F, C) and not cond.is_cuda, "cond: host tensor (N, F, C_in)"
         mine = parallel.contiguous_shard(N, rank, world)
-        out = torch.empty(len(mine), F, 30, dtype=torch.float32).pin_memory()
+        shape = (len(mine), F, 30) if num_samples is None else (len(mine), num_samples, F, 30)
+        out = torch.empty(shape, dtype=torch.float32).pin_memory()
         dev = self.device
         main = torch.cuda.current_stream(dev)
         up, down = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
@@ -284,7 +311,9 @@ class GaussianDiffusion:
             if i + 1 < len(starts):
                 upload(i + 1)
             x0 = self.sample(model, nb, steps=steps, seed=seed + rank + 7919 * i, ddim_steps=ddim_steps, eta=eta,
-                             guidance_scale=guidance_scale)
+                             guidance_scale=guidance_scale, num_samples=num_samples)
+            if num_samples is not None:
+                x0 = x0.transpose(0, 1)                       # (nb, K, F, 30): window-major for the caller
             ready = torch.cuda.Event()
             ready.record(main)
             with torch.cuda.stream(down):

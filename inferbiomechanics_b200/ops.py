@@ -312,6 +312,48 @@ def cond_dropout(xc, B, F, col0, ncols, p, seed, offset, keep_out=None):
     call("ibm_cond_dropout", _p(xc), xc.stride(0), B, F, col0, ncols, p, seed, offset, _p(keep_out), stream_ptr())
 
 
+# ---- ensemble scoring -------------------------------------------------------------------------------
+ENSEMBLE_MAX_DRAWS = 64          # ibm_ensemble_score holds the K draws of an element in registers
+ENSEMBLE_QUANTITIES = ("crps", "var", "sqerr", "pair", "count")     # rows of the fp64 [5, 30] accumulator
+
+
+class EnsembleWorkspace:
+    """Device buffers of ``ensemble_score``: the per-block partials (1024 x 150 fp64) and the last-block counter."""
+
+    def __init__(self, device):
+        self.partials = torch.zeros(1024 * 150, dtype=torch.float64, device=device)
+        self.counter = torch.zeros(1, dtype=torch.int32, device=device)
+
+
+def ensemble_score(draws: torch.Tensor, labels: torch.Tensor, acc: torch.Tensor, mean_out: torch.Tensor, ws: EnsembleWorkspace,
+                   threshold: float = 10.0) -> torch.Tensor:
+    """Scores K draws per window (``ibm_ensemble_score``): draws fp32 (K, B, F, 30) draw-major, as ``GaussianDiffusion.sample(...,
+    num_samples=K)`` returns them; labels fp32 (B, Fo, 30) with Fo in {1, F}.  Writes the ensemble mean to ``mean_out`` (B, Fo, 30)
+    and adds the batch's per-channel sums of CRPS, s^2, (m - y)^2, mean pairwise distance and the count to ``acc`` (fp64 [5, 30],
+    rows in ENSEMBLE_QUANTITIES order).  CoP channels count contact rows only (label force norm > ``threshold``, the fused loss
+    kernel's test).  Every check runs before the launch: a refused call launches nothing.  Returns ``mean_out``."""
+    for name, t, dt in (("draws", draws, torch.float32), ("labels", labels, torch.float32), ("mean_out", mean_out, torch.float32),
+                        ("acc", acc, torch.float64)):
+        if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != dt or not t.is_contiguous():
+            raise ValueError(f"ensemble_score: {name} must be a contiguous {dt} CUDA tensor")
+    if draws.dim() != 4 or draws.shape[-1] != 30:
+        raise ValueError(f"ensemble_score: draws must be (K, B, F, 30), got {tuple(draws.shape)}")
+    K, B, F = draws.shape[:3]
+    if not 2 <= K <= ENSEMBLE_MAX_DRAWS:
+        raise ValueError(f"ensemble_score: K must lie in [2, {ENSEMBLE_MAX_DRAWS}], got {K}")
+    if labels.dim() != 3 or labels.shape[0] != B or labels.shape[2] != 30 or labels.shape[1] not in (1, F):
+        raise ValueError(f"ensemble_score: labels must be (B={B}, 1 or F={F}, 30), got {tuple(labels.shape)}")
+    if tuple(mean_out.shape) != tuple(labels.shape):
+        raise ValueError(f"ensemble_score: mean_out must have the labels' shape {tuple(labels.shape)}, got {tuple(mean_out.shape)}")
+    if tuple(acc.shape) != (len(ENSEMBLE_QUANTITIES), 30):
+        raise ValueError(f"ensemble_score: acc must be fp64 (5, 30), got {tuple(acc.shape)}")
+    if B == 0 or F == 0:
+        raise ValueError("ensemble_score: empty batch")
+    call("ibm_ensemble_score", _p(draws), K, B, F, _p(labels), labels.shape[1], float(threshold), _p(mean_out), _p(acc),
+         _p(ws.partials), _p(ws.counter), stream_ptr())
+    return mean_out
+
+
 def timestep_embed(t, out_bf16, dim, scalar=False):
     B = out_bf16.shape[0]
     call("ibm_timestep_embed", _p(t), int(scalar), B, dim, _p(out_bf16), stream_ptr())
