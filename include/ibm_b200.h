@@ -209,6 +209,21 @@ int ibm_ddpm_guided_step(const float* x0_hat, int64_t x0_ld, const float* x_t, c
                          int64_t bf16_ld, uint64_t seed, uint64_t offset, int32_t* t_next_dev,
                          const int32_t* t_succ, float guidance_scale, void* stream);
 
+/* Builder-owned (DESIGN.md D-1; NOT in the reference): inpainting.  One step of ibm_ddpm_guided_step (guided != 0) or of
+ * the unguided posterior / respaced step (guided == 0; t_succ selects as there, guidance_scale is checked and unused) in
+ * which the known entries of the prediction are held fixed: after the guided combination, and before the unchanged update,
+ * [t>0] noise gate and Philox counter offset + t,
+ *   x0_hat[m, c] = known[m, c]  where bit c of known_mask[m] is set,  else the prediction.
+ * A select, not a blend: an entry of `known` whose bit is clear is never read into the result (it may hold NaN).
+ * known: fp32 [M, 30] contiguous, 8-byte aligned.  known_mask: int32 [M], one word per row, bits 0..29 = channels,
+ * bits 30-31 ignored.  Both are required; everything ibm_ddpm_guided_step refuses is refused too. */
+int ibm_ddpm_inpaint_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const float* z,
+                          const int32_t* t_dev, const float* coef_x0, const float* coef_xt,
+                          const float* sigma, int64_t M, float* x_prev, void* xprev_bf16,
+                          int64_t bf16_ld, uint64_t seed, uint64_t offset, int32_t* t_next_dev,
+                          const int32_t* t_succ, float guidance_scale, int32_t guided, const float* known,
+                          const int32_t* known_mask, void* stream);
+
 /* Per-window condition dropout for classifier-free guidance training.  xc: bf16 [B*F, ld] (window b
  * owns rows b*F .. b*F+F-1).  Window b is dropped iff word 0 of Philox4x32-10 draw b at (seed, offset)
  * is below uint32(p * 2^32) (the keep rule of the dropout kernels); p >= 1 drops every window without

@@ -36,6 +36,7 @@ SIGNATURES = {
     "ibm_ddpm_posterior_step": [P, _i64, P, P, P, P, P, P, _i64, P, P, _i64, _u64, _u64, P, P],
     "ibm_ddpm_respaced_step": [P, _i64, P, P, P, P, P, P, _i64, P, P, _i64, _u64, _u64, P, P, P],
     "ibm_ddpm_guided_step": [P, _i64, P, P, P, P, P, P, _i64, P, P, _i64, _u64, _u64, P, P, _f, P],
+    "ibm_ddpm_inpaint_step": [P, _i64, P, P, P, P, P, P, _i64, P, P, _i64, _u64, _u64, P, P, _f, _i32, P, P, P],
     "ibm_cond_dropout": [P, _i64, _i64, _i32, _i32, _i32, _f, _u64, _u64, P, P],
     "ibm_ensemble_score": [P, _i32, _i64, _i32, P, _i32, _f, P, P, P, P, P],
     "ibm_timestep_embed": [P, _i32, _i64, _i32, P, P],

@@ -10,7 +10,8 @@ reverse sampler per batch (``--sampler ddpm``: the 1000-step chain; ``ddim``: ``
 scores the sampled trajectories with the same evaluator; ``--guidance-scale`` samples it with classifier-free guidance, which
 needs a checkpoint trained with ``train --cond-drop-prob``.  ``--num-samples K`` (K >= 2) draws K samples per window: the
 evaluator scores their mean and an ``EnsembleScorer`` block (CRPS, spread, spread-skill ratio, pairwise distance) follows
-the report.
+the report.  ``--given-quantities force ...`` gives the sampler the labels of those quantities as known values (inpainting):
+they come back exactly, and the report's other quantities are the prediction conditioned on them.
 """
 from __future__ import annotations
 
@@ -24,7 +25,7 @@ import torch.distributed as dist
 from .. import parallel
 from ..diffusion import MAX_NUM_SAMPLES, GaussianDiffusion, check_guidance_scale
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
-from ..loss.ensemble import EnsembleScorer
+from ..loss.ensemble import ENSEMBLE_GROUPS, EnsembleScorer
 from ..trainer import Trainer
 from . import _data
 from .abstract_command import AbstractCommand
@@ -81,6 +82,10 @@ class AnalyzeCommand(AbstractCommand):
                         help=f'--model-type diffusion: samples drawn per window (1..{MAX_NUM_SAMPLES}).  K >= 2 scores the '
                              'ensemble mean with the evaluator and adds CRPS, spread, spread-skill ratio and mean pairwise '
                              'distance per quantity; each launch then samples batch-size // K windows x K draws.')
+        sp.add_argument('--given-quantities', type=str, nargs='+', default=[], choices=list(ENSEMBLE_GROUPS),
+                        help='--model-type diffusion: quantities whose labels the sampler is given and holds fixed '
+                             '(inpainting); they read 0 error and the others are predicted conditionally on them.  Needs '
+                             '--output-data-format all_frames and the whole chain (not --sampler ddpm with --sampling-steps < 1000).')
 
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'analyze':
@@ -94,6 +99,8 @@ class AnalyzeCommand(AbstractCommand):
             self.check_guidance_checkpoint(model_type, guidance, checkpoint_dir)
         K = args.num_samples
         self.check_num_samples(model_type, K, args.batch_size)
+        given = tuple(args.given_quantities)
+        self.check_given_quantities(given, model_type, args)
         # windows per launch: K draws each, so that every launch but the last holds the same number of windows
         per_launch = args.batch_size // K
         root_history_len = 10
@@ -134,6 +141,8 @@ class AnalyzeCommand(AbstractCommand):
                         continue
                     if model_type == 'diffusion':
                         ens = dict(num_samples=K, scorer=scorer) if scorer is not None else {}
+                        if given:
+                            ens["known_quantities"] = given
                         if args.sampler == 'ddim':
                             sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, ddim_steps=args.sampling_steps,
                                              eta=args.eta, guidance_scale=guidance, **ens)
@@ -161,12 +170,13 @@ class AnalyzeCommand(AbstractCommand):
                 scorer.merge(world)
             if rank == 0:
                 print(f'{split} set evaluation ({n} windows' + (f', guidance scale {guidance:g}' if guidance != 1.0 else '') +
-                      (f', ensemble mean of {K} samples' if scorer is not None else '') + '):')
+                      (f', ensemble mean of {K} samples' if scorer is not None else '') +
+                      (f', given {" ".join(given)}' if given else '') + '):')
                 reports[split] = src.aggregate()
                 src.print_report(args, log_to_wandb=not args.no_wandb)
                 if scorer is not None:
                     ensemble_reports[split] = scorer.summary()
-                    scorer.print_report(args, log_to_wandb=not args.no_wandb, summary=ensemble_reports[split])
+                    scorer.print_report(args, log_to_wandb=not args.no_wandb, summary=ensemble_reports[split], given=given)
         if dist.is_initialized():
             dist.destroy_process_group()
         self.last_reports = reports
@@ -184,6 +194,20 @@ class AnalyzeCommand(AbstractCommand):
         if num_samples > batch_size:
             raise ValueError(f"--num-samples {num_samples} exceeds --batch-size {batch_size}: a launch samples batch-size // K "
                              "windows x K draws")
+
+    @staticmethod
+    def check_given_quantities(given, model_type: str, args) -> None:
+        """ValueError unless ``--given-quantities`` can run: a diffusion model, labels of every frame (the known values are the
+        labels) and the whole chain (a truncated DDPM chain stops before the step that returns the known values)."""
+        if not given:
+            return
+        if model_type != 'diffusion':
+            raise ValueError("--given-quantities applies to --model-type diffusion only")
+        if args.output_data_format != 'all_frames':
+            raise ValueError("--given-quantities needs --output-data-format all_frames: last_frame labels hold one frame")
+        if args.sampler == 'ddpm' and args.sampling_steps < 1000:
+            raise ValueError(f"--given-quantities needs the whole chain: --sampler ddpm --sampling-steps {args.sampling_steps} "
+                             "truncates it")
 
     def check_guidance_checkpoint(self, model_type: str, guidance_scale: float, checkpoint_dir: str) -> None:
         """ValueError unless guidance can run: a diffusion model, a finite scale >= 0 and a latest checkpoint whose optimizer

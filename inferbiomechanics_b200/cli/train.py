@@ -25,6 +25,7 @@ from ..data.window_store import WindowStore
 from ..diffusion import GaussianDiffusion
 from ..keys import LOSS_QUANTITIES, MODEL_INPUT_ORDER
 from ..loss.RegressionLossEvaluator import RegressionLossEvaluator
+from ..loss.ensemble import ENSEMBLE_GROUPS
 from ..trainer import LR_SCHEDULES, Trainer, check_clip_sched, check_cond_drop
 from . import _data
 from .abstract_command import AbstractCommand
@@ -56,25 +57,43 @@ def label_dict(store: WindowStore, idx: torch.Tensor):
     return quantity_dict(store.labels(idx))
 
 
+def known_quantity_mask(quantities) -> torch.Tensor:
+    """bool (30,): the rows30 channels of the named quantities (keys of ``ENSEMBLE_GROUPS``: force, cop, moment, wrench)."""
+    mask = torch.zeros(30, dtype=torch.bool)
+    for q in quantities:
+        if q not in ENSEMBLE_GROUPS:
+            raise ValueError(f"unknown quantity {q!r}: choose from {', '.join(ENSEMBLE_GROUPS)}")
+        a, b = ENSEMBLE_GROUPS[q][0]
+        mask[a:b] = True
+    return mask
+
+
 def sample_and_score(diffusion, model, store: WindowStore, idx: torch.Tensor, ev: RegressionLossEvaluator, args, seed: int,
                      *, steps=None, ddim_steps=None, eta: float = 0.0, guidance_scale: float = 1.0, num_samples: int = 1,
-                     scorer=None) -> None:
+                     scorer=None, known_quantities=()) -> None:
     """Reverse-sample the denoiser's trajectories for windows ``idx`` of ``store`` and score them with ``ev`` against the
     store's labels: the condition is the packed kinematics in the engine's concat buffer, x_T ~ Philox(``seed``), and
     ``steps`` / ``ddim_steps`` / ``eta`` select the sampler and ``guidance_scale`` the classifier-free guidance as in
     ``GaussianDiffusion.sample``.  ``num_samples`` K >= 2 draws K samples per window: ``scorer`` (an ``EnsembleScorer`` for
-    K draws) accumulates their probabilistic scores and ``ev`` scores the ensemble mean."""
+    K draws) accumulates their probabilistic scores and ``ev`` scores the ensemble mean.  ``known_quantities`` (names of
+    ``ENSEMBLE_GROUPS``): the store's labels of those quantities are given to the sampler as known values (inpainting), so
+    the others are predicted conditionally on them; needs labels of every frame."""
     store.pack(idx, model.engine().input_layout(idx.numel(), store.F, False))
+    given = {}
+    if known_quantities:
+        if store.Fo != store.F:
+            raise ValueError("known quantities need labels of every frame (--output-data-format all_frames)")
+        given = dict(known=store.labels(idx), known_mask=known_quantity_mask(known_quantities))
     if num_samples > 1:
         if scorer is None or scorer.K != num_samples:
             raise ValueError(f"num_samples={num_samples} needs an EnsembleScorer for {num_samples} draws")
         draws = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
-                                 guidance_scale=guidance_scale, num_samples=num_samples)
+                                 guidance_scale=guidance_scale, num_samples=num_samples, **given)
         labels = store.labels(idx)
         ev({}, quantity_dict(scorer.score(draws, labels)), quantity_dict(labels), [], [], args)
         return
     x0 = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
-                          guidance_scale=guidance_scale)
+                          guidance_scale=guidance_scale, **given)
     if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
         x0 = x0[:, -1:]
     ev({}, quantity_dict(x0), label_dict(store, idx), [], [], args)

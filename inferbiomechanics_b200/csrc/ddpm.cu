@@ -66,21 +66,25 @@ q_sample_kernel(const float* __restrict__ x0, const float* __restrict__ eps, con
 // leading dimension (the head GEMM writes 32-float rows).  kSucc: the next timestep is t_succ[t]
 // (a respaced DDIM sequence) instead of t-1; the instantiation without it is the DDPM chain.  kGuided: x0h holds 2M
 // rows, conditional then unconditional, combined as u + s (c - u) (classifier-free guidance); the bf16 rows go to both
-// halves of the concat buffer.  gscale is the last parameter so the unguided instantiations keep their parameter offsets.
-template <bool kSucc, bool kGuided>
+// halves of the concat buffer.  gscale follows the parameters of the unguided instantiations so they keep their parameter
+// offsets.  kKnown (inpainting): after the guided combination, channel c of row m takes known[m, c] instead of the prediction
+// where bit c of kmask[m] is set (bits 30-31 are ignored); a select, so a NaN in an unknown entry of `known` never reaches
+// the output.  known / kmask come after gscale for the same reason.
+template <bool kSucc, bool kGuided, bool kKnown>
 __global__ void __launch_bounds__(kThreads)
 posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __restrict__ xt,
                  const float* __restrict__ z, const int32_t* __restrict__ t_dev, const float* __restrict__ c1t,
                  const float* __restrict__ c2t, const float* __restrict__ sig, long long M,
                  float* __restrict__ xprev, __nv_bfloat16* __restrict__ xp_bf16, long long bf16_ld,
                  uint64_t seed, uint64_t offset, int32_t* __restrict__ t_next,
-                 const int32_t* __restrict__ t_succ, float gscale) {
+                 const int32_t* __restrict__ t_succ, float gscale, const float* __restrict__ known,
+                 const int32_t* __restrict__ kmask) {
   const int tt = __ldg(t_dev);
   const float c1 = __ldg(c1t + tt), c2 = __ldg(c2t + tt);
   const float s = tt > 0 ? __ldg(sig + tt) : 0.f;
   const long long npair = M * 15;
   const long long stride = (long long)gridDim.x * blockDim.x;
-#pragma unroll 2
+#pragma unroll (kKnown ? 1 : 2)   // unrolled twice, the kKnown loop spills 8 bytes (CUDA 12.9)
   for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < npair; p += stride) {
     const long long m = p / 15, c = (p - m * 15) * 2;
     float2 a = *reinterpret_cast<const float2*>(x0h + m * x0_ld + c);
@@ -88,6 +92,14 @@ posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __
       const float2 u = *reinterpret_cast<const float2*>(x0h + (M + m) * x0_ld + c);
       a.x = fmaf(gscale, a.x - u.x, u.x);
       a.y = fmaf(gscale, a.y - u.y, u.y);
+    }
+    if (kKnown) {
+      const uint32_t w = (uint32_t)__ldg(kmask + m) >> c;
+      if (w & 3u) {
+        const float2 y = __ldg(reinterpret_cast<const float2*>(known + 2 * p));
+        if (w & 1u) a.x = y.x;
+        if (w & 2u) a.y = y.y;
+      }
     }
     const float2 x = *reinterpret_cast<const float2*>(xt + 2 * p);
     float2 n;
@@ -355,9 +367,9 @@ extern "C" int ibm_ddpm_posterior_step(const float* x0_hat, int64_t x0_ld, const
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "posterior_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "posterior_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "posterior_step: bf16 ld must be even");
-  posterior_kernel<false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<false, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev, nullptr, 0.f);
+      seed, offset, t_next_dev, nullptr, 0.f, nullptr, nullptr);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }
@@ -373,9 +385,9 @@ extern "C" int ibm_ddpm_respaced_step(const float* x0_hat, int64_t x0_ld, const 
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "respaced_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "respaced_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "respaced_step: bf16 ld must be even");
-  posterior_kernel<true, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<true, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev, t_succ, 0.f);
+      seed, offset, t_next_dev, t_succ, 0.f, nullptr, nullptr);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }
@@ -396,13 +408,48 @@ extern "C" int ibm_ddpm_guided_step(const float* x0_hat, int64_t x0_ld, const fl
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   auto* xb = static_cast<__nv_bfloat16*>(xprev_bf16);
   if (t_succ)
-    posterior_kernel<true, true><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
+    posterior_kernel<true, true, false><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
                                                                         x_prev, xb, bf16_ld, seed, offset, t_next_dev, t_succ,
-                                                                        guidance_scale);
+                                                                        guidance_scale, nullptr, nullptr);
   else
-    posterior_kernel<false, true><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
+    posterior_kernel<false, true, false><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
                                                                          x_prev, xb, bf16_ld, seed, offset, t_next_dev, nullptr,
-                                                                         guidance_scale);
+                                                                         guidance_scale, nullptr, nullptr);
+  IBM_LAUNCH_CHECK();
+  return IBM_OK;
+}
+
+extern "C" int ibm_ddpm_inpaint_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const float* z,
+                                     const int32_t* t_dev, const float* coef_x0, const float* coef_xt,
+                                     const float* sigma, int64_t M, float* x_prev, void* xprev_bf16, int64_t bf16_ld,
+                                     uint64_t seed, uint64_t offset, int32_t* t_next_dev, const int32_t* t_succ,
+                                     float guidance_scale, int32_t guided, const float* known, const int32_t* known_mask,
+                                     void* stream) {
+  using namespace ibm;
+  IBM_CHECK_ARCH();
+  IBM_CHECK_ARG(x0_hat && x_t && t_dev && coef_x0 && coef_xt && sigma, "inpaint_step: null argument");
+  IBM_CHECK_ARG(known && known_mask, "inpaint_step: null known values or known mask");
+  IBM_CHECK_ARG(reinterpret_cast<uintptr_t>(known) % 8 == 0, "inpaint_step: known values must be 8-byte aligned");
+  IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "inpaint_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
+  IBM_CHECK_ARG(x_prev || xprev_bf16, "inpaint_step: no output requested");
+  IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "inpaint_step: bf16 ld must be even");
+  IBM_CHECK_ARG(guidance_scale >= 0.f && guidance_scale <= 3.402823466e38f, "inpaint_step: guidance scale must be finite and >= 0, got %g",
+                (double)guidance_scale);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  auto* xb = static_cast<__nv_bfloat16*>(xprev_bf16);
+  const int grid = ew_grid(M * 15 / 2);
+#define IBM_INPAINT_LAUNCH(SUCC, GUIDED)                                                                                       \
+  posterior_kernel<SUCC, GUIDED, true><<<grid, kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,     \
+                                                                 x_prev, xb, bf16_ld, seed, offset, t_next_dev, t_succ,         \
+                                                                 guidance_scale, known, known_mask)
+  if (t_succ) {
+    if (guided) IBM_INPAINT_LAUNCH(true, true);
+    else IBM_INPAINT_LAUNCH(true, false);
+  } else {
+    if (guided) IBM_INPAINT_LAUNCH(false, true);
+    else IBM_INPAINT_LAUNCH(false, false);
+  }
+#undef IBM_INPAINT_LAUNCH
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }

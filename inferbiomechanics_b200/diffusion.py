@@ -17,6 +17,10 @@ with no collective.
 Classifier-free guidance (Ho & Salimans 2022) with scale s != 1 runs the forward on 2B windows per step, the B conditioned
 ones and the same B with all-zero kinematics (the null condition the trainer's ``cond_drop_prob`` teaches), and one guided
 step kernel combines x0_hat = u + s (c - u) before the same update; s = 0 is unconditional sampling.
+
+Inpainting (MDM's ``p_mean_variance`` for an x0-predicting model): given known values y and a known-mask, every step
+replaces the known entries of x0_hat (after the guided combination) by y before the unchanged update.  The last step of
+either sampler has coef_x0 = 1, coef_xt = 0 and no noise, so the sample equals y exactly wherever the mask is set.
 """
 from __future__ import annotations
 
@@ -72,6 +76,41 @@ MAX_NUM_SAMPLES = 64             # draws per window: the bound of the ensemble s
 def check_num_samples(num_samples: Optional[int]) -> None:
     if num_samples is not None and not (isinstance(num_samples, int) and 1 <= num_samples <= MAX_NUM_SAMPLES):
         raise ValueError(f"num_samples must be None or an int in [1, {MAX_NUM_SAMPLES}], got {num_samples!r}")
+
+
+def known_mask_words(mask: torch.Tensor, rows: int) -> torch.Tensor:
+    """int32 row words of a bool known-mask (rows, 30), or (30,) for every row: bit c of word m is set iff channel c of row m
+    is known (the ``known_mask`` of ``ops.posterior_step``).  A (30,) mask gives an expanded view of one word."""
+    w = (mask.to(torch.int32) << torch.arange(30, dtype=torch.int32, device=mask.device)).sum(-1, dtype=torch.int32)
+    return w.reshape(1).expand(rows) if mask.dim() == 1 else w.reshape(rows)
+
+
+def check_known(known, known_mask, B: int, F: Optional[int], T: int, steps: Optional[int], device=None) -> bool:
+    """ValueError unless (``known``, ``known_mask``) are inpainting inputs for B windows of F frames (None: not checked):
+    both or neither, known fp32 (B, F, 30) (on ``device`` if given), known_mask bool (B, F, 30) or (30,), and the whole
+    chain (a truncated DDPM chain stops before the step that returns the known values).  True when both are given."""
+    if known is None and known_mask is None:
+        return False
+    if known is None or known_mask is None:
+        raise ValueError("known and known_mask go together: give both or neither")
+    if not isinstance(known, torch.Tensor) or known.dtype != torch.float32 or known.dim() != 3 or known.shape[0] != B \
+            or known.shape[2] != 30 or (F is not None and known.shape[1] != F):
+        raise ValueError(f"known must be an fp32 tensor of shape (B={B}, F={F if F is not None else 'F'}, 30)"
+                         + (f", got {known.dtype} {tuple(known.shape)}" if isinstance(known, torch.Tensor) else ""))
+    if device is not None and not _on(known, device):
+        raise ValueError(f"known must be on {device}, got {known.device}")
+    if not isinstance(known_mask, torch.Tensor) or known_mask.dtype != torch.bool or \
+            tuple(known_mask.shape) not in ((30,), tuple(known.shape)):
+        raise ValueError(f"known_mask must be a bool tensor of shape (30,) or {tuple(known.shape)}"
+                         + (f", got {known_mask.dtype} {tuple(known_mask.shape)}" if isinstance(known_mask, torch.Tensor) else ""))
+    if steps is not None and steps < T:
+        raise ValueError(f"inpainting needs the whole chain: steps={steps} < {T} stops before the known values are returned")
+    return True
+
+
+def _on(t: torch.Tensor, device) -> bool:
+    device = torch.device(device)
+    return t.device.type == device.type and (device.index is None or t.device.index == device.index)
 
 
 def _check_schedule(T: int, steps: Optional[int], ddim_steps: Optional[int], eta: float) -> None:
@@ -133,7 +172,8 @@ class GaussianDiffusion:
     @torch.no_grad()
     def sample(self, model, B: int, *, x_T: Optional[torch.Tensor] = None, noise: Optional[Callable[[int], torch.Tensor]] = None,
                steps: Optional[int] = None, seed: int = 0, use_graph: bool = True, ddim_steps: Optional[int] = None,
-               eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None) -> torch.Tensor:
+               eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None,
+               known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Reverse-sample x_0 (B,F,30) for the kinematics already packed in model.engine().xc(B, False)
         (columns 30…).  ``noise(t)`` supplies z per step for parity tests; None ⇒ on-device Philox.
 
@@ -149,10 +189,31 @@ class GaussianDiffusion:
         ``num_samples`` K (1..64): K independent draws per window.  The B packed conditions are copied into K consecutive
         blocks of xc(B*K) and the loop above runs on B*K windows; the result is (K, B, F, 30), draw k of window b at row
         k*B*F + b*F + f of the fp32 state (the layout ``ops.ensemble_score`` reads).  x_T and the noise are Philox draws indexed
-        by element, so the draws are independent and draw 0 starts from the x_T and noise of a call without ``num_samples``."""
+        by element, so the draws are independent and draw 0 starts from the x_T and noise of a call without ``num_samples``.
+
+        ``known`` (fp32 (B, F, 30) on the device) with ``known_mask`` (bool, (B, F, 30) or (30,) for every row): inpainting.
+        Every step replaces the known entries of x0_hat (after the guidance combination) by ``known`` before the unchanged
+        update, so the sample equals ``known`` exactly where the mask is set, in every draw; unknown entries of ``known`` are
+        never read into the result.  x_T and the noise are those of a call without it.  Needs the whole chain (no
+        ``steps`` < T).  The mask is packed into row words per call and both are copied into buffers of the graph cache
+        entry, so calls with other values or masks replay the same graph."""
         _check_schedule(self.T, steps, ddim_steps, eta)
         check_guidance_scale(guidance_scale)
         check_num_samples(num_samples)
+        words = None
+        if check_known(known, known_mask, B, None, self.T, steps, self.device):
+            F = model.engine().F
+            if known.shape[1] != F:
+                raise ValueError(f"known must have the model's F={F} frames per window, got {tuple(known.shape)}")
+            known = known.reshape(B * F, 30)
+            words = known_mask_words(known_mask.to(self.device), B * F)
+        return self._sample(model, B, x_T=x_T, noise=noise, steps=steps, seed=seed, use_graph=use_graph, ddim_steps=ddim_steps,
+                            eta=eta, guidance_scale=guidance_scale, num_samples=num_samples, known=known, words=words)
+
+    def _sample(self, model, B: int, *, x_T, noise, steps, seed, use_graph, ddim_steps, eta, guidance_scale, num_samples,
+                known: Optional[torch.Tensor], words: Optional[torch.Tensor]) -> torch.Tensor:
+        """``sample`` after its checks: ``known`` fp32 (rows, 30) and ``words`` int32 (rows,) (``known_mask_words``) of the
+        caller's B windows, or None; a call on B*K windows repeats them K times."""
         if num_samples is not None:
             eng = model.engine()
             src = eng.xc(B, False)
@@ -160,10 +221,12 @@ class GaussianDiffusion:
             M = src.shape[0]
             for k in range(num_samples):
                 dst[k * M:(k + 1) * M].copy_(src)
-            x0 = self.sample(model, B * num_samples, x_T=x_T, noise=noise, steps=steps, seed=seed, use_graph=use_graph,
-                             ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale)
+            x0 = self._sample(model, B * num_samples, x_T=x_T, noise=noise, steps=steps, seed=seed, use_graph=use_graph,
+                              ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale, num_samples=None, known=known,
+                              words=words)
             return x0.view(num_samples, B, eng.F, 30)
         guided = guidance_scale != 1.0
+        inpaint = known is not None
         eng = model.engine()
         F, M = eng.F, B * eng.F
         xc = eng.xc(B, False)
@@ -182,8 +245,11 @@ class GaussianDiffusion:
             ts = tab["ts"].tolist()
             coef_x0, coef_xt, sigma, succ = tab["coef_x0"], tab["coef_xt"], tab["sigma"], tab["succ"]
         # the captured launches read the schedule's tables through baked-in pointers, so each schedule has its own graph;
-        # the guidance scale is a baked launch argument
+        # the guidance scale is a baked launch argument; inpainting reads the known values and mask words from the entry's
+        # buffers, refilled per call
         key = (id(model), B, sched) if not guided else (id(model), B, sched, float(guidance_scale))
+        if inpaint:
+            key += ("inpaint",)
         st = self._graphs.get(key)
         if st is None or st["model"] is not model:
             # the entry holds the model (its id() cannot be recycled while cached), the schedule's tables and, below, the
@@ -192,8 +258,18 @@ class GaussianDiffusion:
                       t_a=torch.zeros(1, dtype=torch.int32, device=self.device),
                       t_b=torch.zeros(1, dtype=torch.int32, device=self.device), graph=None, seed=None, model=model, table=None,
                       table_key=None, sched_tables=(coef_x0, coef_xt, sigma, succ))
+            if inpaint:
+                st["known"] = torch.empty(M, 30, dtype=torch.float32, device=self.device)
+                st["words"] = torch.empty(M, dtype=torch.int32, device=self.device)
             self._graphs[key] = st
         x, t_a, t_b = st["x"], st["t_a"], st["t_b"]
+        kn = {}
+        if inpaint:
+            # K = M / rows blocks of the caller's rows (num_samples), like the conditions
+            reps = M // known.shape[0]
+            st["known"].view(reps, -1, 30).copy_(known.unsqueeze(0).expand(reps, -1, -1))
+            st["words"].view(reps, -1).copy_(words.unsqueeze(0).expand(reps, -1))
+            kn = dict(known=st["known"], known_mask=st["words"])
         # the halves of the guided buffer receive the same x_T (the same Philox seed and offset, or the same rows)
         for rows in ((xc,) if not guided else (xc2[:M], xc2[M:])):
             if x_T is None:
@@ -212,11 +288,11 @@ class GaussianDiffusion:
             if not guided:
                 x0_hat = eng.forward(B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
                 ops.posterior_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, x_prev=x, xprev_bf16=xc,
-                                   bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ)
+                                   bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ, **kn)
                 return
             x0_hat = eng.forward(2 * B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
             ops.guided_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, guidance_scale, x_prev=x, xprev_bf16=xc2,
-                            bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ)
+                            bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ, **kn)
 
         # DDPM runs an odd step count eagerly, as it always has; DDIM replays the graph for the even part of any S >= 2
         if noise is not None or not use_graph or (n_steps % 2 if sched is None else n_steps < 2):
@@ -256,7 +332,8 @@ class GaussianDiffusion:
     @torch.no_grad()
     def sample_windows(self, model, cond: torch.Tensor, *, batch: int = 512, steps: Optional[int] = None, seed: int = 0,
                        rank: Optional[int] = None, world: Optional[int] = None, ddim_steps: Optional[int] = None,
-                       eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None):
+                       eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None,
+                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None):
         """Reverse-sample GRF / CoP / torque / wrench trajectories for ``cond``: (N, F, C_in) fp32 packed kinematics of N
         windows (model concat order, FeedForward...py:97-108) in HOST memory (pinned for asynchronous copies).
 
@@ -266,11 +343,14 @@ class GaussianDiffusion:
         ``(range, x0)`` with x0 a pinned host tensor (len(range), F, 30).  No collective; per-rank noise stream = seed + rank.
         The copies of batch i+1 / i-1 overlap the sampling of batch i (separate streams).  ``ddim_steps`` / ``eta`` select
         DDIM sampling and ``guidance_scale`` classifier-free guidance as in ``sample``.  ``num_samples`` K: K draws per window
-        (``sample(..., num_samples=K)`` per batch, ``batch`` still counts windows) and x0 is (len(range), K, F, 30)."""
+        (``sample(..., num_samples=K)`` per batch, ``batch`` still counts windows) and x0 is (len(range), K, F, 30).
+        ``known`` (fp32 (N, F, 30)) with ``known_mask`` (bool (N, F, 30) or (30,)), host tensors: inpainting as in ``sample``;
+        the mask is packed into row words once, and each batch's values and words travel with its conditions."""
         from . import parallel
         _check_schedule(self.T, steps, ddim_steps, eta)
         check_guidance_scale(guidance_scale)
         check_num_samples(num_samples)
+        inpaint = check_known(known, known_mask, cond.shape[0], None, self.T, steps)
         r, w = parallel.world()
         rank = r if rank is None else rank
         world = w if world is None else world
@@ -278,6 +358,12 @@ class GaussianDiffusion:
         F, C = eng.F, eng.c_in
         N = cond.shape[0]
         assert tuple(cond.shape[1:]) == (F, C) and not cond.is_cuda, "cond: host tensor (N, F, C_in)"
+        if inpaint:
+            check_known(known, known_mask, N, F, self.T, steps)
+            if known.is_cuda or known_mask.is_cuda:
+                raise ValueError("sample_windows takes known and known_mask in host memory")
+            known = known.reshape(N * F, 30)
+            words = known_mask_words(known_mask, N * F).contiguous().pin_memory()
         mine = parallel.contiguous_shard(N, rank, world)
         shape = (len(mine), F, 30) if num_samples is None else (len(mine), num_samples, F, 30)
         out = torch.empty(shape, dtype=torch.float32).pin_memory()
@@ -285,6 +371,9 @@ class GaussianDiffusion:
         main = torch.cuda.current_stream(dev)
         up, down = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
         stage = [torch.empty(batch * F, C, dtype=torch.float32, device=dev) for _ in range(2)]
+        if inpaint:
+            stage_y = [torch.empty(batch * F, 30, dtype=torch.float32, device=dev) for _ in range(2)]
+            stage_w = [torch.empty(batch * F, dtype=torch.int32, device=dev) for _ in range(2)]
         uploaded = [torch.cuda.Event() for _ in range(2)]
         packed = [torch.cuda.Event() for _ in range(2)]
         starts = list(range(mine.start, mine.stop, batch))
@@ -294,9 +383,14 @@ class GaussianDiffusion:
             with torch.cuda.stream(up):
                 up.wait_event(packed[i & 1])
                 stage[i & 1][:(b - a) * F].copy_(cond[a:b].reshape(-1, C), non_blocking=True)
+                if inpaint:
+                    up.wait_event(sampled[i & 1])             # batch i - 2 has read its known values and words
+                    stage_y[i & 1][:(b - a) * F].copy_(known[a * F:b * F], non_blocking=True)
+                    stage_w[i & 1][:(b - a) * F].copy_(words[a * F:b * F], non_blocking=True)
                 uploaded[i & 1].record(up)
 
-        for e in packed:
+        sampled = [torch.cuda.Event() for _ in range(2)]
+        for e in packed + sampled:
             e.record(main)
         if starts:
             upload(0)
@@ -310,8 +404,11 @@ class GaussianDiffusion:
             packed[i & 1].record(main)
             if i + 1 < len(starts):
                 upload(i + 1)
-            x0 = self.sample(model, nb, steps=steps, seed=seed + rank + 7919 * i, ddim_steps=ddim_steps, eta=eta,
-                             guidance_scale=guidance_scale, num_samples=num_samples)
+            kn = dict(known=stage_y[i & 1][:nb * F], words=stage_w[i & 1][:nb * F]) if inpaint else dict(known=None, words=None)
+            x0 = self._sample(model, nb, x_T=None, noise=None, steps=steps, seed=seed + rank + 7919 * i, use_graph=True,
+                              ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale, num_samples=num_samples, **kn)
+            if inpaint:
+                sampled[i & 1].record(main)
             if num_samples is not None:
                 x0 = x0.transpose(0, 1)                       # (nb, K, F, 30): window-major for the caller
             ready = torch.cuda.Event()

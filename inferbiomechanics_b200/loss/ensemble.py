@@ -81,12 +81,13 @@ class EnsembleScorer:
             out[q] = ensemble_metrics(acc[:, a:b].sum(axis=1), self.K)
         return out
 
-    def print_report(self, args=None, log_to_wandb: bool = False, summary: Optional[Dict] = None) -> None:
+    def print_report(self, args=None, log_to_wandb: bool = False, summary: Optional[Dict] = None, given=()) -> None:
+        """``given``: quantities the sampler was given as known values (inpainting), marked "(given)"."""
         s = self.summary() if summary is None else summary
         print(f'\tEnsemble of {self.K} samples (fair CRPS, ensemble-mean RMSE, spread, spread-skill ratio, mean pairwise distance):')
         for q, (_, unit) in ENSEMBLE_GROUPS.items():
             v = s[q]
-            print(f'\t{q}: CRPS {v["crps"]} | RMSE {v["rmse"]} | spread {v["spread"]} | spread/skill {v["spread_skill"]} | '
+            print(f'\t{q}{" (given)" if q in given else ""}: CRPS {v["crps"]} | RMSE {v["rmse"]} | spread {v["spread"]} | spread/skill {v["spread_skill"]} | '
                   f'pair dist {v["pair_dist"]} {unit} | {v["count"]} elements')
         if log_to_wandb:
             import wandb

@@ -281,11 +281,28 @@ def q_sample(x0, eps, t, sqrt_abar, sqrt_1m_abar, xt_f32=None, xt_bf16=None, bf1
          seed, offset, _p(eps_out), stream_ptr())
 
 
+def _check_known(known, known_mask, M):
+    """Validates the inpainting inputs of ``posterior_step`` / ``guided_step``; True when both are given."""
+    if known is None and known_mask is None:
+        return False
+    if known is None or known_mask is None:
+        raise ValueError("known and known_mask go together: give both or neither")
+    for name, t, dt, shape in (("known", known, torch.float32, (M, 30)), ("known_mask", known_mask, torch.int32, (M,))):
+        if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != dt or not t.is_contiguous() or tuple(t.shape) != shape:
+            raise ValueError(f"{name} must be a contiguous {dt} CUDA tensor of shape {shape}")
+    return True
+
+
 def posterior_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev=None, xprev_bf16=None, bf16_ld=0,
-                   seed=0, offset=0, t_next=None, t_succ=None):
+                   seed=0, offset=0, t_next=None, t_succ=None, known=None, known_mask=None):
     """t_succ (device int32 [T]): the step of a respaced (DDIM) sequence, t_next receives t_succ[t]; None ⇒ the DDPM
-    posterior step, t_next receives t-1."""
-    if t_succ is None:
+    posterior step, t_next receives t-1.  ``known`` (fp32 [M, 30]) with ``known_mask`` (int32 [M], bit c = channel c is known):
+    the known entries replace the prediction before the update (``ibm_ddpm_inpaint_step``, inpainting)."""
+    if _check_known(known, known_mask, M):
+        call("ibm_ddpm_inpaint_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
+             _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), 1.0, 0, _p(known), _p(known_mask),
+             stream_ptr())
+    elif t_succ is None:
         call("ibm_ddpm_posterior_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
              _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), stream_ptr())
     else:
@@ -294,11 +311,17 @@ def posterior_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_p
 
 
 def guided_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, guidance_scale, x_prev=None, xprev_bf16=None,
-                bf16_ld=0, seed=0, offset=0, t_next=None, t_succ=None):
+                bf16_ld=0, seed=0, offset=0, t_next=None, t_succ=None, known=None, known_mask=None):
     """``posterior_step`` on a classifier-free guided prediction: x0_hat holds 2M rows, conditional then unconditional,
-    combined in fp32 as u + guidance_scale (c - u); xprev_bf16 receives the bf16 rows at m and at M + m."""
-    call("ibm_ddpm_guided_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
-         _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), float(guidance_scale), stream_ptr())
+    combined in fp32 as u + guidance_scale (c - u); xprev_bf16 receives the bf16 rows at m and at M + m.  ``known`` /
+    ``known_mask`` as in ``posterior_step``, applied to the guided prediction."""
+    if _check_known(known, known_mask, M):
+        call("ibm_ddpm_inpaint_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
+             _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), float(guidance_scale), 1, _p(known),
+             _p(known_mask), stream_ptr())
+    else:
+        call("ibm_ddpm_guided_step", _p(x0_hat), x0_ld, _p(x_t), _p(z), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(sigma), M,
+             _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), float(guidance_scale), stream_ptr())
 
 
 def cond_dropout(xc, B, F, col0, ncols, p, seed, offset, keep_out=None):
