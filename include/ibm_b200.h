@@ -385,14 +385,17 @@ int ibm_layernorm_bwd(const void* dy, const void* s, int64_t ld, const float* ga
  * q,k,v,o: bf16 matrices with one row per (window, frame) (n_win*T rows); head h occupies columns
  * [h*hd_qk, (h+1)*hd_qk) of q and k and [h*hd_v, (h+1)*hd_v) of v and o.  For a fused QKV
  * projection pass q = qkv, k = qkv + kv_off, v = qkv + 2*kv_off with ldq = ldk = ldv.
- * Supported (hd_qk, hd_v): (64,64) (48,48) (32,32) and (112,8) — the latter is SimpleAttention
- * (TransformerBaseline.py:51-70: scale = 1, d = 108 padded to 112, value dim 3 padded to 8).
- * T <= 256 (whole K and V of a head live in shared memory). */
+ * Supported (hd_qk, hd_v): (64,64) (48,48) (32,32) and ({64,80,96,112,128},8) — the value-width-8 pairs
+ * serve SimpleAttention (TransformerBaseline.py:51-70: scale = 1, d = 108 padded to 112, value dim 3
+ * padded to 8).  T <= 256 (whole K and V of a head live in shared memory).  scale must be finite and
+ * > 0 (the kernels take the row maximum of the raw scores); q, k, v 16-byte aligned with leading
+ * dimensions that are multiples of 8; o 4-byte aligned with an even ldo.  Anything else is IBM_E_ARG. */
 int ibm_attention_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
                       void* o, int64_t ldo, int64_t n_win, int32_t T, int32_t H, int32_t hd_qk,
                       int32_t hd_v, float scale, void* stream);
 /* dqkv (same layout as qkv: q | k | v blocks kv_off columns apart) from d_o; probabilities are
- * recomputed on chip.  T <= 64, head_dim in {32,48,64}.  dbias_qkv (may be NULL): fp32
+ * recomputed on chip.  T <= 64, head_dim in {32,48,64}, scale finite and > 0; qkv, d_o, dqkv 16-byte
+ * aligned, ld_qkv, ld_o, kv_off multiples of 8.  dbias_qkv (may be NULL): fp32
  * [2*kv_off + H*head_dim] vector that the column sums of dqkv are ADDED to — the gradient of
  * nn.MultiheadAttention.in_proj_bias (TransformerBaseline.py:12) without a second pass over dqkv. */
 int ibm_attention_bwd(const void* qkv, int64_t ld_qkv, int64_t kv_off, const void* d_o, int64_t ld_o,
@@ -405,7 +408,9 @@ int ibm_attention_bwd(const void* qkv, int64_t ld_qkv, int64_t kv_off, const voi
  * (o = the forward output); dq,dk,dv: bf16 outputs with their own leading dimensions (head h at columns h*hd).
  * Probabilities are recomputed on chip.  dbias_q/k/v (each may be NULL): fp32 [H*hd] vectors the column sums of
  * dq/dk/dv are ADDED to (in_proj_bias / query_linear.bias / key_linear.bias gradients).
- * Supported: (64,64) (48,48) (32,32) with dv, (112,8) without. */
+ * Supported: (64,64) (48,48) (32,32) with dv, ({64,80,96,112,128},8) without.  scale must be finite and > 0;
+ * q, k, v, d_o 16-byte aligned with leading dimensions that are multiples of 8; o, dq, dk, dv (bf16 pairs)
+ * 4-byte aligned with even leading dimensions.  Anything else is IBM_E_ARG. */
 int ibm_attention_bwd_long(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
                            const void* o, int64_t ldo, const void* d_o, int64_t ld_do, void* dq, int64_t lddq,
                            void* dk, int64_t lddk, void* dv, int64_t lddv, int64_t n_win, int32_t T, int32_t H,

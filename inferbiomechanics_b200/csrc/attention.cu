@@ -804,6 +804,8 @@ extern "C" int ibm_attention_fwd(const void* q, int64_t ldq, const void* k, int6
   IBM_CHECK_ARG(T <= 256, "attention_fwd: T=%d > 256 unsupported (whole sequence must fit in shared memory)", T);
   IBM_CHECK_ARG(ldq % 8 == 0 && ldk % 8 == 0 && ldv % 8 == 0 && ldo % 2 == 0 && aligned16(q) && aligned16(k) && aligned16(v),
                 "attention_fwd: leading dimensions must be multiples of 8 and pointers 16-byte aligned");
+  IBM_CHECK_ARG(aligned4(o), "attention_fwd: o must be 4-byte aligned (outputs are stored as bf16 pairs)");
+  IBM_CHECK_ARG(attn_scale_ok(scale), "attention_fwd: scale %g unsupported; it must be finite and > 0", scale);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   // short windows, 64-wide heads (the denoiser): a tcgen05 forward kernel exists (attention_tc.cu, same construction as the
   // backward) and is parity-tested, but with half the work per window pair its per-pair latency chain leaves it at
@@ -870,6 +872,7 @@ extern "C" int ibm_attention_bwd(const void* qkv, int64_t ld_qkv, int64_t kv_off
   IBM_CHECK_ARG(T <= 64, "attention_bwd: T=%d > 64 unsupported", T);
   IBM_CHECK_ARG(ld_qkv % 8 == 0 && ld_o % 8 == 0 && kv_off % 8 == 0 && aligned16(qkv) && aligned16(d_o) && aligned16(dqkv),
                 "attention_bwd: leading dimensions must be multiples of 8 and pointers 16-byte aligned");
+  IBM_CHECK_ARG(attn_scale_ok(scale), "attention_bwd: scale %g unsupported; it must be finite and > 0", scale);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   {
     // tcgen05 kernel for the denoiser's heads (head_dim 64); IBM_ATTN_BWD=mma keeps the mma.sync kernel (A/B measurements)

@@ -390,6 +390,9 @@ extern "C" int ibm_attention_bwd_long(const void* q, int64_t ldq, const void* k,
   IBM_CHECK_ARG(ldq % 8 == 0 && ldk % 8 == 0 && ldv % 8 == 0 && ld_do % 8 == 0 && ldo % 2 == 0 && lddq % 2 == 0 && lddk % 2 == 0 &&
                     (dv == nullptr || lddv % 2 == 0) && aligned16(q) && aligned16(k) && aligned16(v) && aligned16(d_o),
                 "attention_bwd_long: q/k/v/d_o need leading dimensions that are multiples of 8 and 16-byte aligned pointers");
+  IBM_CHECK_ARG(aligned4(o) && aligned4(dq) && aligned4(dk) && (dv == nullptr || aligned4(dv)),
+                "attention_bwd_long: o, dq, dk and dv must be 4-byte aligned (they are read and stored as bf16 pairs)");
+  IBM_CHECK_ARG(attn_scale_ok(scale), "attention_bwd_long: scale %g unsupported; it must be finite and > 0", scale);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
 #define IBM_BWD_LONG(HQV, HVV, DV) \
   return attn::launch_bwd_long<HQV, HVV, DV>(q, ldq, k, ldk, v, ldv, o, ldo, d_o, ld_do, dq, lddq, dk, lddk, dv, lddv, n_win, T, H, scale, \

@@ -45,6 +45,9 @@ int next_walk_reverse(int64_t bytes_streamed);
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+static inline bool aligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3) == 0; }
+// a softmax scale the attention kernels handle: they take the row maximum of the raw scores and scale afterwards
+static inline bool attn_scale_ok(float s) { return s > 0.f && s < INFINITY; }
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
