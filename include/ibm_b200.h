@@ -224,6 +224,22 @@ int ibm_ddpm_inpaint_step(const float* x0_hat, int64_t x0_ld, const float* x_t, 
                           const int32_t* t_succ, float guidance_scale, int32_t guided, const float* known,
                           const int32_t* known_mask, void* stream);
 
+/* Builder-owned (DESIGN.md D-1; NOT in the reference): one step of the second-order multistep sampler DPM-Solver++(2M)
+ * (Lu et al. 2022) from t = *t_dev to p = t_succ[t], on the tables of diffusion.dpm_schedule:
+ *   x_p = coef_x0[t] x0_hat + coef_prev[t] x0_prev + coef_xt[t] x_t      (no noise)
+ * x0_hat is the prediction after the guided combination (guided != 0: 2M rows as in ibm_ddpm_guided_step) and the known-entry
+ * select (known / known_mask as in ibm_ddpm_inpaint_step, both or neither).  x0_prev: fp32 [M, 30] contiguous, 8-byte aligned,
+ * the previous step's prediction; it is read only when coef_prev[t] != 0 (never on the first step, so it may hold anything
+ * there) and receives this step's x0_hat in place.  x_t / x_prev / xprev_bf16 / t_next_dev as in ibm_ddpm_respaced_step
+ * (x_prev may be x_t).  Refused (IBM_E_ARG, nothing launched): a null x0_hat, x_t, t_dev, coefficient table, t_succ or
+ * x0_prev; x0_prev misaligned or equal to x_prev, x_t or x0_hat; known without known_mask or the reverse; known misaligned;
+ * the shapes and leading dimensions the other step entries refuse; no output; guidance_scale not finite and >= 0. */
+int ibm_ddpm_multistep_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const int32_t* t_dev,
+                            const float* coef_x0, const float* coef_xt, const float* coef_prev,
+                            const int32_t* t_succ, int64_t M, float* x0_prev, float* x_prev, void* xprev_bf16,
+                            int64_t bf16_ld, int32_t* t_next_dev, float guidance_scale, int32_t guided,
+                            const float* known, const int32_t* known_mask, void* stream);
+
 /* Per-window condition dropout for classifier-free guidance training.  xc: bf16 [B*F, ld] (window b
  * owns rows b*F .. b*F+F-1).  Window b is dropped iff word 0 of Philox4x32-10 draw b at (seed, offset)
  * is below uint32(p * 2^32) (the keep rule of the dropout kernels); p >= 1 drops every window without

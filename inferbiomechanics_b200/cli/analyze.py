@@ -6,7 +6,8 @@ independent, so here each rank takes a CONTIGUOUS range of windows in large equa
 collective during the pass), keeps the per-batch fp32[40] results on the device and merges them once at the end —
 equal batch sizes keep the reference's mean-of-batch-means aggregate (RegressionLossEvaluator.py:383-387) exact.
 Per-window plots (matplotlib) and the names CSV are outside the hot path.  ``--model-type diffusion`` runs the
-reverse sampler per batch (``--sampler ddpm``: the 1000-step chain; ``ddim``: ``--sampling-steps`` respaced steps) and
+reverse sampler per batch (``--sampler ddpm``: the 1000-step chain; ``ddim``: ``--sampling-steps`` respaced steps;
+``dpmpp2m``: ``--sampling-steps`` steps of the second-order multistep DPM-Solver++(2M) on log-SNR-spaced timesteps) and
 scores the sampled trajectories with the same evaluator; ``--guidance-scale`` samples it with classifier-free guidance, which
 needs a checkpoint trained with ``train --cond-drop-prob``.  ``--num-samples K`` (K >= 2) draws K samples per window: the
 evaluator scores their mean and an ``EnsembleScorer`` block (CRPS, spread, spread-skill ratio, pairwise distance) follows
@@ -65,12 +66,15 @@ class AnalyzeCommand(AbstractCommand):
         sp.add_argument('--batch-size', type=int, default=4096, help='Windows per launch (the reference analyses one at a time).')
         sp.add_argument('--sampling-steps', type=int, default=1000,
                         help='Reverse-diffusion steps for --model-type diffusion.  --sampler ddpm: the first N steps of the '
-                             '1000-step chain (N < 1000 truncates it and scores a partially denoised sample); --sampler ddim: '
-                             'the number S of respaced steps (1..1000).')
-        sp.add_argument('--sampler', type=str, default='ddpm', choices=['ddpm', 'ddim'],
-                        help='Reverse sampler for --model-type diffusion: the ancestral DDPM chain or few-step DDIM.')
+                             '1000-step chain (N < 1000 truncates it and scores a partially denoised sample); --sampler ddim '
+                             'and dpmpp2m: the number S of steps (1..1000).')
+        sp.add_argument('--sampler', type=str, default='ddpm', choices=['ddpm', 'ddim', 'dpmpp2m'],
+                        help='Reverse sampler for --model-type diffusion: the ancestral DDPM chain, few-step DDIM, or the '
+                             'second-order multistep DPM-Solver++(2M) (deterministic given x_T, one forward per step like '
+                             'DDIM, more accurate at the same S).')
         sp.add_argument('--eta', type=float, default=0.0,
-                        help='DDIM noise scale in [0, 1] (0: deterministic given x_T; 1: respaced ancestral sampling).')
+                        help='DDIM noise scale in [0, 1] (0: deterministic given x_T; 1: respaced ancestral sampling); '
+                             '--sampler ddim only.')
         sp.add_argument('--ema', action='store_true', default=False,
                         help="Evaluate the checkpoint's EMA weights (ema_state_dict, written by train --ema-decay) instead of "
                              "the trained ones.")
@@ -90,7 +94,7 @@ class AnalyzeCommand(AbstractCommand):
     def run(self, args: argparse.Namespace):
         if 'command' in args and args.command != 'analyze':
             return False
-        if args.sampler == 'ddpm' and args.eta != 0.0:
+        if args.sampler != 'ddim' and args.eta != 0.0:
             raise ValueError("--eta applies to --sampler ddim only")
         model_type: str = args.model_type
         checkpoint_dir: str = os.path.join(os.path.abspath(args.checkpoint_dir), model_type)
@@ -146,6 +150,9 @@ class AnalyzeCommand(AbstractCommand):
                         if args.sampler == 'ddim':
                             sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, ddim_steps=args.sampling_steps,
                                              eta=args.eta, guidance_scale=guidance, **ens)
+                        elif args.sampler == 'dpmpp2m':
+                            sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, dpm_steps=args.sampling_steps,
+                                             guidance_scale=guidance, **ens)
                         else:
                             sample_and_score(diffusion, model, store, idx, ev, args, 1234 + rank, steps=args.sampling_steps,
                                              guidance_scale=guidance, **ens)

@@ -70,10 +70,10 @@ def known_quantity_mask(quantities) -> torch.Tensor:
 
 def sample_and_score(diffusion, model, store: WindowStore, idx: torch.Tensor, ev: RegressionLossEvaluator, args, seed: int,
                      *, steps=None, ddim_steps=None, eta: float = 0.0, guidance_scale: float = 1.0, num_samples: int = 1,
-                     scorer=None, known_quantities=()) -> None:
+                     scorer=None, known_quantities=(), dpm_steps=None) -> None:
     """Reverse-sample the denoiser's trajectories for windows ``idx`` of ``store`` and score them with ``ev`` against the
     store's labels: the condition is the packed kinematics in the engine's concat buffer, x_T ~ Philox(``seed``), and
-    ``steps`` / ``ddim_steps`` / ``eta`` select the sampler and ``guidance_scale`` the classifier-free guidance as in
+    ``steps`` / ``ddim_steps`` / ``eta`` / ``dpm_steps`` select the sampler and ``guidance_scale`` the classifier-free guidance as in
     ``GaussianDiffusion.sample``.  ``num_samples`` K >= 2 draws K samples per window: ``scorer`` (an ``EnsembleScorer`` for
     K draws) accumulates their probabilistic scores and ``ev`` scores the ensemble mean.  ``known_quantities`` (names of
     ``ENSEMBLE_GROUPS``): the store's labels of those quantities are given to the sampler as known values (inpainting), so
@@ -88,12 +88,12 @@ def sample_and_score(diffusion, model, store: WindowStore, idx: torch.Tensor, ev
         if scorer is None or scorer.K != num_samples:
             raise ValueError(f"num_samples={num_samples} needs an EnsembleScorer for {num_samples} draws")
         draws = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
-                                 guidance_scale=guidance_scale, num_samples=num_samples, **given)
+                                 guidance_scale=guidance_scale, num_samples=num_samples, dpm_steps=dpm_steps, **given)
         labels = store.labels(idx)
         ev({}, quantity_dict(scorer.score(draws, labels)), quantity_dict(labels), [], [], args)
         return
     x0 = diffusion.sample(model, idx.numel(), steps=steps, seed=seed, ddim_steps=ddim_steps, eta=eta,
-                          guidance_scale=guidance_scale, **given)
+                          guidance_scale=guidance_scale, dpm_steps=dpm_steps, **given)
     if store.Fo == 1:                     # --output-data-format last_frame: labels hold the last frame only
         x0 = x0[:, -1:]
     ev({}, quantity_dict(x0), label_dict(store, idx), [], [], args)

@@ -69,8 +69,11 @@ q_sample_kernel(const float* __restrict__ x0, const float* __restrict__ eps, con
 // halves of the concat buffer.  gscale follows the parameters of the unguided instantiations so they keep their parameter
 // offsets.  kKnown (inpainting): after the guided combination, channel c of row m takes known[m, c] instead of the prediction
 // where bit c of kmask[m] is set (bits 30-31 are ignored); a select, so a NaN in an unknown entry of `known` never reaches
-// the output.  known / kmask come after gscale for the same reason.
-template <bool kSucc, bool kGuided, bool kKnown>
+// the output.  known / kmask come after gscale for the same reason.  kMulti (DPM-Solver++(2M), always with kSucc): no noise
+// term; the update adds coef_prev[t] x0_prev (the previous step's prediction, read only when coef_prev[t] != 0, so the
+// uninitialised buffer of the first step is never read) and stores this step's prediction, after the guided combination and
+// the known-entry select, into x0_prev in place.  coef_prev / x0_prev come last for the same reason.
+template <bool kSucc, bool kGuided, bool kKnown, bool kMulti>
 __global__ void __launch_bounds__(kThreads)
 posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __restrict__ xt,
                  const float* __restrict__ z, const int32_t* __restrict__ t_dev, const float* __restrict__ c1t,
@@ -78,10 +81,11 @@ posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __
                  float* __restrict__ xprev, __nv_bfloat16* __restrict__ xp_bf16, long long bf16_ld,
                  uint64_t seed, uint64_t offset, int32_t* __restrict__ t_next,
                  const int32_t* __restrict__ t_succ, float gscale, const float* __restrict__ known,
-                 const int32_t* __restrict__ kmask) {
+                 const int32_t* __restrict__ kmask, const float* __restrict__ coef_prev, float* __restrict__ x0_prev) {
   const int tt = __ldg(t_dev);
   const float c1 = __ldg(c1t + tt), c2 = __ldg(c2t + tt);
-  const float s = tt > 0 ? __ldg(sig + tt) : 0.f;
+  const float s = !kMulti && tt > 0 ? __ldg(sig + tt) : 0.f;
+  const float cp = kMulti ? __ldg(coef_prev + tt) : 0.f;
   const long long npair = M * 15;
   const long long stride = (long long)gridDim.x * blockDim.x;
 #pragma unroll (kKnown ? 1 : 2)   // unrolled twice, the kKnown loop spills 8 bytes (CUDA 12.9)
@@ -102,17 +106,29 @@ posterior_kernel(const float* __restrict__ x0h, long long x0_ld, const float* __
       }
     }
     const float2 x = *reinterpret_cast<const float2*>(xt + 2 * p);
-    float2 n;
-    if (z) n = *reinterpret_cast<const float2*>(z + 2 * p);
-    else {
-      // counter offset includes the step so a CUDA-graph replay (frozen arguments) still draws fresh noise
-      float4 z4 = philox_normal4(seed, offset + (uint64_t)tt, (uint64_t)(p >> 1));
-      n = (p & 1) ? make_float2(z4.z, z4.w) : make_float2(z4.x, z4.y);
-    }
     float2 r;
-    r.x = fmaf(c1, a.x, c2 * x.x);
-    r.y = fmaf(c1, a.y, c2 * x.y);
-    if (tt > 0) { r.x = fmaf(s, n.x, r.x); r.y = fmaf(s, n.y, r.y); }
+    if (kMulti) {
+      r.x = fmaf(c1, a.x, c2 * x.x);
+      r.y = fmaf(c1, a.y, c2 * x.y);
+      float2* const q = reinterpret_cast<float2*>(x0_prev + 2 * p);
+      if (cp != 0.f) {                      // tt is uniform per launch, so is this branch
+        const float2 d = *q;
+        r.x = fmaf(cp, d.x, r.x);
+        r.y = fmaf(cp, d.y, r.y);
+      }
+      *q = a;
+    } else {
+      float2 n;
+      if (z) n = *reinterpret_cast<const float2*>(z + 2 * p);
+      else {
+        // counter offset includes the step so a CUDA-graph replay (frozen arguments) still draws fresh noise
+        float4 z4 = philox_normal4(seed, offset + (uint64_t)tt, (uint64_t)(p >> 1));
+        n = (p & 1) ? make_float2(z4.z, z4.w) : make_float2(z4.x, z4.y);
+      }
+      r.x = fmaf(c1, a.x, c2 * x.x);
+      r.y = fmaf(c1, a.y, c2 * x.y);
+      if (tt > 0) { r.x = fmaf(s, n.x, r.x); r.y = fmaf(s, n.y, r.y); }
+    }
     if (xprev) *reinterpret_cast<float2*>(xprev + 2 * p) = r;
     if (xp_bf16) {
       const uint32_t v = pack_bf16x2(r.x, r.y);
@@ -367,9 +383,9 @@ extern "C" int ibm_ddpm_posterior_step(const float* x0_hat, int64_t x0_ld, const
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "posterior_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "posterior_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "posterior_step: bf16 ld must be even");
-  posterior_kernel<false, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<false, false, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev, nullptr, 0.f, nullptr, nullptr);
+      seed, offset, t_next_dev, nullptr, 0.f, nullptr, nullptr, nullptr, nullptr);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }
@@ -385,9 +401,9 @@ extern "C" int ibm_ddpm_respaced_step(const float* x0_hat, int64_t x0_ld, const 
   IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "respaced_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
   IBM_CHECK_ARG(x_prev || xprev_bf16, "respaced_step: no output requested");
   IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "respaced_step: bf16 ld must be even");
-  posterior_kernel<true, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  posterior_kernel<true, false, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, x_prev, static_cast<__nv_bfloat16*>(xprev_bf16), bf16_ld,
-      seed, offset, t_next_dev, t_succ, 0.f, nullptr, nullptr);
+      seed, offset, t_next_dev, t_succ, 0.f, nullptr, nullptr, nullptr, nullptr);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }
@@ -408,13 +424,13 @@ extern "C" int ibm_ddpm_guided_step(const float* x0_hat, int64_t x0_ld, const fl
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   auto* xb = static_cast<__nv_bfloat16*>(xprev_bf16);
   if (t_succ)
-    posterior_kernel<true, true, false><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
+    posterior_kernel<true, true, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
                                                                         x_prev, xb, bf16_ld, seed, offset, t_next_dev, t_succ,
-                                                                        guidance_scale, nullptr, nullptr);
+                                                                        guidance_scale, nullptr, nullptr, nullptr, nullptr);
   else
-    posterior_kernel<false, true, false><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
+    posterior_kernel<false, true, false, false><<<ew_grid(M * 15 / 2), kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,
                                                                          x_prev, xb, bf16_ld, seed, offset, t_next_dev, nullptr,
-                                                                         guidance_scale, nullptr, nullptr);
+                                                                         guidance_scale, nullptr, nullptr, nullptr, nullptr);
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }
@@ -439,9 +455,9 @@ extern "C" int ibm_ddpm_inpaint_step(const float* x0_hat, int64_t x0_ld, const f
   auto* xb = static_cast<__nv_bfloat16*>(xprev_bf16);
   const int grid = ew_grid(M * 15 / 2);
 #define IBM_INPAINT_LAUNCH(SUCC, GUIDED)                                                                                       \
-  posterior_kernel<SUCC, GUIDED, true><<<grid, kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,     \
+  posterior_kernel<SUCC, GUIDED, true, false><<<grid, kThreads, 0, s>>>(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M,     \
                                                                  x_prev, xb, bf16_ld, seed, offset, t_next_dev, t_succ,         \
-                                                                 guidance_scale, known, known_mask)
+                                                                 guidance_scale, known, known_mask, nullptr, nullptr)
   if (t_succ) {
     if (guided) IBM_INPAINT_LAUNCH(true, true);
     else IBM_INPAINT_LAUNCH(true, false);
@@ -450,6 +466,44 @@ extern "C" int ibm_ddpm_inpaint_step(const float* x0_hat, int64_t x0_ld, const f
     else IBM_INPAINT_LAUNCH(false, false);
   }
 #undef IBM_INPAINT_LAUNCH
+  IBM_LAUNCH_CHECK();
+  return IBM_OK;
+}
+
+extern "C" int ibm_ddpm_multistep_step(const float* x0_hat, int64_t x0_ld, const float* x_t, const int32_t* t_dev,
+                                       const float* coef_x0, const float* coef_xt, const float* coef_prev,
+                                       const int32_t* t_succ, int64_t M, float* x0_prev, float* x_prev, void* xprev_bf16,
+                                       int64_t bf16_ld, int32_t* t_next_dev, float guidance_scale, int32_t guided,
+                                       const float* known, const int32_t* known_mask, void* stream) {
+  using namespace ibm;
+  IBM_CHECK_ARCH();
+  IBM_CHECK_ARG(x0_hat && x_t && t_dev && coef_x0 && coef_xt && coef_prev && t_succ && x0_prev, "multistep_step: null argument");
+  IBM_CHECK_ARG(reinterpret_cast<uintptr_t>(x0_prev) % 8 == 0, "multistep_step: x0_prev must be 8-byte aligned");
+  IBM_CHECK_ARG(x0_prev != x_prev && x0_prev != x_t && x0_prev != x0_hat,
+                "multistep_step: x0_prev must not be x_prev, x_t or x0_hat");
+  IBM_CHECK_ARG(!known == !known_mask, "multistep_step: known values and known mask go together");
+  IBM_CHECK_ARG(reinterpret_cast<uintptr_t>(known) % 8 == 0, "multistep_step: known values must be 8-byte aligned");
+  IBM_CHECK_ARG(M > 0 && x0_ld >= 30 && x0_ld % 2 == 0, "multistep_step: bad shape (M=%lld ld=%lld)", (long long)M, (long long)x0_ld);
+  IBM_CHECK_ARG(x_prev || xprev_bf16, "multistep_step: no output requested");
+  IBM_CHECK_ARG(!xprev_bf16 || (bf16_ld % 2 == 0 && bf16_ld >= 30), "multistep_step: bf16 ld must be even");
+  IBM_CHECK_ARG(guidance_scale >= 0.f && guidance_scale <= 3.402823466e38f, "multistep_step: guidance scale must be finite and >= 0, got %g",
+                (double)guidance_scale);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  auto* xb = static_cast<__nv_bfloat16*>(xprev_bf16);
+  const int grid = ew_grid(M * 15 / 2);
+#define IBM_MULTISTEP_LAUNCH(GUIDED, KNOWN)                                                                                    \
+  posterior_kernel<true, GUIDED, KNOWN, true><<<grid, kThreads, 0, s>>>(x0_hat, x0_ld, x_t, nullptr, t_dev, coef_x0, coef_xt,  \
+                                                                        nullptr, M, x_prev, xb, bf16_ld, 0, 0, t_next_dev,      \
+                                                                        t_succ, guidance_scale, known, known_mask, coef_prev,  \
+                                                                        x0_prev)
+  if (known) {
+    if (guided) IBM_MULTISTEP_LAUNCH(true, true);
+    else IBM_MULTISTEP_LAUNCH(false, true);
+  } else {
+    if (guided) IBM_MULTISTEP_LAUNCH(true, false);
+    else IBM_MULTISTEP_LAUNCH(false, false);
+  }
+#undef IBM_MULTISTEP_LAUNCH
   IBM_LAUNCH_CHECK();
   return IBM_OK;
 }

@@ -9,6 +9,11 @@ Few-step sampling (DDIM, Song et al. 2021) walks a respaced sequence ts = round(
 same kernel: each step from t to its successor p = succ[t] is linear in (x0_hat, x_t, z) with per-timestep tables
 (``ddim_schedule``); eta = 1 over all T steps is the DDPM chain above, bit for bit.
 
+DPM-Solver++(2M) (Lu et al. 2022) is the second-order multistep solver of the same probability-flow ODE as DDIM eta = 0, in
+its data-prediction form, so the x0-predicting denoiser is used as trained.  It walks log-SNR-spaced timesteps and applies
+DDIM's step to the extrapolated prediction (1 + 1/2r) x0_hat - (1/2r) x0_hat_prev, one forward per step, with a step kernel
+that keeps the previous prediction in an fp32 buffer (``dpm_schedule``).
+
 The reverse loop runs the denoiser forward + one fused posterior kernel per step; the timestep lives
 in device memory so two consecutive steps are captured once in a CUDA graph and replayed (sampling at
 512 windows/GPU is launch-bound otherwise).  Windows are independent: multi-GPU sampling shards them
@@ -20,7 +25,7 @@ step kernel combines x0_hat = u + s (c - u) before the same update; s = 0 is unc
 
 Inpainting (MDM's ``p_mean_variance`` for an x0-predicting model): given known values y and a known-mask, every step
 replaces the known entries of x0_hat (after the guided combination) by y before the unchanged update.  The last step of
-either sampler has coef_x0 = 1, coef_xt = 0 and no noise, so the sample equals y exactly wherever the mask is set.
+every sampler has coef_x0 = 1, coef_xt = 0 and no noise, so the sample equals y exactly wherever the mask is set.
 """
 from __future__ import annotations
 
@@ -48,21 +53,77 @@ def ddim_schedule(ddim_steps: int, eta: float = 0.0, num_timesteps: int = 1000, 
     posterior tables bit for bit (sigma at t >= 1; the step at t = 0 draws no noise in either)."""
     T = num_timesteps
     _check_schedule(T, None, ddim_steps, eta)
-    abar = np.cumprod(1.0 - np.linspace(beta_start, beta_end, T, dtype=np.float64))
+    abar = _abar(T, beta_start, beta_end)
     ts = np.round(np.linspace(T - 1, 0, ddim_steps)).astype(np.int64)
+    return _tabulate(T, ts, _ddim_steps(abar, ts, eta))
+
+
+def _abar(T: int, beta_start: float, beta_end: float) -> np.ndarray:
+    return np.cumprod(1.0 - np.linspace(beta_start, beta_end, T, dtype=np.float64))
+
+
+def _ddim_steps(abar: np.ndarray, ts: np.ndarray, eta: float) -> dict:
+    """fp64 coef_x0 / coef_xt / sigma [S] of the DDIM steps ts[i] -> ts[i+1] (the formulas of ``ddim_schedule``)."""
     succ = np.append(ts[1:], -1)
     a_t = abar[ts]
     a_p = np.where(succ >= 0, abar[np.maximum(succ, 0)], 1.0)
     sigma = eta * np.sqrt((1.0 - a_p) / (1.0 - a_t)) * np.sqrt(1.0 - a_t / a_p)
     c = np.sqrt(np.maximum(1.0 - a_p - sigma * sigma, 0.0))
-    tab = dict(coef_x0=np.sqrt(a_p) - c * np.sqrt(a_t) / np.sqrt(1.0 - a_t), coef_xt=c / np.sqrt(1.0 - a_t), sigma=sigma)
-    out = {k: np.zeros(T, dtype=np.float32) for k in tab}
-    for k, v in tab.items():
+    return dict(coef_x0=np.sqrt(a_p) - c * np.sqrt(a_t) / np.sqrt(1.0 - a_t), coef_xt=c / np.sqrt(1.0 - a_t), sigma=sigma)
+
+
+def _tabulate(T: int, ts: np.ndarray, steps: dict) -> dict:
+    """The per-step values ``steps`` as fp32 [T] tables indexed by timestep (0 off the sequence), ``succ`` and ``ts``."""
+    out = {k: np.zeros(T, dtype=np.float32) for k in steps}
+    for k, v in steps.items():
         out[k][ts] = v.astype(np.float32)
     out["succ"] = np.zeros(T, dtype=np.int32)
-    out["succ"][ts] = succ
+    out["succ"][ts] = np.append(ts[1:], -1)
     out["ts"] = ts
     return out
+
+
+def dpm_timesteps(S: int, abar: np.ndarray) -> np.ndarray:
+    """int64 [S]: the timesteps of S-step DPM-Solver++(2M) (DESIGN.md D-1), spaced uniformly in the log-SNR
+    lambda(t) = 1/2 ln(a_t / (1 - a_t)): the t nearest each of S equally spaced targets from lambda(T-1) to lambda(0) (the
+    smaller t on a tie), then made S distinct, strictly decreasing entries from T-1 to 0."""
+    T = len(abar)
+    if S == 1:
+        return np.array([T - 1], dtype=np.int64)
+    lam = 0.5 * np.log(abar / (1.0 - abar))
+    target = lam[T - 1] + (lam[0] - lam[T - 1]) * np.arange(S) / (S - 1)
+    u = np.abs(lam[None, :] - target[:, None]).argmin(axis=1).astype(np.int64)
+    u = np.minimum(u, T - 1 - np.arange(S))
+    u[-1] = 0
+    for i in range(S - 2, -1, -1):
+        u[i] = max(u[i], u[i + 1] + 1)
+    return u
+
+
+def dpm_schedule(dpm_steps: int, num_timesteps: int = 1000, beta_start: float = 1e-4, beta_end: float = 2e-2) -> dict:
+    """Host tables (numpy, no GPU) of S = ``dpm_steps``-step DPM-Solver++(2M) (Lu et al. 2022; DESIGN.md D-1) over the trained
+    schedule, on ``dpm_timesteps``.  The step from t = ts[i] to p = ts[i+1] (p = -1 after the last, abar[-1] := 1) is
+      x_p = coef_x0[t] x0_hat + coef_prev[t] x0_hat_prev + coef_xt[t] x_t
+    with base, coef_xt the DDIM eta = 0 coefficients of (t, p) (``ddim_schedule``'s formulas) and, for the interior steps
+    0 < i < S-1 with q = ts[i-1] and r = (lambda_t - lambda_q) / (lambda_p - lambda_t),
+      coef_x0 = base (1 + 1/(2r)),   coef_prev = -base/(2r);
+    the first and last steps are first order (coef_x0 = base, coef_prev = 0), so they are DDIM's steps bit for bit and the
+    last one returns x0_hat.  ``coef_x0``, ``coef_xt``, ``coef_prev`` (fp32 [T]) and ``succ`` (int32 [T], = p) are indexed by
+    timestep, 0 off the sequence; ``ts`` (int64 [S])."""
+    T = num_timesteps
+    _check_schedule(T, None, None, 0.0, dpm_steps)
+    abar = _abar(T, beta_start, beta_end)
+    ts = dpm_timesteps(dpm_steps, abar)
+    d = _ddim_steps(abar, ts, 0.0)
+    base = d["coef_x0"]
+    coef_x0, coef_prev = base.copy(), np.zeros(dpm_steps)
+    if dpm_steps > 2:
+        lam = 0.5 * np.log(abar[ts] / (1.0 - abar[ts]))
+        i = np.arange(1, dpm_steps - 1)
+        r = (lam[i] - lam[i - 1]) / (lam[i + 1] - lam[i])
+        coef_x0[i] = base[i] * (1.0 + 1.0 / (2.0 * r))
+        coef_prev[i] = -base[i] / (2.0 * r)
+    return _tabulate(T, ts, dict(coef_x0=coef_x0, coef_xt=d["coef_xt"], coef_prev=coef_prev))
 
 
 def check_guidance_scale(guidance_scale: float) -> None:
@@ -113,11 +174,16 @@ def _on(t: torch.Tensor, device) -> bool:
     return t.device.type == device.type and (device.index is None or t.device.index == device.index)
 
 
-def _check_schedule(T: int, steps: Optional[int], ddim_steps: Optional[int], eta: float) -> None:
+def _check_schedule(T: int, steps: Optional[int], ddim_steps: Optional[int], eta: float, dpm_steps: Optional[int] = None) -> None:
     if steps is not None and ddim_steps is not None:
         raise ValueError("give either steps (a truncated DDPM chain) or ddim_steps (a respaced DDIM sequence), not both")
+    if dpm_steps is not None and (steps is not None or ddim_steps is not None):
+        raise ValueError("give at most one of steps (a truncated DDPM chain), ddim_steps (DDIM) and dpm_steps "
+                         "(DPM-Solver++(2M))")
     if ddim_steps is not None and not 1 <= ddim_steps <= T:
         raise ValueError(f"ddim_steps must lie in [1, {T}], got {ddim_steps}")
+    if dpm_steps is not None and not (isinstance(dpm_steps, (int, np.integer)) and 1 <= dpm_steps <= T):
+        raise ValueError(f"dpm_steps must be an int in [1, {T}], got {dpm_steps!r}")
     if not 0.0 <= eta <= 1.0:
         raise ValueError(f"eta must lie in [0, 1], got {eta}")
     if eta != 0.0 and ddim_steps is None:
@@ -143,6 +209,7 @@ class GaussianDiffusion:
         self.device = torch.device(device)
         self._graphs = {}
         self._ddim = {}                 # (S, eta) -> device tables of ddim_schedule
+        self._dpm = {}                  # S -> device tables of dpm_schedule
         # reverse sampling: take the time MLP from the engine's per-timestep table (DenoiserEngine.temb_table) instead of
         # evaluating it every step; False re-runs it per step (parity check, tests/test_gpu_models.py)
         self.use_temb_table = True
@@ -168,20 +235,34 @@ class GaussianDiffusion:
             self._ddim[key] = tab
         return tab
 
+    def dpm_tables(self, dpm_steps: int) -> dict:
+        """``dpm_schedule`` of this schedule on the device (cached per S): coef_x0 / coef_xt / coef_prev fp32 [T], succ
+        int32 [T], ts (host numpy)."""
+        tab = self._dpm.get(dpm_steps)
+        if tab is None:
+            h = dpm_schedule(dpm_steps, self.T, self.beta_start, self.beta_end)
+            tab = {k: v if k == "ts" else torch.from_numpy(v).to(self.device) for k, v in h.items()}
+            self._dpm[dpm_steps] = tab
+        return tab
+
     # ---- reverse process -----------------------------------------------------------------------
     @torch.no_grad()
     def sample(self, model, B: int, *, x_T: Optional[torch.Tensor] = None, noise: Optional[Callable[[int], torch.Tensor]] = None,
                steps: Optional[int] = None, seed: int = 0, use_graph: bool = True, ddim_steps: Optional[int] = None,
                eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None,
-               known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+               known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None,
+               dpm_steps: Optional[int] = None) -> torch.Tensor:
         """Reverse-sample x_0 (B,F,30) for the kinematics already packed in model.engine().xc(B, False)
         (columns 30…).  ``noise(t)`` supplies z per step for parity tests; None ⇒ on-device Philox.
 
         ``ddim_steps=None``: the DDPM chain; ``steps`` < T runs only its first ``steps`` steps and returns x at timestep
         T - steps (a truncated chain, not a sample).  ``ddim_steps=S``: S-step DDIM with noise scale ``eta`` in [0, 1]
         (``ddim_schedule``); eta = 0 draws no noise after x_T.  ``noise(t)`` is called with each timestep walked.
+        ``dpm_steps=S``: the second-order multistep DPM-Solver++(2M) on S log-SNR-spaced timesteps (``dpm_schedule``), one
+        forward per step like DDIM; it draws no noise (``seed`` only selects x_T, and ``noise`` is refused) and keeps the
+        previous step's prediction in an fp32 buffer of the graph cache entry.  S in {1, 2} is DDIM-S at eta = 0 bit for bit.
 
-        ``guidance_scale`` s != 1: classifier-free guidance with either sampler.  The kinematics of xc(B) are copied into
+        ``guidance_scale`` s != 1: classifier-free guidance with any sampler.  The kinematics of xc(B) are copied into
         the first half of xc(2B) and the second half gets the null condition (zeros); x_T goes into both halves, each step
         runs the forward on 2B windows and the guided step kernel.  s = 1 runs the unguided loop, s = 0 samples
         unconditionally.  The result depends on s only through the prediction: x_T and the noise are those of s = 1.
@@ -197,7 +278,9 @@ class GaussianDiffusion:
         never read into the result.  x_T and the noise are those of a call without it.  Needs the whole chain (no
         ``steps`` < T).  The mask is packed into row words per call and both are copied into buffers of the graph cache
         entry, so calls with other values or masks replay the same graph."""
-        _check_schedule(self.T, steps, ddim_steps, eta)
+        _check_schedule(self.T, steps, ddim_steps, eta, dpm_steps)
+        if dpm_steps is not None and noise is not None:
+            raise ValueError("dpm_steps draws no noise: noise= applies to the DDPM and DDIM samplers")
         check_guidance_scale(guidance_scale)
         check_num_samples(num_samples)
         words = None
@@ -208,10 +291,11 @@ class GaussianDiffusion:
             known = known.reshape(B * F, 30)
             words = known_mask_words(known_mask.to(self.device), B * F)
         return self._sample(model, B, x_T=x_T, noise=noise, steps=steps, seed=seed, use_graph=use_graph, ddim_steps=ddim_steps,
-                            eta=eta, guidance_scale=guidance_scale, num_samples=num_samples, known=known, words=words)
+                            eta=eta, guidance_scale=guidance_scale, num_samples=num_samples, known=known, words=words,
+                            dpm_steps=dpm_steps)
 
     def _sample(self, model, B: int, *, x_T, noise, steps, seed, use_graph, ddim_steps, eta, guidance_scale, num_samples,
-                known: Optional[torch.Tensor], words: Optional[torch.Tensor]) -> torch.Tensor:
+                known: Optional[torch.Tensor], words: Optional[torch.Tensor], dpm_steps: Optional[int] = None) -> torch.Tensor:
         """``sample`` after its checks: ``known`` fp32 (rows, 30) and ``words`` int32 (rows,) (``known_mask_words``) of the
         caller's B windows, or None; a call on B*K windows repeats them K times."""
         if num_samples is not None:
@@ -223,7 +307,7 @@ class GaussianDiffusion:
                 dst[k * M:(k + 1) * M].copy_(src)
             x0 = self._sample(model, B * num_samples, x_T=x_T, noise=noise, steps=steps, seed=seed, use_graph=use_graph,
                               ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale, num_samples=None, known=known,
-                              words=words)
+                              words=words, dpm_steps=dpm_steps)
             return x0.view(num_samples, B, eng.F, 30)
         guided = guidance_scale != 1.0
         inpaint = known is not None
@@ -235,7 +319,13 @@ class GaussianDiffusion:
             xc2 = eng.xc(2 * B, False)
             xc2[:M].copy_(xc)
             ops.cond_dropout(xc2[M:], B, F, 30, eng.c_in, 1.0, 0, 0)
-        if ddim_steps is None:
+        coef_prev = None
+        if dpm_steps is not None:
+            sched = ("dpm", dpm_steps)
+            tab = self.dpm_tables(dpm_steps)
+            ts = tab["ts"].tolist()
+            coef_x0, coef_xt, sigma, succ, coef_prev = tab["coef_x0"], tab["coef_xt"], None, tab["succ"], tab["coef_prev"]
+        elif ddim_steps is None:
             sched = None
             ts = range(self.T - 1, self.T - 1 - (self.T if steps is None else steps), -1)
             coef_x0, coef_xt, sigma, succ = self.coef_x0, self.coef_xt, self.sigma, None
@@ -257,7 +347,10 @@ class GaussianDiffusion:
             st = dict(x=torch.empty(M, 30, dtype=torch.float32, device=self.device),
                       t_a=torch.zeros(1, dtype=torch.int32, device=self.device),
                       t_b=torch.zeros(1, dtype=torch.int32, device=self.device), graph=None, seed=None, model=model, table=None,
-                      table_key=None, sched_tables=(coef_x0, coef_xt, sigma, succ))
+                      table_key=None, sched_tables=(coef_x0, coef_xt, sigma, succ, coef_prev))
+            if coef_prev is not None:
+                # the previous step's prediction (after guidance and the known values); the first step does not read it
+                st["prev"] = torch.empty(M, 30, dtype=torch.float32, device=self.device)
             if inpaint:
                 st["known"] = torch.empty(M, 30, dtype=torch.float32, device=self.device)
                 st["words"] = torch.empty(M, dtype=torch.int32, device=self.device)
@@ -285,6 +378,12 @@ class GaussianDiffusion:
         t_a.fill_(self.T - 1)
 
         def step(t_in, t_out, z):
+            if coef_prev is not None:
+                x0_hat = eng.forward((2 if guided else 1) * B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
+                ops.multistep_step(x0_hat, 32, x, t_in, coef_x0, coef_xt, coef_prev, succ, M, st["prev"], x_prev=x,
+                                   xprev_bf16=xc2 if guided else xc, bf16_ld=eng.ld_in, t_next=t_out,
+                                   guidance_scale=guidance_scale if guided else None, **kn)
+                return
             if not guided:
                 x0_hat = eng.forward(B, F, False, t_scalar=t_in, t_count=self.T if self.use_temb_table else 0)
                 ops.posterior_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, x_prev=x, xprev_bf16=xc,
@@ -294,7 +393,7 @@ class GaussianDiffusion:
             ops.guided_step(x0_hat, 32, x, z, t_in, coef_x0, coef_xt, sigma, M, guidance_scale, x_prev=x, xprev_bf16=xc2,
                             bf16_ld=eng.ld_in, seed=seed, offset=0, t_next=t_out, t_succ=succ, **kn)
 
-        # DDPM runs an odd step count eagerly, as it always has; DDIM replays the graph for the even part of any S >= 2
+        # DDPM runs an odd step count eagerly, as it always has; DDIM and DPM replay the graph for the even part of any S >= 2
         if noise is not None or not use_graph or (n_steps % 2 if sched is None else n_steps < 2):
             cur, nxt = t_a, t_b
             for t in ts:
@@ -333,7 +432,8 @@ class GaussianDiffusion:
     def sample_windows(self, model, cond: torch.Tensor, *, batch: int = 512, steps: Optional[int] = None, seed: int = 0,
                        rank: Optional[int] = None, world: Optional[int] = None, ddim_steps: Optional[int] = None,
                        eta: float = 0.0, guidance_scale: float = 1.0, num_samples: Optional[int] = None,
-                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None):
+                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None,
+                       dpm_steps: Optional[int] = None):
         """Reverse-sample GRF / CoP / torque / wrench trajectories for ``cond``: (N, F, C_in) fp32 packed kinematics of N
         windows (model concat order, FeedForward...py:97-108) in HOST memory (pinned for asynchronous copies).
 
@@ -342,12 +442,12 @@ class GaussianDiffusion:
         ``steps`` (default: the full schedule) CUDA-graph-replayed denoise steps, D2H copy of the trajectories — and returns
         ``(range, x0)`` with x0 a pinned host tensor (len(range), F, 30).  No collective; per-rank noise stream = seed + rank.
         The copies of batch i+1 / i-1 overlap the sampling of batch i (separate streams).  ``ddim_steps`` / ``eta`` select
-        DDIM sampling and ``guidance_scale`` classifier-free guidance as in ``sample``.  ``num_samples`` K: K draws per window
+        DDIM sampling, ``dpm_steps`` DPM-Solver++(2M) and ``guidance_scale`` classifier-free guidance as in ``sample``.  ``num_samples`` K: K draws per window
         (``sample(..., num_samples=K)`` per batch, ``batch`` still counts windows) and x0 is (len(range), K, F, 30).
         ``known`` (fp32 (N, F, 30)) with ``known_mask`` (bool (N, F, 30) or (30,)), host tensors: inpainting as in ``sample``;
         the mask is packed into row words once, and each batch's values and words travel with its conditions."""
         from . import parallel
-        _check_schedule(self.T, steps, ddim_steps, eta)
+        _check_schedule(self.T, steps, ddim_steps, eta, dpm_steps)
         check_guidance_scale(guidance_scale)
         check_num_samples(num_samples)
         inpaint = check_known(known, known_mask, cond.shape[0], None, self.T, steps)
@@ -406,7 +506,8 @@ class GaussianDiffusion:
                 upload(i + 1)
             kn = dict(known=stage_y[i & 1][:nb * F], words=stage_w[i & 1][:nb * F]) if inpaint else dict(known=None, words=None)
             x0 = self._sample(model, nb, x_T=None, noise=None, steps=steps, seed=seed + rank + 7919 * i, use_graph=True,
-                              ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale, num_samples=num_samples, **kn)
+                              ddim_steps=ddim_steps, eta=eta, guidance_scale=guidance_scale, num_samples=num_samples,
+                              dpm_steps=dpm_steps, **kn)
             if inpaint:
                 sampled[i & 1].record(main)
             if num_samples is not None:

@@ -324,6 +324,23 @@ def guided_step(x0_hat, x0_ld, x_t, z, t_dev, coef_x0, coef_xt, sigma, M, guidan
              _p(x_prev), _p(xprev_bf16), bf16_ld, seed, offset, _p(t_next), _p(t_succ), float(guidance_scale), stream_ptr())
 
 
+def multistep_step(x0_hat, x0_ld, x_t, t_dev, coef_x0, coef_xt, coef_prev, t_succ, M, x0_prev, x_prev=None, xprev_bf16=None,
+                   bf16_ld=0, t_next=None, guidance_scale=None, known=None, known_mask=None):
+    """One DPM-Solver++(2M) step (``ibm_ddpm_multistep_step``) on the tables of ``diffusion.dpm_schedule``: x_p =
+    coef_x0[t] x0_hat + coef_prev[t] x0_prev + coef_xt[t] x_t, no noise; t_next receives t_succ[t].  ``x0_prev`` (fp32 [M, 30])
+    holds the previous step's prediction, is read only where coef_prev[t] != 0 and receives this step's in place.
+    ``guidance_scale`` None: x0_hat holds M rows; a scale: 2M rows combined as in ``guided_step``.  ``known`` /
+    ``known_mask`` as in ``posterior_step``, applied after the guided combination."""
+    if not isinstance(x0_prev, torch.Tensor) or not x0_prev.is_cuda or x0_prev.dtype != torch.float32 or \
+            not x0_prev.is_contiguous() or tuple(x0_prev.shape) != (M, 30):
+        raise ValueError(f"x0_prev must be a contiguous fp32 CUDA tensor of shape {(M, 30)}")
+    _check_known(known, known_mask, M)
+    guided = guidance_scale is not None
+    call("ibm_ddpm_multistep_step", _p(x0_hat), x0_ld, _p(x_t), _p(t_dev), _p(coef_x0), _p(coef_xt), _p(coef_prev), _p(t_succ), M,
+         _p(x0_prev), _p(x_prev), _p(xprev_bf16), bf16_ld, _p(t_next), float(guidance_scale) if guided else 1.0, int(guided),
+         _p(known), _p(known_mask), stream_ptr())
+
+
 def cond_dropout(xc, B, F, col0, ncols, p, seed, offset, keep_out=None):
     """Zeroes columns col0 .. col0+ncols-1 of the F rows of each dropped window of xc (bf16 [B*F, ld]); window b is dropped
     iff word 0 of Philox draw b at (seed, offset) is below uint32(p * 2^32), every window at p = 1.  keep_out (uint8 [B]):
